@@ -3,6 +3,7 @@
 20 power iterations, on a synthetic Twitter-shaped graph (1 M users, 10 M tweets, ~200 M links, power-law degrees).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp64|fp32] [--scale S]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one seed: init + 20 x (SpMV + cut rows + epilogue) with the graph resident in HBM.
   value      GTEPS = nnz(W) x iterations x seeds / time, K steps bracketed by barrier + synchronize, CUDA events on
@@ -213,6 +214,8 @@ def run_ours(args):
     ev1.record()
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, int(seeds[args.warmup + args.steps - 1]))
     model.close()
 
     # ---- the same device-resident loop in the other precision (C2 is specified for FP64 and FP32)
@@ -362,6 +365,29 @@ def run_ours(args):
         dist.destroy_process_group()
     if line is not None:
         print(json.dumps(line), flush=True)
+
+
+DUMP_SAMPLE = 2_000_000         # scores kept by --dump-outputs: 2 x 16 MB with their node indices (C2 has 11 M nodes)
+
+
+def dump_outputs(out_dir: str, model, seed: int) -> None:
+    """--dump-outputs: what the last timed step hands its caller, as float64 .npy files -- the rank vector of `seed`
+    (all of it, or the same DUMP_SAMPLE nodes drawn with a fixed seed when it is longer) and its top-10 (node, score)."""
+    import numpy as np
+    scores = model.scores(0)
+    idx = np.arange(len(scores))
+    if len(scores) > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(20260102).choice(len(scores), DUMP_SAMPLE, replace=False))
+    ids, sc, cnt = model.topk(TOP_K)
+    save_outputs(out_dir, {"seed": [seed], "scores": scores[idx], "scores_nodes": idx, "top10_nodes": ids[0, :cnt[0]],
+                           "top10_scores": sc[0, :cnt[0]]})
+
+
+def save_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
 
 
 def batched_frac(n: int, nnz: int, vb: int, width: int, seeds_per_rank: int, iterate_s: float) -> float:
@@ -709,8 +735,10 @@ def run_reference(args):
         og.run_many(seeds[i * threads:(i + 1) * threads], C_FLOAT, sample_iters, threads)
     t0 = time.perf_counter()
     for i in range(args.warmup, n_total):
-        og.run_many(seeds[i * threads:(i + 1) * threads], C_FLOAT, sample_iters, threads)
+        last = og.run_many(seeds[i * threads:(i + 1) * threads], C_FLOAT, sample_iters, threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        save_outputs(args.dump_outputs, {"seeds": seeds[(n_total - 1) * threads:n_total * threads], "rank_at_seed": last})
     value = nnz * sample_iters * threads * args.steps / dt / 1e9
     reference_itself = reference_on_a_scaled_graph(args.scale)
     sample = (f"each step = {threads} seeds on {threads} threads (one graph per thread, Program.cs:11/:61-66), "
@@ -778,7 +806,11 @@ def main():
     ap.add_argument("--c5-parity-users", type=int, default=8, help="test users of the C5 leg checked against the CPU oracle (rank 0)")
     ap.add_argument("--no-extended-parity", action="store_true", help="skip the 20-iteration oracle / extended-precision / GPU comparison (~50 s of CPU)")
     ap.add_argument("--parity-seeds", type=int, default=8, help="seeds of the batched (C3) leg checked against the CPU oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (float64): "
+                                                          "scores and top-10 (ours), rank[seed] of each seed (reference)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

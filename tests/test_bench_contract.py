@@ -5,15 +5,18 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 from conftest import ROOT
 
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 
 
-def test_reference_arm_prints_the_contract_line():
+def test_reference_arm_prints_the_contract_line(tmp_path):
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--scale", "0.004", "--steps", "2",
-                        "--warmup", "1", "--gpus", "1"], capture_output=True, text=True, timeout=600)
+                        "--warmup", "1", "--gpus", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [l for l in p.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1                                        # ONE JSON line
@@ -33,6 +36,17 @@ def test_reference_arm_prints_the_contract_line():
     ri = cb["reference_itself"]
     if ri is not None:
         assert ri["kind"] == "reference" and "error" not in ri and ri["gteps"] > 0
+    # --dump-outputs: rank[seed] after Model.run(cpu_iters) of every seed of the last timed step (step 3 of warm-up 1 + 2)
+    import oracle as O
+    seeds, got = np.load(tmp_path / "seeds.npy"), np.load(tmp_path / "rank_at_seed.npy")
+    assert seeds.dtype == got.dtype == np.float64 and len(seeds) == len(got) == cb["cores"]
+    links = O.synth_generate(bench.scaled_spec(0.004))
+    og = O.OracleGraph(links["node_id"], links["node_type"], links["src"], links["dst"], links["etype"], links["w"])
+    assert og.build() == 0
+    raw_deg = np.bincount(links["src"], minlength=og.n)
+    assert seeds.tolist() == bench.pick_seeds(raw_deg, bench.scaled_spec(0.004)["n_users"], 3 * len(seeds))[-len(seeds):].tolist()
+    want = [og.run(int(s), O.widen_float(bench.C_FLOAT), n_iter=2)[0][int(s)] for s in seeds]
+    assert np.array_equal(got, want)
 
 
 def test_other_ranks_of_the_reference_arm_exit_without_work():
@@ -40,6 +54,76 @@ def test_other_ranks_of_the_reference_arm_exit_without_work():
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--scale", "0.004", "--gpus", "2"],
                        capture_output=True, text=True, timeout=120, env=env)
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_zero_steps_are_refused():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert p.returncode == 2 and "--steps must be at least 1" in p.stderr
+
+
+def test_dump_outputs_samples_a_long_rank_vector(tmp_path):
+    """Above DUMP_SAMPLE nodes the rank vector is dumped as the same seeded sample of nodes, with their indices, every time."""
+    n = bench.DUMP_SAMPLE + 12_345
+
+    class Model:
+        def scores(self, slot):
+            return np.arange(n) * 0.5
+
+        def topk(self, k):
+            return np.arange(k)[None, ::-1] * 3, np.arange(k)[None, ::-1] * 1.5, np.array([k], np.int32)
+
+    outs = []
+    for k in range(2):
+        bench.dump_outputs(str(tmp_path / f"run{k}"), Model(), 7)
+        outs.append({f[:-4]: np.load(tmp_path / f"run{k}" / f) for f in os.listdir(tmp_path / f"run{k}")})
+        assert sum(os.path.getsize(tmp_path / f"run{k}" / f) for f in os.listdir(tmp_path / f"run{k}")) <= 64 << 20
+    a, b = outs
+    assert all(x.dtype == np.float64 and np.array_equal(x, b[name]) for name, x in a.items())
+    nodes = a["scores_nodes"]
+    assert len(nodes) == bench.DUMP_SAMPLE and np.all(np.diff(nodes) > 0) and nodes[0] >= 0 and nodes[-1] < n
+    assert np.array_equal(a["scores"], nodes * 0.5) and a["seed"].tolist() == [7]
+    assert a["top10_nodes"].tolist() == list(range(27, -1, -3)) and a["top10_scores"].tolist() == [i * 1.5 for i in range(9, -1, -1)]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_match_the_json_line(tmp_path):
+    """--dump-outputs on a scaled-down C2 graph, twice: the same arrays bit for bit (seeded inputs), float64, under 64 MB,
+    --steps timed steps in the JSON line, and the dump is the last timed step's seed, rank vector and top-10."""
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--scale", "0.004", "--steps", "3", "--warmup", "3",
+                            "--no-cpu", "--no-c5", "--batch-seeds", "16", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900)
+        assert p.returncode == 0, p.stderr[-2000:]
+        d = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
+        assert d["steps"] == 3
+        files = sorted(os.listdir(out))
+        assert files == ["scores.npy", "scores_nodes.npy", "seed.npy", "top10_nodes.npy", "top10_scores.npy"]
+        assert sum(os.path.getsize(out / f) for f in files) <= 64 << 20
+        runs.append({f[:-4]: np.load(out / f) for f in files})
+    a, b = runs
+    for name, x in a.items():
+        assert x.dtype == np.float64 and np.array_equal(x.view(np.uint64), b[name].view(np.uint64)), name
+    # the seed of the last timed step (warm-up 3 + 3 steps: the sixth bench seed), its whole rank vector at this size and its
+    # top-10 against the oracle on the same graph
+    import oracle as O
+    import recommendersystems_b200 as rs
+    spec = bench.scaled_spec(0.004)
+    g = rs.Graph.synthetic(spec)
+    g.buildGraph()
+    seed = int(bench.pick_seeds(g.degrees(raw=True), spec["n_users"], 12)[5])
+    links = g.export_links()
+    g.close()
+    assert a["seed"].tolist() == [seed] and np.array_equal(a["scores_nodes"], np.arange(d["config"]["n_nodes"]))
+    og = O.OracleGraph(links["node_id"], links["node_type"], links["src"], links["dst"], links["etype"], links["w"])
+    assert og.build() == 0
+    want, _ = og.run(seed, O.widen_float(bench.C_FLOAT), n_iter=bench.N_ITER)
+    nz = want != 0
+    assert np.all(a["scores"][~nz] == 0) and (np.abs(a["scores"][nz] - want[nz]) / want[nz]).max() <= 1e-12
+    ids, sc = og.recommend(seed, bench.C_FLOAT, bench.N_ITER, top_n=bench.TOP_K)
+    assert a["top10_nodes"].tolist() == ids.tolist() and (np.abs(a["top10_scores"] - sc) / sc).max() <= 1e-12
+    og.close()
 
 
 def test_byte_formulas_of_survey_8d():

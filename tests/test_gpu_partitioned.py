@@ -16,6 +16,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_single_rank_communicator_degenerates_to_the_whole_graph():
     """n_ranks == 1: NCCL is bound and initialised, the slice is the whole graph, results equal the plain path."""
     import numpy as np
+    # torch first, as in every process that creates a Comm: the library dlopens "libnccl.so.2" with RTLD_GLOBAL, and an older
+    # system NCCL loaded first would be bound by torch's libtorch_cuda.so too when a later test of this process imports torch
+    import torch  # noqa: F401
     from recommendersystems_b200.rwr import run_fixed
     comm = rs.Comm(0, 1, rs.Comm.unique_id(), device=0)
     spec = dict(seed=3, n_users=500, n_items=4000, n_third=50, authorship_per_mille=800, n_like=15000, n_friend=3000,
