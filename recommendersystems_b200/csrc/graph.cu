@@ -13,6 +13,7 @@
 #include "graph.h"
 #include "primitives.cuh"
 #include "dist.h"
+#include "stream.h"
 
 // ------------------------------------------------------------------------------------------------ kernels
 __global__ void k_i32_to_u8(const int32_t* __restrict__ in, u8* __restrict__ out, size_t n, int* bad) {
@@ -1002,8 +1003,8 @@ int rwr_graph_get_info(rwr_graph* g, rwr_graph_info* info) {
     info->layout = g->built ? g->layout : 0;
     info->relabelled = g->relabelled ? 1 : 0;
     info->n_hot = g->n_hot;
-    info->hub_entries_fp64 = g->built ? hub_entries_for(g, RWR_FP64) : 0;
-    info->hub_entries_fp32 = g->built ? hub_entries_for(g, RWR_FP32) : 0;
+    info->hub_entries_fp64 = g->built ? ws_hub_entries(g, RWR_FP64) : 0;
+    info->hub_entries_fp32 = g->built ? ws_hub_entries(g, RWR_FP32) : 0;
     info->n_chunks = g->n_chunks;
     info->row_begin = g->row_begin;
     info->row_end = g->built ? g->row_end : 0;

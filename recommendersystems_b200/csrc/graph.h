@@ -146,4 +146,3 @@ void graph_init_device(rwr_graph* g, const rwr_opts* opts);
 void graph_finish_create(rwr_graph* g);          // canonicalise raw links on the device (sort by source if needed)
 // iterate.cu
 void iterate_prepare(rwr_graph* g);              // partition table, hub sizing
-int hub_entries_for(const rwr_graph* g, int precision);

@@ -75,8 +75,6 @@ __global__ void k_unpermute(const T* __restrict__ y_int, const int32_t* __restri
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-int hub_entries_for(const rwr_graph* g, int precision) { return ws_hub_entries(g, precision); }
-
 void iterate_prepare(rwr_graph* g) {
     cudaStream_t st = g->stream;
     const u64 total = (u64)g->n + (u64)g->nnz_in;
@@ -140,20 +138,35 @@ static void launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, d
     }
 }
 
+// The scratch of one run of the iteration kernels.  Nothing in it needs initialising: k_init sets up ctl at the start of
+// every run, and every other entry is written earlier in the same iteration than it is read.  k_spmv_ws stores carry[t]
+// at the end of every tile t and head[t] at the first row end of a tile whose first row is continued; k_cutrows_ws reads
+// carry[m..t) and head[t] only for such a tile t whose continued row ends inside it.  Every block of k_finish_ws stores
+// its slot_S / slot_R entry before it takes its ticket, and only the block that takes the last ticket reads them.  (The
+// probe ablation RWR_DEBUG_MODE=1 stores no row ends, so its k_cutrows_ws reads head unwritten: its sums mean nothing.)
 struct RunWorkspace {
     Scratch<unsigned char> xa, xb, ya, yv;
     Scratch<double> carry, head, slot_S, slot_R;
     Scratch<IterCtl> ctl;
     void* x[2] = {nullptr, nullptr};      // the two gather vectors: scratch, or the peer-mapped buffers of a partitioned graph
-    void alloc_x(rwr_graph* g, size_t vec_bytes) {
-        if (g->p2p) { x[0] = g->px[0]; x[1] = g->px[1]; return; }
-        xa.alloc(&g->scratch, vec_bytes); xb.alloc(&g->scratch, vec_bytes);
-        x[0] = xa.p; x[1] = xb.p;
-    }
-    // column blocking of x (experimental): partial row sums of the virtual rows
-    void alloc_yv(rwr_graph* g, size_t elt) {
-        if (g->ws_compact) yv.alloc(&g->scratch, (size_t)g->v_compact * elt + 16);
-        else if (g->x_blocks > 1) yv.alloc(&g->scratch, (size_t)g->x_blocks * (size_t)g->v_rows * elt + 16);
+    // ya: the second rank vector of threshold mode and the probe's y (a fixed-count run into y_out leaves it unused)
+    template <typename T>
+    void alloc(rwr_graph* g, size_t ya_bytes) {
+        const size_t vec_bytes = ((size_t)g->n + 8) * sizeof(T);
+        if (g->p2p) {
+            x[0] = g->px[0]; x[1] = g->px[1];
+        } else {
+            xa.alloc(&g->scratch, vec_bytes); xb.alloc(&g->scratch, vec_bytes);
+            x[0] = xa.p; x[1] = xb.p;
+        }
+        // column blocking of x (experimental): partial row sums of the virtual rows
+        if (g->ws_compact) yv.alloc(&g->scratch, (size_t)g->v_compact * sizeof(T) + 16);
+        else if (g->x_blocks > 1) yv.alloc(&g->scratch, (size_t)g->x_blocks * (size_t)g->v_rows * sizeof(T) + 16);
+        ya.alloc(&g->scratch, ya_bytes);
+        carry.alloc(&g->scratch, (size_t)g->ws_tiles + 1); head.alloc(&g->scratch, (size_t)g->ws_tiles + 1);
+        const size_t slots = (size_t)g->sm_count * 8 + 8;
+        slot_S.alloc(&g->scratch, slots); slot_R.alloc(&g->scratch, slots);
+        ctl.alloc(&g->scratch, 1);
     }
 };
 
@@ -212,38 +225,44 @@ static void set_exchange(rwr_graph* g, IterParams<T>& p, const void* x_next, boo
     }
 }
 
+// The launch parameters every iteration of a run shares: graph, seed (internal label of seed_orig, -1: uniform restart),
+// hub, hot limit and workspace.  The vectors (x, x_next, r_prev, y) and the exchange are set per launch.
+template <typename T>
+static IterParams<T> iter_params(rwr_graph* g, const RunWorkspace& ws, int seed_orig, double c) {
+    int seed_int = -1;
+    if (seed_orig >= 0) {
+        CUDA_CHECK(cudaMemcpyAsync(&seed_int, g->new_of_old.p + seed_orig, sizeof(int), cudaMemcpyDeviceToHost, g->stream));
+        CUDA_CHECK(cudaStreamSynchronize(g->stream));
+    }
+    IterParams<T> p{};
+    p.n = g->n; p.inv = Prec<T>::inv(g);
+    p.ws_src = g->ws_src.p; p.ws_val = Prec<T>::wsval(g); p.ws_tile = g->ws_tile.p; p.ws_tiles = g->ws_tiles; p.tile_links = g->ws_tile_links;
+    p.row_begin = g->row_begin; p.row_end = g->row_end;
+    p.omc = (T)(1.0 - c);                                      // Model.cs:84 `(1 - dampingFactor)`
+    p.seed = seed_int; p.inv_n = g->n ? 1.0 / (double)g->n : 0.0; p.hub = ws_hub_entries(g, Prec<T>::id); p.n_hot = hot_limit(g);
+    p.head_partial = ws.head.p; p.carry = ws.carry.p;
+    p.slot_S = ws.slot_S.p; p.slot_R = ws.slot_R.p; p.ctl = ws.ctl.p;
+    p.yv = reinterpret_cast<T*>(ws.yv.p); p.x_blocks = g->x_blocks; p.v_rows = g->v_rows;
+    return p;
+}
+
 // Runs one seed.  mode 0: fixed n_iter; mode 1: threshold.  Final rank lands in y_out (internal labels).
 template <typename T>
 static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int mode, int n_iter, double thr, int max_iter,
                     T* y_out, int* iters_out, double* resid_out, float* iter_ms, cudaEvent_t ev0, cudaEvent_t ev1) {
     cudaStream_t st = g->stream;
     const int n = g->n;
-    int seed_int = -1;
-    if (seed_orig >= 0) {
-        CUDA_CHECK(cudaMemcpyAsync(&seed_int, g->new_of_old.p + seed_orig, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-    }
-    const int hub = hub_entries_for(g, Prec<T>::id);
-
+    IterParams<T> p = iter_params<T>(g, ws, seed_orig, c);
     T* xa = reinterpret_cast<T*>(ws.x[0]);
     T* xb = reinterpret_cast<T*>(ws.x[1]);
     T* ya = reinterpret_cast<T*>(ws.ya.p);
-    IterParams<T> p;
-    p.n = n; p.inv = Prec<T>::inv(g);
-    p.ws_src = g->ws_src.p; p.ws_val = Prec<T>::wsval(g); p.ws_tile = g->ws_tile.p; p.ws_tiles = g->ws_tiles; p.tile_links = g->ws_tile_links;
-    p.row_begin = g->row_begin; p.row_end = g->row_end;
-    p.omc = (T)(1.0 - c);                                      // Model.cs:84 `(1 - dampingFactor)`
-    p.seed = seed_int; p.inv_n = n ? 1.0 / (double)n : 0.0; p.hub = hub; p.n_hot = hot_limit(g); p.debug = 0;
-    p.head_partial = ws.head.p; p.carry = ws.carry.p;
-    p.slot_S = ws.slot_S.p; p.slot_R = ws.slot_R.p; p.ctl = ws.ctl.p;
-    p.yv = reinterpret_cast<T*>(ws.yv.p); p.x_blocks = g->x_blocks; p.v_rows = g->v_rows;
 
     // uniform constructor: S0 = sum over nodes of (dangling ? 1 : 1 - fl((1-c)*1))
     const double omc_d = (double)p.omc;
     const double S_uniform = (double)g->n_dangling + (double)(n - g->n_dangling) * (1.0 - omc_d);
     // r0 goes to y_out in fixed mode (also the answer for n_iter == 0); threshold mode ping-pongs ya <-> y_out
     T* r_cur = (mode == 0) ? y_out : ya;
-    k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, seed_int, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform);
+    k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform);
     KERNEL_CHECK();
     g->pool.launches += 1;
 
@@ -265,7 +284,7 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
         rwr_graph::IterGraph& ig = g->iter_graph[Prec<T>::id];
         const void* key[8] = {xa, xb, y_out, ws.ctl.p, ws.head.p, ws.carry.p, ws.slot_S.p, ws.slot_R.p};
         const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1;
-        const bool same = ig.n_iter == n_iter && ig.hub == hub && ig.c == c && memcmp(ig.ptr, key, sizeof(key)) == 0;
+        const bool same = ig.n_iter == n_iter && ig.hub == p.hub && ig.c == c && memcmp(ig.ptr, key, sizeof(key)) == 0;
         if (graphable && same && (ig.exec || ig.seen)) {
             // second and later runs with this key: replay the graph of the whole loop (captured now if this is the second
             // run); nothing in it depends on the seed
@@ -293,7 +312,7 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
             // than one run saves, and the reference asks each graph for a single recommendation (Experiment.cs:109).
             if (graphable) {
                 if (ig.exec) { cudaGraphExecDestroy(ig.exec); ig.exec = nullptr; }
-                ig.seen = true; ig.n_iter = n_iter; ig.hub = hub; ig.c = c;
+                ig.seen = true; ig.n_iter = n_iter; ig.hub = p.hub; ig.c = c;
                 memcpy(ig.ptr, key, sizeof(key));
             }
             launch_all();
@@ -366,17 +385,7 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     if (Prec<T>::ybuf(res).n != std::max<size_t>(1, ld * (size_t)n_seeds))      // a re-run keeps its rank buffers
         Prec<T>::ybuf(res).alloc(std::max<size_t>(1, ld * (size_t)n_seeds), nullptr);
     RunWorkspace ws;
-    const size_t vec_bytes = (n + 8) * sizeof(T);
-    ws.alloc_x(g, vec_bytes); ws.alloc_yv(g, sizeof(T)); ws.ya.alloc(&g->scratch, vec_bytes);
-    ws.carry.alloc(&g->scratch, (size_t)g->ws_tiles + 1); ws.head.alloc(&g->scratch, (size_t)g->ws_tiles + 1);
-    CUDA_CHECK(cudaMemsetAsync(ws.carry.p, 0, ((size_t)g->ws_tiles + 1) * sizeof(double), st));
-    CUDA_CHECK(cudaMemsetAsync(ws.head.p, 0, ((size_t)g->ws_tiles + 1) * sizeof(double), st));
-    const size_t slots = (size_t)g->sm_count * 8 + 8;
-    ws.slot_S.alloc(&g->scratch, slots); ws.slot_R.alloc(&g->scratch, slots);
-    CUDA_CHECK(cudaMemsetAsync(ws.slot_S.p, 0, slots * sizeof(double), st));
-    CUDA_CHECK(cudaMemsetAsync(ws.slot_R.p, 0, slots * sizeof(double), st));
-    ws.ctl.alloc(&g->scratch, 1);
-    CUDA_CHECK(cudaMemsetAsync(ws.ctl.p, 0, sizeof(IterCtl), st));
+    ws.alloc<T>(g, (n + 8) * sizeof(T));
     DevEvent ev0, ev1, evA, evB;
     const int64_t launches0 = g->pool.launches;
     CUDA_CHECK(cudaEventRecord(evA, st));
@@ -394,7 +403,7 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     CUDA_CHECK(cudaEventSynchronize(evB));
     CUDA_CHECK(cudaEventElapsedTime(&res->total_ms, evA, evB));
     res->launches = g->pool.launches - launches0;
-    check_exchange_fault(g, ws.ctl.p);
+    if (n_seeds) check_exchange_fault(g, ws.ctl.p);       // (no seed: nothing ran, and nothing has set up ctl)
 }
 
 template <typename T>
@@ -403,33 +412,14 @@ static void profile_impl(rwr_graph* g, int seed_orig, double c, int reps, float*
     const size_t n = (size_t)g->n;
     if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
     RunWorkspace ws;
-    const size_t vec_bytes = (n + 8) * sizeof(T);
-    ws.alloc_x(g, vec_bytes); ws.alloc_yv(g, sizeof(T)); ws.ya.alloc(&g->scratch, vec_bytes);
-    ws.carry.alloc(&g->scratch, (size_t)g->ws_tiles + 1); ws.head.alloc(&g->scratch, (size_t)g->ws_tiles + 1);
-    CUDA_CHECK(cudaMemsetAsync(ws.carry.p, 0, ((size_t)g->ws_tiles + 1) * sizeof(double), st));
-    CUDA_CHECK(cudaMemsetAsync(ws.head.p, 0, ((size_t)g->ws_tiles + 1) * sizeof(double), st));
-    const size_t slots = (size_t)g->sm_count * 8 + 8;
-    ws.slot_S.alloc(&g->scratch, slots); ws.slot_R.alloc(&g->scratch, slots);
-    CUDA_CHECK(cudaMemsetAsync(ws.slot_S.p, 0, slots * sizeof(double), st));
-    CUDA_CHECK(cudaMemsetAsync(ws.slot_R.p, 0, slots * sizeof(double), st));
-    ws.ctl.alloc(&g->scratch, 1);
-    int seed_int = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&seed_int, g->new_of_old.p + seed_orig, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    const int hub = hub_entries_for(g, Prec<T>::id);
+    ws.alloc<T>(g, (n + 8) * sizeof(T));
+    IterParams<T> p = iter_params<T>(g, ws, seed_orig, c);
     T* xa = reinterpret_cast<T*>(ws.x[0]);
     T* xb = reinterpret_cast<T*>(ws.x[1]);
     T* ya = reinterpret_cast<T*>(ws.ya.p);
-    IterParams<T> p;
-    p.n = g->n; p.inv = Prec<T>::inv(g);
-    p.ws_src = g->ws_src.p; p.ws_val = Prec<T>::wsval(g); p.ws_tile = g->ws_tile.p; p.ws_tiles = g->ws_tiles; p.tile_links = g->ws_tile_links;
-    p.row_begin = g->row_begin; p.row_end = g->row_end;
-    p.omc = (T)(1.0 - c); p.seed = seed_int; p.inv_n = n ? 1.0 / (double)n : 0.0; p.hub = hub; p.n_hot = hot_limit(g);
-    p.head_partial = ws.head.p; p.carry = ws.carry.p; p.slot_S = ws.slot_S.p; p.slot_R = ws.slot_R.p; p.ctl = ws.ctl.p;
     p.r_prev = nullptr; p.y = ya;
-    p.yv = reinterpret_cast<T*>(ws.yv.p); p.x_blocks = g->x_blocks; p.v_rows = g->v_rows;
     { const char* dm = getenv("RWR_DEBUG_MODE"); p.debug = dm ? atoi(dm) : 0; }
-    k_init<T><<<div_up(std::max((int)n, 1), 256), 256, 0, st>>>((int)n, seed_int, p.omc, p.inv, ya, xa, xb, ws.ctl.p, 0.0);
+    k_init<T><<<div_up(std::max((int)n, 1), 256), 256, 0, st>>>((int)n, p.seed, p.omc, p.inv, ya, xa, xb, ws.ctl.p, 0.0);
     KERNEL_CHECK();
     std::vector<DevEvent> ev(3 * (size_t)reps);
     T* x_cur = xa;
@@ -465,15 +455,9 @@ static void profile_impl(rwr_graph* g, int seed_orig, double c, int reps, float*
 template <typename T>
 void iterate_single_into(rwr_graph* g, int seed_orig, double c, int n_iter, T* y_out, float* iter_ms, int64_t* launches,
                          cudaEvent_t ext0, cudaEvent_t ext1) {
-    const size_t n = (size_t)g->n;
     if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
     RunWorkspace ws;
-    const size_t vec_bytes = (n + 8) * sizeof(T);
-    ws.alloc_x(g, vec_bytes); ws.alloc_yv(g, sizeof(T)); ws.ya.alloc(&g->scratch, 16);
-    ws.carry.alloc(&g->scratch, (size_t)g->ws_tiles + 1); ws.head.alloc(&g->scratch, (size_t)g->ws_tiles + 1);
-    const size_t slots = (size_t)g->sm_count * 8 + 8;
-    ws.slot_S.alloc(&g->scratch, slots); ws.slot_R.alloc(&g->scratch, slots);
-    ws.ctl.alloc(&g->scratch, 1);
+    ws.alloc<T>(g, 16);
     const int64_t l0 = g->pool.launches;
     int it = 0;
     double rs = 0;

@@ -415,16 +415,46 @@ static void mark_excluded(rwr_graph* g, int seed, u32* excl, size_t words) {
     g->pool.launches += 1;
 }
 
+// blocks of the top-k scans over a rank vector or a seed tile
+static int topk_grid(const rwr_graph* g) {
+    return std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up((size_t)std::max(g->n, 1), TOPK_THREADS)));
+}
+
+// Scratch of the k <= 16 top-k of `lists` rank vectors: the exclusion bitmap and the block candidates serve one list after
+// the other; the results of all lists are zeroed up front (the slots past a short list's count read 0) and go out together.
+struct TopkScratch {
+    const size_t words;         // exclusion bitmap, + 1 spare word (a partitioned build's "the seed has links" flag)
+    const int grid, k, lists;
+    Scratch<u32> excl;
+    Scratch<Cand> block_out;
+    Scratch<int64_t> ids;
+    Scratch<double> scores;
+    Scratch<int> counts;
+    TopkScratch(rwr_graph* g, int k_, int lists_) : words(((size_t)g->n + 31) / 32 + 1), grid(topk_grid(g)), k(k_), lists(lists_) {
+        excl.alloc(&g->scratch, words); block_out.alloc(&g->scratch, (size_t)grid * k);
+        ids.alloc(&g->scratch, (size_t)lists * k); scores.alloc(&g->scratch, (size_t)lists * k); counts.alloc(&g->scratch, lists);
+        CUDA_CHECK(cudaMemsetAsync(ids.p, 0, (size_t)lists * k * 8, g->stream));
+        CUDA_CHECK(cudaMemsetAsync(scores.p, 0, (size_t)lists * k * 8, g->stream));
+    }
+    // enqueues the copies of every list's result; the caller synchronises
+    void copy_out(cudaStream_t st, int64_t* out_ids, double* out_scores, int32_t* out_counts) const {
+        CUDA_CHECK(cudaMemcpyAsync(out_ids, ids.p, (size_t)lists * k * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaMemcpyAsync(out_scores, scores.p, (size_t)lists * k * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaMemcpyAsync(out_counts, counts.p, (size_t)lists * 4, cudaMemcpyDeviceToHost, st));
+    }
+};
+
+// top-k of the rank vector y (stride ld) into result `list` of ts
 template <typename T>
-static void topk_one(rwr_graph* g, const T* y, int ld, int seed, int k, u32* excl, size_t words, Cand* block_out, int grid,
-                     int64_t* d_ids, double* d_scores, int* d_count, bool marked = false) {
-    if (!marked) mark_excluded(g, seed, excl, words);
+static void topk_one(rwr_graph* g, TopkScratch& ts, int list, const T* y, int ld, int seed, bool marked = false) {
+    if (!marked) mark_excluded(g, seed, ts.excl.p, ts.words);
     Scratch<u64> block_max;
-    block_max.alloc(&g->scratch, (size_t)grid);
-    k_topk_bound<T><<<grid, TOPK_THREADS, 0, g->stream>>>(y, ld, g->node_type_int.p, excl, g->n, block_max.p);
-    k_topk_scan<T><<<grid, TOPK_THREADS, 0, g->stream>>>(y, ld, g->node_type_int.p, g->node_id_int.p, excl, g->n, k, block_max.p,
-                                                         block_out);
-    k_topk_merge<T><<<1, TOPK_THREADS, 0, g->stream>>>(block_out, grid * k, k, y, ld, d_ids, d_scores, d_count);
+    block_max.alloc(&g->scratch, (size_t)ts.grid);
+    k_topk_bound<T><<<ts.grid, TOPK_THREADS, 0, g->stream>>>(y, ld, g->node_type_int.p, ts.excl.p, g->n, block_max.p);
+    k_topk_scan<T><<<ts.grid, TOPK_THREADS, 0, g->stream>>>(y, ld, g->node_type_int.p, g->node_id_int.p, ts.excl.p, g->n, ts.k,
+                                                            block_max.p, ts.block_out.p);
+    k_topk_merge<T><<<1, TOPK_THREADS, 0, g->stream>>>(ts.block_out.p, ts.grid * ts.k, ts.k, y, ld, ts.ids.p + (size_t)list * ts.k,
+                                                       ts.scores.p + (size_t)list * ts.k, ts.counts.p + list);
     KERNEL_CHECK();
     g->pool.launches += 3;
 }
@@ -512,28 +542,12 @@ int rwr_topk(rwr_result* r, int32_t k, int64_t* out_ids, double* out_scores, int
         }
         return RWR_OK;
     }
-    const size_t words = ((size_t)g->n + 31) / 32 + 1;
-    const int grid = std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up((size_t)std::max(g->n, 1), TOPK_THREADS)));
-    Scratch<u32> excl;
-    Scratch<Cand> block_out;
-    Scratch<int64_t> d_ids;
-    Scratch<double> d_sc;
-    Scratch<int> d_cnt;
-    excl.alloc(&g->scratch, words); block_out.alloc(&g->scratch, (size_t)grid * k);
-    d_ids.alloc(&g->scratch, (size_t)S * k); d_sc.alloc(&g->scratch, (size_t)S * k); d_cnt.alloc(&g->scratch, S);
-    CUDA_CHECK(cudaMemsetAsync(d_ids.p, 0, (size_t)S * k * 8, st));
-    CUDA_CHECK(cudaMemsetAsync(d_sc.p, 0, (size_t)S * k * 8, st));
+    TopkScratch ts(g, k, S);
     for (int s = 0; s < S; s++) {
-        if (r->precision == RWR_FP64)
-            topk_one<double>(g, r->y64.p + (size_t)s * r->ld, 1, r->seeds[s], k, excl.p, words, block_out.p, grid,
-                             d_ids.p + (size_t)s * k, d_sc.p + (size_t)s * k, d_cnt.p + s);
-        else
-            topk_one<float>(g, r->y32.p + (size_t)s * r->ld, 1, r->seeds[s], k, excl.p, words, block_out.p, grid,
-                            d_ids.p + (size_t)s * k, d_sc.p + (size_t)s * k, d_cnt.p + s);
+        if (r->precision == RWR_FP64) topk_one<double>(g, ts, s, r->y64.p + (size_t)s * r->ld, 1, r->seeds[s]);
+        else topk_one<float>(g, ts, s, r->y32.p + (size_t)s * r->ld, 1, r->seeds[s]);
     }
-    CUDA_CHECK(cudaMemcpyAsync(out_ids, d_ids.p, (size_t)S * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_scores, d_sc.p, (size_t)S * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_counts, d_cnt.p, (size_t)S * 4, cudaMemcpyDeviceToHost, st));
+    ts.copy_out(st, out_ids, out_scores, out_counts);
     CUDA_CHECK(cudaStreamSynchronize(st));
     return RWR_OK;
     RWR_API_END
@@ -566,6 +580,32 @@ template <typename T>
 void iterate_single_into(rwr_graph* g, int seed_orig, double c, int n_iter, T* y_out, float* iter_ms, int64_t* launches,
                          cudaEvent_t ext0, cudaEvent_t ext1);
 
+// What a fixed-count run of n_seeds seeds reports (no residual: no convergence test ran)
+template <typename T>
+static void fill_info(rwr_run_info* info, const rwr_graph* g, int n_seeds, int n_iter, float iterate_ms, float total_ms,
+                      int64_t launches) {
+    if (!info) return;
+    info->n_seeds = n_seeds; info->n_nodes = g->n; info->precision = sizeof(T) == 4 ? RWR_FP32 : RWR_FP64;
+    info->iterations = n_iter; info->residual = NAN; info->iterate_ms = iterate_ms; info->total_ms = total_ms;
+    info->kernel_launches = launches;
+}
+
+// The internal labels of a seed list (for the SpMM tiles), and its original labels copied to d_orig (the tile kernels
+// read the seeds' raw link ranges)
+static std::vector<int32_t> seed_labels(rwr_graph* g, const int32_t* seeds, int n_seeds, Scratch<int32_t>& d_orig) {
+    cudaStream_t st = g->stream;
+    std::vector<int32_t> internal((size_t)n_seeds);
+    d_orig.alloc(&g->scratch, n_seeds);
+    Scratch<int32_t> d_int;
+    d_int.alloc(&g->scratch, n_seeds);
+    CUDA_CHECK(cudaMemcpyAsync(d_orig.p, seeds, (size_t)n_seeds * 4, cudaMemcpyHostToDevice, st));
+    k_lookup<<<div_up((size_t)n_seeds, 256), 256, 0, st>>>(g->new_of_old.p, d_orig.p, n_seeds, d_int.p);
+    KERNEL_CHECK();
+    CUDA_CHECK(cudaMemcpyAsync(internal.data(), d_int.p, (size_t)n_seeds * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    return internal;
+}
+
 // seeds one by one through the single-column kernel (k <= 16): no result objects, scratch from the handle's pool
 template <typename T>
 static void recommend_singles(rwr_graph* g, const int32_t* seeds, int n_seeds, double c, int n_iter, int k, int64_t* out_ids,
@@ -574,17 +614,7 @@ static void recommend_singles(rwr_graph* g, const int32_t* seeds, int n_seeds, d
     const size_t n = (size_t)g->n;
     Scratch<T> y;
     y.alloc(&g->scratch, n + 8);
-    const size_t words = (n + 31) / 32 + 1;
-    const int grid = std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up(std::max<size_t>(n, 1), TOPK_THREADS)));
-    Scratch<u32> excl;
-    Scratch<Cand> block_out;
-    Scratch<int64_t> d_ids;
-    Scratch<double> d_sc;
-    Scratch<int> d_cnt;
-    excl.alloc(&g->scratch, words); block_out.alloc(&g->scratch, (size_t)grid * k);
-    d_ids.alloc(&g->scratch, (size_t)n_seeds * k); d_sc.alloc(&g->scratch, (size_t)n_seeds * k); d_cnt.alloc(&g->scratch, n_seeds);
-    CUDA_CHECK(cudaMemsetAsync(d_ids.p, 0, (size_t)n_seeds * k * 8, st));
-    CUDA_CHECK(cudaMemsetAsync(d_sc.p, 0, (size_t)n_seeds * k * 8, st));
+    TopkScratch ts(g, k, n_seeds);
     float it_ms = 0.f;
     int64_t launches = 0;
     struct Events {                                 // destroyed on every exit path (a seed without links throws)
@@ -599,25 +629,18 @@ static void recommend_singles(rwr_graph* g, const int32_t* seeds, int n_seeds, d
     if (one) { CUDA_CHECK(cudaEventCreate(&i0)); CUDA_CHECK(cudaEventCreate(&i1)); }
     CUDA_CHECK(cudaEventRecord(e0, st));
     for (int s = 0; s < n_seeds; s++) {
-        if (one) mark_excluded(g, seeds[s], excl.p, words);
+        if (one) mark_excluded(g, seeds[s], ts.excl.p, ts.words);
         iterate_single_into<T>(g, seeds[s], c, n_iter, y.p, &it_ms, &launches, i0, i1);
-        topk_one<T>(g, y.p, 1, seeds[s], k, excl.p, words, block_out.p, grid, d_ids.p + (size_t)s * k, d_sc.p + (size_t)s * k,
-                    d_cnt.p + s, /*marked=*/one);
+        topk_one<T>(g, ts, s, y.p, 1, seeds[s], /*marked=*/one);
         launches += 3;
     }
-    CUDA_CHECK(cudaMemcpyAsync(out_ids, d_ids.p, (size_t)n_seeds * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_scores, d_sc.p, (size_t)n_seeds * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_counts, d_cnt.p, (size_t)n_seeds * 4, cudaMemcpyDeviceToHost, st));
+    ts.copy_out(st, out_ids, out_scores, out_counts);
     CUDA_CHECK(cudaEventRecord(e1, st));
     CUDA_CHECK(cudaEventSynchronize(e1));
     float tot = 0.f;
     CUDA_CHECK(cudaEventElapsedTime(&tot, e0, e1));
     if (one) CUDA_CHECK(cudaEventElapsedTime(&it_ms, i0, i1));
-    if (info) {
-        info->n_seeds = n_seeds; info->n_nodes = g->n; info->precision = sizeof(T) == 4 ? RWR_FP32 : RWR_FP64;
-        info->iterations = n_iter; info->residual = NAN; info->iterate_ms = it_ms; info->total_ms = tot;
-        info->kernel_launches = launches;
-    }
+    fill_info<T>(info, g, n_seeds, n_iter, it_ms, tot, launches);
 }
 
 template <typename T>
@@ -627,32 +650,13 @@ static void recommend_tiles(rwr_graph* g, const int32_t* seeds, int n_seeds, dou
     const int B = spmm_tile_width(sizeof(T) == 4 ? RWR_FP32 : RWR_FP64);
     const size_t n = (size_t)g->n;
     if (sizeof(T) == 4) ensure_fp32_arrays(g);
-    // internal labels of all seeds in one go
-    std::vector<int32_t> n2o((size_t)n_seeds);
-    Scratch<int32_t> d_seeds_all;                  // original labels of all seeds (the tile top-k reads their raw link ranges)
-    d_seeds_all.alloc(&g->scratch, n_seeds);
-    {
-        Scratch<int32_t> d_int;
-        d_int.alloc(&g->scratch, n_seeds);
-        CUDA_CHECK(cudaMemcpyAsync(d_seeds_all.p, seeds, (size_t)n_seeds * 4, cudaMemcpyHostToDevice, st));
-        k_lookup<<<div_up((size_t)n_seeds, 256), 256, 0, st>>>(g->new_of_old.p, d_seeds_all.p, n_seeds, d_int.p);
-        KERNEL_CHECK();
-        CUDA_CHECK(cudaMemcpyAsync(n2o.data(), d_int.p, (size_t)n_seeds * 4, cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-    }
+    Scratch<int32_t> d_seeds_all;
+    const std::vector<int32_t> n2o = seed_labels(g, seeds, n_seeds, d_seeds_all);
     Scratch<T> y;
     y.alloc(&g->scratch, n * B + 16);
-    const size_t words = (n + 31) / 32 + 1;
-    const int grid = std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up(std::max<size_t>(n, 1), TOPK_THREADS)));
-    Scratch<u32> excl;
-    Scratch<Cand> block_out;
-    Scratch<int64_t> d_ids;
-    Scratch<double> d_sc;
-    Scratch<int> d_cnt;
-    excl.alloc(&g->scratch, words); block_out.alloc(&g->scratch, (size_t)grid * k);
-    d_ids.alloc(&g->scratch, (size_t)n_seeds * k); d_sc.alloc(&g->scratch, (size_t)n_seeds * k); d_cnt.alloc(&g->scratch, n_seeds);
-    CUDA_CHECK(cudaMemsetAsync(d_ids.p, 0, (size_t)n_seeds * k * 8, st));
-    CUDA_CHECK(cudaMemsetAsync(d_sc.p, 0, (size_t)n_seeds * k * 8, st));
+    TopkScratch ts(g, k, n_seeds);
+    const size_t words = ts.words;
+    const int grid = ts.grid;
     Scratch<u32> excl_t;                           // [B][words] exclusion bitmaps of a tile
     Scratch<u64> tile_max, tile_bound;             // [grid][B] block maxima, [B] bounds
     Scratch<Cand> tile_cand;                       // [B][TILE_CAND_CAP]
@@ -683,8 +687,8 @@ static void recommend_tiles(rwr_graph* g, const int32_t* seeds, int n_seeds, dou
             k_topk_scan_tile<T, 16><<<grid, TOPK_THREADS, 0, st>>>(y.p, g->node_type_int.p, g->node_id_int.p, excl_t.p, words, g->n, cnt,
                                                                   tile_bound.p, tile_cand.p, tile_cnt.p);
         }
-        k_topk_merge_tile<T><<<cnt, TOPK_THREADS, 0, st>>>(tile_cand.p, tile_cnt.p, k, y.p, B, d_ids.p + (size_t)s0 * k,
-                                                          d_sc.p + (size_t)s0 * k, d_cnt.p + s0);
+        k_topk_merge_tile<T><<<cnt, TOPK_THREADS, 0, st>>>(tile_cand.p, tile_cnt.p, k, y.p, B, ts.ids.p + (size_t)s0 * k,
+                                                          ts.scores.p + (size_t)s0 * k, ts.counts.p + s0);
         KERNEL_CHECK();
         launches += 5;
         int h_cnt[2 * TILE_MAXB];
@@ -695,8 +699,7 @@ static void recommend_tiles(rwr_graph* g, const int32_t* seeds, int n_seeds, dou
             if (h_cnt[TILE_MAXB + j] && !g->opts.empty_seed_ok)
                 RWR_FAIL(RWR_E_BADSEED, "seed %d has no `edges` entry (KeyNotFoundException, Recommender.cs:21)", seeds[s0 + j]);
             if (h_cnt[j] > TILE_CAND_CAP) {              // too many candidates at the bound (ties): exact per-column path
-                topk_one<T>(g, y.p + j, B, seeds[s0 + j], k, excl.p, words, block_out.p, grid, d_ids.p + (size_t)(s0 + j) * k,
-                            d_sc.p + (size_t)(s0 + j) * k, d_cnt.p + s0 + j);
+                topk_one<T>(g, ts, s0 + j, y.p + j, B, seeds[s0 + j]);
                 launches += 4;
             }
         }
@@ -705,15 +708,9 @@ static void recommend_tiles(rwr_graph* g, const int32_t* seeds, int n_seeds, dou
         CUDA_CHECK(cudaEventElapsedTime(&b, e0, e2));
         it_ms += a; tot_ms += b;
     }
-    CUDA_CHECK(cudaMemcpyAsync(out_ids, d_ids.p, (size_t)n_seeds * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_scores, d_sc.p, (size_t)n_seeds * k * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(out_counts, d_cnt.p, (size_t)n_seeds * 4, cudaMemcpyDeviceToHost, st));
+    ts.copy_out(st, out_ids, out_scores, out_counts);
     CUDA_CHECK(cudaStreamSynchronize(st));
-    if (info) {
-        info->n_seeds = n_seeds; info->n_nodes = g->n; info->precision = sizeof(T) == 4 ? RWR_FP32 : RWR_FP64;
-        info->iterations = n_iter; info->residual = NAN; info->iterate_ms = it_ms; info->total_ms = tot_ms;
-        info->kernel_launches = launches;
-    }
+    fill_info<T>(info, g, n_seeds, n_iter, it_ms, tot_ms, launches);
 }
 
 extern "C" {
@@ -941,18 +938,8 @@ static void evaluate_tiles(rwr_graph* g, const int32_t* users, int n_users, cons
     const size_t n = (size_t)g->n;
     if (sizeof(T) == 4) ensure_fp32_arrays(g);
     ensure_id_lookup(g);
-    std::vector<int32_t> n2o((size_t)n_users);
     Scratch<int32_t> d_users;
-    d_users.alloc(&g->scratch, n_users);
-    {
-        Scratch<int32_t> d_int;
-        d_int.alloc(&g->scratch, n_users);
-        CUDA_CHECK(cudaMemcpyAsync(d_users.p, users, (size_t)n_users * 4, cudaMemcpyHostToDevice, st));
-        k_lookup<<<div_up((size_t)n_users, 256), 256, 0, st>>>(g->new_of_old.p, d_users.p, n_users, d_int.p);
-        KERNEL_CHECK();
-        CUDA_CHECK(cudaMemcpyAsync(n2o.data(), d_int.p, (size_t)n_users * 4, cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-    }
+    const std::vector<int32_t> n2o = seed_labels(g, users, n_users, d_users);
     const int64_t total_items = test_ptr[n_users];
     Scratch<int64_t> d_test;
     d_test.alloc(&g->scratch, (size_t)std::max<int64_t>(total_items, 1));
@@ -963,7 +950,7 @@ static void evaluate_tiles(rwr_graph* g, const int32_t* users, int n_users, cons
     Scratch<T> y;
     y.alloc(&g->scratch, n * B + 16);
     const size_t words = (n + 31) / 32 + 1;
-    const int grid = std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up(std::max<size_t>(n, 1), TOPK_THREADS)));
+    const int grid = topk_grid(g);
     Scratch<u32> excl_t, hist;
     Scratch<EvalItem> items;
     Scratch<u64> skey;
@@ -1024,11 +1011,7 @@ static void evaluate_tiles(rwr_graph* g, const int32_t* users, int n_users, cons
     CUDA_CHECK(cudaMemcpyAsync(hits_at_k, d_atk.p, (size_t)n_users * 4, cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaMemcpyAsync(avg_precision, d_ap.p, (size_t)n_users * 8, cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaStreamSynchronize(st));
-    if (info) {
-        info->n_seeds = n_users; info->n_nodes = g->n; info->precision = sizeof(T) == 4 ? RWR_FP32 : RWR_FP64;
-        info->iterations = n_iter; info->residual = NAN; info->iterate_ms = it_ms; info->total_ms = tot_ms;
-        info->kernel_launches = launches;
-    }
+    fill_info<T>(info, g, n_users, n_iter, it_ms, tot_ms, launches);
 }
 
 extern "C" {
