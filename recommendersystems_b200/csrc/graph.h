@@ -49,6 +49,7 @@ struct rwr_graph {
                                         //     non-uniform row, 0.0 for a dangling row
     int32_t n_dangling = 0;
     bool all_uniform = false;
+    bool fr_finite = false;             // every inv and weight entry is finite: single-seed runs may push from the frontier
     u32 max_out_degree = 0, max_in_degree = 0;
 
     // ---- internal labelling (descending out-degree) and the pull CSR of W^T in internal labels
@@ -134,7 +135,9 @@ struct rwr_graph {
         bool seen = false;              // the key below was used by a direct run; the next identical run captures
         int n_iter = 0, hub = 0;
         double c = 0.0;
-        const void* ptr[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+        u64 fr_budget = 0;              // links per sparse iteration (0: no frontier kernels in the graph)
+        int64_t launches = 0;           // kernels one replay stands for
+        const void* ptr[9] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     } iter_graph[2];
     float build_ms = 0.f, synth_ms = 0.f;
     int sm_count = 148;

@@ -16,22 +16,31 @@
 
 #include "iterate_dev.cuh"
 #include "stream.h"
+#include "frontier.h"
 #include "dist.h"
 
 
 // ------------------------------------------------------------------------------------------------ K6: init
+// fr_bits (a run that may go sparse, frontier.cu): the frontier bitmap over the original labels gets the seed (when it
+// has out-links) and nothing else, and x1 -- the first x_next, which the frontier kernels write only at the active rows --
+// is zeroed.
 template <typename T>
 __global__ void k_init(int n, int seed, T omc, const T* __restrict__ inv, T* __restrict__ r0, T* __restrict__ x0,
-                       T* __restrict__ x1, IterCtl* ctl, double S_uniform) {
+                       T* __restrict__ x1, IterCtl* ctl, double S_uniform, u32* __restrict__ fr_bits, u32 fr_words, int seed_orig) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j < 8) { x0[n + j] = (T)0; x1[n + j] = (T)0; }     // x[n] is the always-zero entry the edge stream pads with
     if (j == 0) {
         ctl->resid = 0.0; ctl->done = 0; ctl->iters = 0; ctl->ticket = 0; ctl->fault = 0; ctl->wait_clk = 0;
         ctl->tile_ctr = 0;
         ctl->seed = seed;
+        ctl->sparse = fr_bits != nullptr;
+        ctl->sparse_iters = 0;
         if (seed < 0) ctl->S = S_uniform;
     }
+    if (fr_bits && (u32)j < fr_words)
+        fr_bits[j] = ((seed_orig >> 5) == j && inv[seed] != (T)0) ? 1u << (seed_orig & 31) : 0u;
     if (j >= n) return;
+    if (fr_bits) x1[j] = (T)0;
     const T r = (seed < 0) ? (T)1 : ((j == seed) ? (T)n : (T)0);           // Model.cs:24 / :44
     const T invj = inv[j];
     const T rw = mul_rn(omc, r);
@@ -84,6 +93,7 @@ void iterate_prepare(rwr_graph* g) {
     KERNEL_CHECK();
     CUDA_CHECK(cudaStreamSynchronize(st));
     stream_prepare(g);
+    frontier_prepare(g);
 }
 
 void ensure_fp32_arrays(rwr_graph* g) {
@@ -144,14 +154,18 @@ static void launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, d
 // carry[m..t) and head[t] only for such a tile t whose continued row ends inside it.  Every block of k_finish_ws stores
 // its slot_S / slot_R entry before it takes its ticket, and only the block that takes the last ticket reads them.  (The
 // probe ablation RWR_DEBUG_MODE=1 stores no row ends, so its k_cutrows_ws reads head unwritten: its sums mean nothing.)
+// The frontier workspace (fr, fw) of a run that may go sparse follows from the push-link budget; the bitmap in it is
+// set up by k_init, and the frontier kernels write every other entry before they read it.
 struct RunWorkspace {
-    Scratch<unsigned char> xa, xb, ya, yv;
+    Scratch<unsigned char> xa, xb, ya, yv, fr;
     Scratch<double> carry, head, slot_S, slot_R;
     Scratch<IterCtl> ctl;
+    FrontierWs fw;
     void* x[2] = {nullptr, nullptr};      // the two gather vectors: scratch, or the peer-mapped buffers of a partitioned graph
     // ya: the second rank vector of threshold mode and the probe's y (a fixed-count run into y_out leaves it unused)
+    // fr_budget: push links per sparse iteration (0: the run stays dense)
     template <typename T>
-    void alloc(rwr_graph* g, size_t ya_bytes) {
+    void alloc(rwr_graph* g, size_t ya_bytes, u64 fr_budget = 0) {
         const size_t vec_bytes = ((size_t)g->n + 8) * sizeof(T);
         if (g->p2p) {
             x[0] = g->px[0]; x[1] = g->px[1];
@@ -167,6 +181,8 @@ struct RunWorkspace {
         const size_t slots = (size_t)g->sm_count * 8 + 8;
         slot_S.alloc(&g->scratch, slots); slot_R.alloc(&g->scratch, slots);
         ctl.alloc(&g->scratch, 1);
+        if (fr_budget) fr.alloc(&g->scratch, frontier_carve(g, fr_budget, sizeof(T), nullptr, fw));
+        frontier_carve(g, fr_budget, sizeof(T), fr.p, fw);
     }
 };
 
@@ -262,7 +278,10 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
     const double S_uniform = (double)g->n_dangling + (double)(n - g->n_dangling) * (1.0 - omc_d);
     // r0 goes to y_out in fixed mode (also the answer for n_iter == 0); threshold mode ping-pongs ya <-> y_out
     T* r_cur = (mode == 0) ? y_out : ya;
-    k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform);
+    // single-seed fixed-count run: the first iterations may be pushed from the frontier (frontier.cu)
+    const bool fr_on = mode == 0 && ws.fw.budget > 0 && seed_orig >= 0;
+    k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform,
+                                                            fr_on ? ws.fw.bits : nullptr, ws.fw.words, seed_orig);
     KERNEL_CHECK();
     g->pool.launches += 1;
 
@@ -271,9 +290,11 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
     T* x_nxt = xb;
     int launched = 0;
     if (mode == 0) {
+        const int fr_iters = fr_on ? std::min(FR_ITERS, n_iter) : 0;
         auto launch_all = [&]() {
             for (int it = 0; it < n_iter; it++) {
-                p.x = x_cur; p.x_next = x_nxt; p.r_prev = nullptr; p.y = y_out;
+                p.x = x_cur; p.x_next = x_nxt; p.r_prev = nullptr; p.y = y_out; p.iter = it;
+                if (it < fr_iters) frontier_launch<T>(g, ws.fw, p, it + 1 < fr_iters);
                 set_peers<T>(g, p, x_nxt);
                 set_exchange<T>(g, p, x_nxt, it == 0, true);
                 launch_iteration<T>(g, p, /*resid=*/false, 0.0, 0);
@@ -282,9 +303,11 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
         };
         static const bool no_graph = getenv("RWR_NO_GRAPH") != nullptr;
         rwr_graph::IterGraph& ig = g->iter_graph[Prec<T>::id];
-        const void* key[8] = {xa, xb, y_out, ws.ctl.p, ws.head.p, ws.carry.p, ws.slot_S.p, ws.slot_R.p};
+        const u64 fr_budget = fr_on ? ws.fw.budget : 0;
+        const void* key[9] = {xa, xb, y_out, ws.ctl.p, ws.head.p, ws.carry.p, ws.slot_S.p, ws.slot_R.p, fr_on ? ws.fr.p : nullptr};
         const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1;
-        const bool same = ig.n_iter == n_iter && ig.hub == p.hub && ig.c == c && memcmp(ig.ptr, key, sizeof(key)) == 0;
+        const bool same = ig.n_iter == n_iter && ig.hub == p.hub && ig.c == c && ig.fr_budget == fr_budget &&
+                          memcmp(ig.ptr, key, sizeof(key)) == 0;
         if (graphable && same && (ig.exec || ig.seen)) {
             // second and later runs with this key: replay the graph of the whole loop (captured now if this is the second
             // run); nothing in it depends on the seed
@@ -303,16 +326,17 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
                 const cudaError_t err = cudaGraphInstantiate(&ig.exec, graph, 0);
                 cudaGraphDestroy(graph);
                 if (err != cudaSuccess) { ig.exec = nullptr; CUDA_CHECK(err); }
+                ig.launches = g->pool.launches - counted;
                 g->pool.launches = counted;
             }
             CUDA_CHECK(cudaGraphLaunch(ig.exec, st));
-            g->pool.launches += 3 * (int64_t)n_iter;
+            g->pool.launches += ig.launches;
         } else {
             // first run with this key (or no graph at all): launch kernel by kernel.  Capturing and instantiating costs more
             // than one run saves, and the reference asks each graph for a single recommendation (Experiment.cs:109).
             if (graphable) {
                 if (ig.exec) { cudaGraphExecDestroy(ig.exec); ig.exec = nullptr; }
-                ig.seen = true; ig.n_iter = n_iter; ig.hub = p.hub; ig.c = c;
+                ig.seen = true; ig.n_iter = n_iter; ig.hub = p.hub; ig.c = c; ig.fr_budget = fr_budget;
                 memcpy(ig.ptr, key, sizeof(key));
             }
             launch_all();
@@ -374,6 +398,15 @@ static void check_exchange_fault(rwr_graph* g, const IterCtl* ctl) {
     if (h.fault) RWR_FAIL(RWR_E_NCCL, "row-partitioned exchange: a peer's slice of x did not arrive in time (rank out of step or down)");
 }
 
+// probe RWR_FRONTIER_TRACE: how many iterations of the run just finished the frontier kernels did (host sync per seed)
+static void trace_frontier(rwr_graph* g, const RunWorkspace& ws, int seed_orig) {
+    IterCtl h{};
+    CUDA_CHECK(cudaMemcpyAsync(&h, ws.ctl.p, sizeof(h), cudaMemcpyDeviceToHost, g->stream));
+    CUDA_CHECK(cudaStreamSynchronize(g->stream));
+    fprintf(stderr, "[rwr frontier] seed %d: %d of %d iterations sparse (budget %llu links)\n", seed_orig, h.sparse_iters, h.iters,
+            (unsigned long long)ws.fw.budget);
+}
+
 template <typename T>
 static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_seeds, double c, int mode, int n_iter,
                     double thr, int max_iter, int32_t* iters_out) {
@@ -385,7 +418,7 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     if (Prec<T>::ybuf(res).n != std::max<size_t>(1, ld * (size_t)n_seeds))      // a re-run keeps its rank buffers
         Prec<T>::ybuf(res).alloc(std::max<size_t>(1, ld * (size_t)n_seeds), nullptr);
     RunWorkspace ws;
-    ws.alloc<T>(g, (n + 8) * sizeof(T));
+    ws.alloc<T>(g, (n + 8) * sizeof(T), mode == 0 ? frontier_budget(g) : 0);
     DevEvent ev0, ev1, evA, evB;
     const int64_t launches0 = g->pool.launches;
     CUDA_CHECK(cudaEventRecord(evA, st));
@@ -398,6 +431,7 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
         res->iters[s] = it;
         res->residual = rs;
         if (iters_out) iters_out[s] = it;
+        if (getenv("RWR_FRONTIER_TRACE")) trace_frontier(g, ws, seeds[s]);
     }
     CUDA_CHECK(cudaEventRecord(evB, st));
     CUDA_CHECK(cudaEventSynchronize(evB));
@@ -419,7 +453,8 @@ static void profile_impl(rwr_graph* g, int seed_orig, double c, int reps, float*
     T* ya = reinterpret_cast<T*>(ws.ya.p);
     p.r_prev = nullptr; p.y = ya;
     { const char* dm = getenv("RWR_DEBUG_MODE"); p.debug = dm ? atoi(dm) : 0; }
-    k_init<T><<<div_up(std::max((int)n, 1), 256), 256, 0, st>>>((int)n, p.seed, p.omc, p.inv, ya, xa, xb, ws.ctl.p, 0.0);
+    k_init<T><<<div_up(std::max((int)n, 1), 256), 256, 0, st>>>((int)n, p.seed, p.omc, p.inv, ya, xa, xb, ws.ctl.p, 0.0,
+                                                                    nullptr, 0u, -1);
     KERNEL_CHECK();
     std::vector<DevEvent> ev(3 * (size_t)reps);
     T* x_cur = xa;
@@ -457,7 +492,7 @@ void iterate_single_into(rwr_graph* g, int seed_orig, double c, int n_iter, T* y
                          cudaEvent_t ext0, cudaEvent_t ext1) {
     if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
     RunWorkspace ws;
-    ws.alloc<T>(g, 16);
+    ws.alloc<T>(g, 16, frontier_budget(g));
     const int64_t l0 = g->pool.launches;
     int it = 0;
     double rs = 0;

@@ -15,6 +15,8 @@ struct IterCtl {
     double red[2];     // row-partitioned graphs: this rank's {restart mass, residual} partials, summed over the ranks in place
     int fault;         // k_spmv_ws gave up waiting for a peer's slice (exchange timeout): the run is void
     unsigned long long wait_clk;   // probe (RWR_XCHG_TRACE): cycles the warps of k_spmv_ws spent waiting for slices, summed
+    int sparse;         // the run may still push from its frontier (frontier.cu); cleared for good once it goes dense
+    int sparse_iters;   // iterations done by the frontier kernels: the dense kernels of iteration `it` return when it < this
 };
 
 struct rwr_result {

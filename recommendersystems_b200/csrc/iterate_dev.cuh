@@ -34,6 +34,7 @@ struct IterParams {
     int hub;                // x entries staged in shared memory
     int n_hot;              // labels below: hot, L2-resident (evict-last); above: clustered cold nodes (streamed)
     int debug;              // measurement-only ablations (RWR_DEBUG_MODE, profile hook only)
+    int iter;               // iteration of the run this launch computes (0-based): skipped when the frontier kernels did it
     double* head_partial;   // [ws_tiles] sum of the first row of a tile when that row started in an earlier tile
     double* carry;          // [ws_tiles] sum of the open row at the end of a tile (row sums are double in both precisions)
     double* slot_S;         // [blocks of k_finish_ws] restart-mass partials

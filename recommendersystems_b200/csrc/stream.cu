@@ -734,7 +734,7 @@ __device__ __noinline__ void ws_push_slices(const IterParams<T>& p, unsigned cha
 template <typename T, bool VALUED, bool DBG, bool XWAIT>
 __global__ void __launch_bounds__(WsCfg<T, VALUED, XWAIT>::THREADS, 1) k_spmv_ws(const IterParams<T> p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    if (p.ctl->done) return;
+    if (p.ctl->done || p.iter < p.ctl->sparse_iters) return;
     u32 smem0;
     asm volatile("{ .reg .u64 t; cvta.to.shared.u64 t, %1; cvt.u32.u64 %0, t; }" : "=r"(smem0) : "l"(smem_raw));
     const u32 hub_addr = smem0 + WS_HDR;
@@ -950,7 +950,7 @@ __global__ void __launch_bounds__(WsCfg<T, VALUED, XWAIT>::THREADS, 1) k_spmv_ws
 // tile order and stored like any other row sum
 template <typename T>
 __global__ void __launch_bounds__(FIX_THREADS) k_cutrows_ws(const IterParams<T> p) {
-    if (p.ctl->done) return;
+    if (p.ctl->done || p.iter < p.ctl->sparse_iters) return;
     const int t = blockIdx.x * FIX_THREADS + threadIdx.x;
     if (t >= p.ws_tiles) return;
     const u32 meta = p.ws_tile[t];
@@ -977,7 +977,7 @@ __global__ void __launch_bounds__(FIN_THREADS) k_finish_ws(const IterParams<T> p
     __shared__ double scratch[2 * FIN_THREADS / 32];
     __shared__ int is_last;
     IterCtl* ctl = p.ctl;
-    if (ctl->done) return;
+    if (ctl->done || p.iter < ctl->sparse_iters) return;       // (done sparsely: frontier.cu)
     const double S = ctl->S;
     const int seed = ctl->seed;
     const T uni_add = (T)((seed < 0) ? S * p.inv_n : 0.0);
