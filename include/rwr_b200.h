@@ -169,6 +169,24 @@ int rwr_run_fixed(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c,
  * bitwise fixed point exists); iters_out[n_seeds] receives the number of deliverRanks() calls.            */
 int rwr_run_threshold(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, double thr,
                       int32_t max_iter, int32_t precision, int32_t* iters_out, rwr_result** out);
+/* ---- restart set: `Model.restart` (Model.cs:9) overwritten with a weighted node set, then run(int) / run(double) ----
+ * q = weights[k] at nodes[k] (original labels, distinct), 0 elsewhere; q is not normalised (Model.cs:92-93, :96-97 add
+ * `rank_restart * restart[r]` to every node r).  Personalized PageRank with a preference vector: a group of users, a
+ * session of items.  The initial rank:
+ *   RWR_INIT_UNIFORM  1 everywhere        (`new Model(graph, c)`, Model.cs:24, then restart overwritten)
+ *   RWR_INIT_NODE     N at init_node      (`new Model(graph, c, init_node)`, Model.cs:44, then restart overwritten)
+ *   RWR_INIT_RESTART  fl(N * q_i)         (for a one-hot q the same as RWR_INIT_NODE)
+ * init_node is read for RWR_INIT_NODE only.  The result holds one rank vector (seed slot 0); rwr_topk / rwr_rank_all
+ * exclude the union of the LIKE targets of the raw links of every listed node (Recommender.cs:20-24 for each of them;
+ * a listed node without links adds nothing).  RWR_E_INVALID: a NULL pointer, n_restart < 1, a node listed twice, a
+ * negative or non-finite weight, an unknown init; RWR_E_BADSEED: a node or init_node outside [0, N);
+ * RWR_E_UNSUPPORTED: a row-partitioned handle.  rwr_rerun_fixed does not take a restart-set result (RWR_E_INVALID).  */
+enum { RWR_INIT_UNIFORM = 0, RWR_INIT_NODE = 1, RWR_INIT_RESTART = 2 };
+int rwr_run_fixed_restart(rwr_graph* g, const int32_t* nodes, const double* weights, int32_t n_restart, int32_t init,
+                          int32_t init_node, double c, int32_t n_iter, int32_t precision, rwr_result** out);
+int rwr_run_threshold_restart(rwr_graph* g, const int32_t* nodes, const double* weights, int32_t n_restart, int32_t init,
+                              int32_t init_node, double c, double thr, int32_t max_iter, int32_t precision,
+                              int32_t* iters_out, rwr_result** out);
 /* the same Model re-run from the constructor state with other seeds (same count): rank buffers are reused, no
  * device allocation happens on the call.  The graph handle must still be alive.                             */
 int rwr_rerun_fixed(rwr_result* r, const int32_t* seeds, double c, int32_t n_iter);

@@ -6,10 +6,12 @@ extension must be built (`python -c "import __graft_entry__ as g; g.build()"`) a
 for anything that computes.
 """
 from .rwr import (Comm, EdgeType, Feature, ForwardLink, Graph, Methodology, Model, Node, NodeType, Recommender, RwrError,
-                  SynthSpec, FP32, FP64, evaluate, evaluate_users, methodology_masks, methodology_options, widen_float)
+                  SynthSpec, FP32, FP64, INIT_NODE, INIT_RESTART, INIT_UNIFORM, evaluate, evaluate_users, methodology_masks,
+                  methodology_options, run_fixed_restart, run_threshold_restart, widen_float)
 from . import _native
 from .ingest import EgoNetwork, load_ego_network, run_experiment
 
 __all__ = ["Comm", "EdgeType", "Feature", "ForwardLink", "Graph", "Methodology", "Model", "Node", "NodeType", "Recommender",
-           "RwrError", "SynthSpec", "FP32", "FP64", "evaluate", "evaluate_users", "methodology_masks", "methodology_options",
-           "widen_float", "_native", "EgoNetwork", "load_ego_network", "run_experiment"]
+           "RwrError", "SynthSpec", "FP32", "FP64", "INIT_NODE", "INIT_RESTART", "INIT_UNIFORM", "evaluate", "evaluate_users",
+           "methodology_masks", "methodology_options", "run_fixed_restart", "run_threshold_restart", "widen_float", "_native",
+           "EgoNetwork", "load_ego_network", "run_experiment"]

@@ -17,6 +17,7 @@ RWR_E_INVALID, RWR_E_BADSEED, RWR_E_ALREADY_BUILT, RWR_E_BADINDEX, RWR_E_NOT_BUI
 RWR_E_CUDA, RWR_E_NCCL, RWR_E_OOM, RWR_E_UNSUPPORTED = -6, -7, -8, -9
 FP64, FP32 = 0, 1
 LAYOUT_AUTO, LAYOUT_VALUED, LAYOUT_INDEX = 0, 1, 2
+INIT_UNIFORM, INIT_NODE, INIT_RESTART = 0, 1, 2
 
 
 class rwr_opts(C.Structure):
@@ -66,6 +67,8 @@ SYMBOLS = {
     "rwr_graph_destroy": (None, [_vp]),
     "rwr_run_fixed": (C.c_int, [_vp, _vp, _i32, _f64, _i32, _i32, _pp]),
     "rwr_run_threshold": (C.c_int, [_vp, _vp, _i32, _f64, _f64, _i32, _i32, _vp, _pp]),
+    "rwr_run_fixed_restart": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _f64, _i32, _i32, _pp]),
+    "rwr_run_threshold_restart": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _f64, _f64, _i32, _i32, _vp, _pp]),
     "rwr_rerun_fixed": (C.c_int, [_vp, _vp, _f64, _i32]),
     "rwr_result_get_info": (C.c_int, [_vp, C.POINTER(rwr_run_info)]),
     "rwr_scores": (C.c_int, [_vp, _i32, _vp]),

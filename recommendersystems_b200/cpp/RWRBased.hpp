@@ -180,17 +180,25 @@ class Model {                                                                   
 public:
     Graph* graph;
     std::vector<double> rank;
+    // Model.cs:9: e_seed, or 1/N everywhere.  A caller may overwrite it: a vector that differs from the constructor's runs
+    // as a restart set (its nonzeros, rwr_run_*_restart) from the constructor's initial rank
+    std::vector<double> restart;
     int nNodes;
     double dampingFactor;
     int nIterations = 0;            // deliverRanks() calls so far
 
     Model(Graph& graph, double dampingFactor) : graph(&graph), nNodes(graph.size()), dampingFactor(dampingFactor), seed_(-1) {
         rank.assign((size_t)nNodes, 1.0);                                                                // Model.cs:24
+        restart.assign((size_t)nNodes, 1.0 / nNodes);                                                    // Model.cs:25
     }
     Model(Graph& graph, double dampingFactor, int targetNode)
         : graph(&graph), nNodes(graph.size()), dampingFactor(dampingFactor), seed_(targetNode) {
         rank.assign((size_t)nNodes, 0.0);                                                                // Model.cs:44
-        if (targetNode >= 0 && targetNode < nNodes) rank[(size_t)targetNode] = nNodes;
+        restart.assign((size_t)nNodes, 0.0);                                                             // Model.cs:45-48
+        if (targetNode >= 0 && targetNode < nNodes) {
+            rank[(size_t)targetNode] = nNodes;
+            restart[(size_t)targetNode] = 1.0;
+        }
     }
     // a C# class variable is a reference: `new Model(graph, c, seed)` with `Graph* graph` reads the same here
     Model(Graph* graph, double dampingFactor) : Model(*graph, dampingFactor) {}
@@ -201,7 +209,13 @@ public:
     void run(int nIterations) {                                           // Model.cs:68-73; successive calls accumulate, as in the reference
         total_ += nIterations > 0 ? nIterations : 0;
         rwr_result* r = nullptr;
-        check(rwr_run_fixed(graph->handle(), &seed_, 1, dampingFactor, total_, RWR_FP64, &r));
+        std::vector<int32_t> nodes;
+        std::vector<double> weights;
+        if (restart_set(nodes, weights))
+            check(rwr_run_fixed_restart(graph->handle(), nodes.data(), weights.data(), (int32_t)nodes.size(), init_kind(), seed_,
+                                        dampingFactor, total_, RWR_FP64, &r));
+        else
+            check(rwr_run_fixed(graph->handle(), &seed_, 1, dampingFactor, total_, RWR_FP64, &r));
         fetch(r);
         this->nIterations = total_;
     }
@@ -210,10 +224,28 @@ private:
     void run_threshold(double thr) {
         rwr_result* r = nullptr;
         int32_t iters = 0;
-        check(rwr_run_threshold(graph->handle(), &seed_, 1, dampingFactor, thr, 0, RWR_FP64, &iters, &r));
+        std::vector<int32_t> nodes;
+        std::vector<double> weights;
+        if (restart_set(nodes, weights))
+            check(rwr_run_threshold_restart(graph->handle(), nodes.data(), weights.data(), (int32_t)nodes.size(), init_kind(), seed_,
+                                            dampingFactor, thr, 0, RWR_FP64, &iters, &r));
+        else
+            check(rwr_run_threshold(graph->handle(), &seed_, 1, dampingFactor, thr, 0, RWR_FP64, &iters, &r));
         fetch(r);
         nIterations = iters;
     }
+    // the nonzeros of `restart` when it differs from the constructor's vector; false: unchanged
+    bool restart_set(std::vector<int32_t>& nodes, std::vector<double>& weights) const {
+        if ((int)restart.size() != nNodes) throw ArgumentException("restart must hold one weight per node");
+        bool same = true;
+        for (int i = 0; i < nNodes && same; i++)
+            same = restart[(size_t)i] == (seed_ < 0 ? 1.0 / nNodes : (i == seed_ ? 1.0 : 0.0));
+        if (same) return false;
+        for (int i = 0; i < nNodes; i++)
+            if (restart[(size_t)i] != 0.0) { nodes.push_back(i); weights.push_back(restart[(size_t)i]); }
+        return true;
+    }
+    int32_t init_kind() const { return seed_ < 0 ? RWR_INIT_UNIFORM : RWR_INIT_NODE; }
     void fetch(rwr_result* r) {
         const int rc = rwr_scores(r, 0, rank.data());
         rwr_result_destroy(r);
@@ -261,6 +293,29 @@ public:
         List<KeyValuePair<long long, double>> topNRecommendation;
         for (int i = 0; i < count; i++) topNRecommendation.Add(KeyValuePair<long long, double>((long long)ids[i], scores[i]));
         return topNRecommendation;
+    }
+
+    // Not in the reference: the ranking for a weighted node set (a group of users, a session of items) from a Model whose
+    // `restart` is `weights` at `nodes`, initial rank fl(N * weight).  Candidates: the ITEM nodes none of the listed nodes
+    // has liked (Recommender.cs:20-24 for each), (score desc, id desc); topN > 0 keeps the first topN.
+    List<KeyValuePair<long long, double>> RecommendationForSet(const std::vector<int>& nodes, const std::vector<double>& weights,
+                                                               float dampingFactor, int nIteration, int topN = 0) {
+        if (nodes.size() != weights.size()) throw ArgumentException("one weight per node");
+        const std::vector<int32_t> n32(nodes.begin(), nodes.end());
+        rwr_result* r = nullptr;
+        check(rwr_run_fixed_restart(graph.handle(), n32.data(), weights.data(), (int32_t)n32.size(), RWR_INIT_RESTART, 0,
+                                    (double)dampingFactor, nIteration, RWR_FP64, &r));
+        const size_t cap = topN > 0 ? (size_t)topN : (size_t)graph.size();
+        std::vector<int64_t> ids(cap ? cap : 1);
+        std::vector<double> scores(cap ? cap : 1);
+        int64_t count = 0;
+        const int rc = rwr_rank_all(r, 0, ids.data(), scores.data(), (int64_t)cap, &count);
+        rwr_result_destroy(r);
+        check(rc);
+        if ((size_t)count > cap) count = (int64_t)cap;
+        List<KeyValuePair<long long, double>> recommendation;
+        for (int64_t i = 0; i < count; i++) recommendation.Add(KeyValuePair<long long, double>((long long)ids[(size_t)i], scores[(size_t)i]));
+        return recommendation;
     }
 
 private:

@@ -49,6 +49,31 @@ namespace Recommenders.RWRBased {
             return list;
         }
 
+        // Not in the reference: the ranking for a weighted node set -- a group of users, a session of items -- from a Model whose
+        // `restart` is `weights` at `nodes` (personalized PageRank with a preference vector), initial rank fl(N * weight).  The
+        // candidates are the ITEM nodes none of the listed nodes has liked (Recommender.cs:20-24 for each), (score desc, id desc);
+        // topN > 0 keeps the first topN.
+        public List<KeyValuePair<long, double>> RecommendationForSet(int[] nodes, double[] weights, float dampingFactor, int nIteration,
+                                                                     int topN = 0) {
+            double c = dampingFactor;
+            graph.RequireBuilt();
+            if (nodes == null || weights == null || nodes.Length != weights.Length) throw new ArgumentException("one weight per node");
+            ResultHandle res;
+            RwrNative.Check(RwrNative.rwr_run_fixed_restart(graph.handle, nodes, weights, nodes.Length, RwrNative.INIT_RESTART, 0, c,
+                                                            nIteration, RwrNative.FP64, out res));
+            using (res) {
+                int n = graph.size();
+                long cap = topN > 0 ? topN : n;
+                var ids = new long[cap]; var scores = new double[cap];
+                long count;
+                RwrNative.Check(RwrNative.rwr_rank_all(res, 0, ids, scores, cap, out count));
+                long m = Math.Min(count, cap);
+                var list = new List<KeyValuePair<long, double>>((int)m);
+                for (long i = 0; i < m; i++) list.Add(new KeyValuePair<long, double>(ids[i], scores[i]));
+                return list;
+            }
+        }
+
         // Not in the reference: n seeds at once through the SpMM tiles (Experiment-style evaluation of many users).
         public List<KeyValuePair<long, double>>[] RecommendationBatch(int[] users, float dampingFactor, int nIteration, int topN) {
             double c = dampingFactor;

@@ -82,6 +82,12 @@ namespace Recommenders.RWRBased.Native {
             int precision, out ResultHandle result);
         [DllImport(Lib)] public static extern int rwr_run_threshold(GraphHandle g, int[] seeds, int nSeeds, double c, double thr,
             int maxIter, int precision, int[] itersOut, out ResultHandle result);
+        // a restart set: Model.restart overwritten with weights at nodes (RWR_INIT_*: the initial rank)
+        public const int INIT_UNIFORM = 0, INIT_NODE = 1, INIT_RESTART = 2;
+        [DllImport(Lib)] public static extern int rwr_run_fixed_restart(GraphHandle g, int[] nodes, double[] weights, int nRestart, int init,
+            int initNode, double c, int nIter, int precision, out ResultHandle result);
+        [DllImport(Lib)] public static extern int rwr_run_threshold_restart(GraphHandle g, int[] nodes, double[] weights, int nRestart,
+            int init, int initNode, double c, double thr, int maxIter, int precision, int[] itersOut, out ResultHandle result);
         [DllImport(Lib)] public static extern int rwr_rerun_fixed(ResultHandle r, int[] seeds, double c, int nIter);
         [DllImport(Lib)] public static extern int rwr_result_get_info(ResultHandle r, out RwrRunInfo info);
         [DllImport(Lib)] public static extern int rwr_scores(ResultHandle r, int seedSlot, double[] outN);

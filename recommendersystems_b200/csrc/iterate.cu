@@ -7,14 +7,18 @@
 //   :103-108 updateRanks   rank <- next, next <- 0                          -> buffer swap (nothing to zero)
 //   :110-115 checkConvergence  sum |rank - next|                            -> fused into the epilogue
 //   :52-73   run() / run(double) / run(int)                                 -> rwr_run_threshold / rwr_run_fixed
+//   :9       `restart` overwritten by the caller (a weighted node set)      -> rwr_run_fixed_restart / rwr_run_threshold_restart
+//                                                                              (k_init_set, k_finish_set_ws)
 //
 // The iteration kernels live in stream.cu (K7: k_spmv_ws, k_cutrows_ws, k_finish_ws); this file holds the run modes,
 // K6 (k_init), the workspaces and the result handle.
+#include <algorithm>
 #include <cmath>
 
 #include "iterate.h"
 
 #include "iterate_dev.cuh"
+#include "primitives.cuh"
 #include "stream.h"
 #include "frontier.h"
 #include "dist.h"
@@ -47,6 +51,78 @@ __global__ void k_init(int n, int seed, T omc, const T* __restrict__ inv, T* __r
     r0[j] = r;
     x0[j] = mul_rn(rw, invj);
     if (j == seed) ctl->S = (invj == (T)0) ? (double)r : (double)sub_rn(r, rw);
+}
+
+// ---- restart sets: q over a node list, in internal labels (RestartSet, iterate_dev.cuh)
+// the bitmap of the listed nodes; lbl[k] = internal label of nodes[k]
+__global__ void k_restart_mark(const int32_t* __restrict__ nodes, int m, const int32_t* __restrict__ new_of_old,
+                               int32_t* __restrict__ lbl, u32* __restrict__ bits) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const int j = new_of_old[nodes[k]];
+    lbl[k] = j;
+    atomicOr(&bits[j >> 5], 1u << (j & 31));
+}
+__global__ void k_restart_popc(const u32* __restrict__ bits, int words, u32* __restrict__ cnt) {
+    const int w = blockIdx.x * blockDim.x + threadIdx.x;
+    if (w < words) cnt[w] = (u32)__popc(bits[w]);
+}
+// q in label order: member j is number word_base[j >> 5] + popc(bits below j) (the nodes are distinct)
+__global__ void k_restart_place(const int32_t* __restrict__ lbl, const double* __restrict__ weights, int m, const RestartSet rs,
+                                double* __restrict__ q) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const int j = lbl[k];
+    q[rs.word_base[j >> 5] + __popc(rs.bits[j >> 5] & ((1u << (j & 31)) - 1u))] = weights[k];
+}
+
+// K6 of a restart-set run: the initial rank of `init` (RWR_INIT_UNIFORM: 1 everywhere, Model.cs:24; RWR_INIT_NODE: N at the
+// internal label `node`, Model.cs:44; RWR_INIT_RESTART: fl(N q_i)) and x0.  S0 is set here for UNIFORM (S_uniform) and NODE;
+// k_restart_s0 sums it for RESTART.  No frontier: a restart-set run is dense from its first iteration.
+template <typename T>
+__global__ void k_init_set(int n, int init, int node, T omc, const T* __restrict__ inv, T* __restrict__ r0, T* __restrict__ x0,
+                           T* __restrict__ x1, IterCtl* ctl, double S_uniform, const RestartSet rs) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < 8) { x0[n + j] = (T)0; x1[n + j] = (T)0; }
+    if (j == 0) {
+        ctl->resid = 0.0; ctl->done = 0; ctl->iters = 0; ctl->ticket = 0; ctl->fault = 0; ctl->wait_clk = 0;
+        ctl->tile_ctr = 0;
+        ctl->seed = -1;
+        ctl->sparse = 0;
+        ctl->sparse_iters = 0;
+        if (init == RWR_INIT_UNIFORM) ctl->S = S_uniform;
+    }
+    if (j >= n) return;
+    T r = (T)0;
+    if (init == RWR_INIT_UNIFORM) {
+        r = (T)1;
+    } else if (init == RWR_INIT_NODE) {
+        r = (j == node) ? (T)n : (T)0;
+    } else {
+        const u32 word = rs.bits[j >> 5];
+        if ((word >> (j & 31)) & 1u)
+            r = (T)__dmul_rn((double)n, rs.q[rs.word_base[j >> 5] + __popc(word & ((1u << (j & 31)) - 1u))]);
+    }
+    const T invj = inv[j];
+    const T rw = mul_rn(omc, r);
+    r0[j] = r;
+    x0[j] = mul_rn(rw, invj);
+    if (init == RWR_INIT_NODE && j == node) ctl->S = (invj == (T)0) ? (double)r : (double)sub_rn(r, rw);
+}
+
+// S0 of RWR_INIT_RESTART: the restart mass of the listed nodes, in one block and a fixed order (reruns are bit-identical)
+template <typename T>
+__global__ void __launch_bounds__(FIN_THREADS) k_restart_s0(int n, T omc, const T* __restrict__ inv, const int32_t* __restrict__ lbl,
+                                                            const double* __restrict__ weights, int m, IterCtl* ctl) {
+    __shared__ double scratch[2 * FIN_THREADS / 32];
+    double a = 0.0, b = 0.0;
+    for (int k = threadIdx.x; k < m; k += FIN_THREADS) {
+        const T r = (T)__dmul_rn((double)n, weights[k]);
+        const T rw = mul_rn(omc, r);
+        a += (inv[lbl[k]] == (T)0) ? (double)r : (double)sub_rn(r, rw);
+    }
+    block_sum2<FIN_THREADS>(a, b, scratch);
+    if (threadIdx.x == 0) ctl->S = a;
 }
 
 __global__ void k_partition(const u32* __restrict__ in_ptr, int n, u32 nnz, int n_chunks, int2* __restrict__ part) {
@@ -133,11 +209,11 @@ template <> struct Prec<float> {
 
 // One iteration: K7 on this handle's stream, plus the exchange of a row-partitioned graph.
 template <typename T>
-static void launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr) {
+static void launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet* rs) {
     cudaStream_t st = g->stream;
     const bool parted = dist_n_ranks(g->comm) > 1;
     // on a row slice the convergence test needs the residual of all slices: it runs after the exchange
-    ws_launch_iteration<T>(g, p, resid, thr, parted ? 0 : use_thr);
+    ws_launch_iteration<T>(g, p, resid, thr, parted ? 0 : use_thr, rs);
     static const bool skip_exchange = getenv("RWR_DIST_SKIP") != nullptr;      // timing probe only: wrong results
     if (parted && !skip_exchange) {
         // x_next: pushed by the next k_spmv_ws while it gathers (overlapped exchange), or already in every peer's copy when
@@ -262,10 +338,22 @@ static IterParams<T> iter_params(rwr_graph* g, const RunWorkspace& ws, int seed_
     return p;
 }
 
-// Runs one seed.  mode 0: fixed n_iter; mode 1: threshold.  Final rank lands in y_out (internal labels).
+// The restart set of one rwr_run_*_restart call on the device, built by restart_prepare
+struct RestartDev {
+    Scratch<u32> bits, word_base;
+    Scratch<int32_t> nodes, lbl;
+    Scratch<double> w, q;
+    RestartSet rs{};
+    int init = RWR_INIT_RESTART;
+    int init_node = -1;       // internal label (RWR_INIT_NODE)
+};
+
+// Runs one seed (or the restart set `set`, seed_orig -1).  mode 0: fixed n_iter; mode 1: threshold.  Final rank lands in
+// y_out (internal labels).
 template <typename T>
 static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int mode, int n_iter, double thr, int max_iter,
-                    T* y_out, int* iters_out, double* resid_out, float* iter_ms, cudaEvent_t ev0, cudaEvent_t ev1) {
+                    T* y_out, int* iters_out, double* resid_out, float* iter_ms, cudaEvent_t ev0, cudaEvent_t ev1,
+                    const RestartDev* set = nullptr) {
     cudaStream_t st = g->stream;
     const int n = g->n;
     IterParams<T> p = iter_params<T>(g, ws, seed_orig, c);
@@ -279,11 +367,24 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
     // r0 goes to y_out in fixed mode (also the answer for n_iter == 0); threshold mode ping-pongs ya <-> y_out
     T* r_cur = (mode == 0) ? y_out : ya;
     // single-seed fixed-count run: the first iterations may be pushed from the frontier (frontier.cu)
-    const bool fr_on = mode == 0 && ws.fw.budget > 0 && seed_orig >= 0;
-    k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform,
-                                                            fr_on ? ws.fw.bits : nullptr, ws.fw.words, seed_orig);
-    KERNEL_CHECK();
-    g->pool.launches += 1;
+    const bool fr_on = mode == 0 && ws.fw.budget > 0 && seed_orig >= 0 && !set;
+    if (set) {
+        k_init_set<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, set->init, set->init_node, p.omc, p.inv, r_cur, xa, xb,
+                                                                   ws.ctl.p, S_uniform, set->rs);
+        KERNEL_CHECK();
+        g->pool.launches += 1;
+        if (set->init == RWR_INIT_RESTART) {
+            k_restart_s0<T><<<1, FIN_THREADS, 0, st>>>(n, p.omc, p.inv, set->lbl.p, set->w.p, set->rs.m, ws.ctl.p);
+            KERNEL_CHECK();
+            g->pool.launches += 1;
+        }
+    } else {
+        k_init<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, r_cur, xa, xb, ws.ctl.p, S_uniform,
+                                                                fr_on ? ws.fw.bits : nullptr, ws.fw.words, seed_orig);
+        KERNEL_CHECK();
+        g->pool.launches += 1;
+    }
+    const RestartSet* rs = set ? &set->rs : nullptr;
 
     CUDA_CHECK(cudaEventRecord(ev0, st));
     T* x_cur = xa;
@@ -297,7 +398,7 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
                 if (it < fr_iters) frontier_launch<T>(g, ws.fw, p, it + 1 < fr_iters);
                 set_peers<T>(g, p, x_nxt);
                 set_exchange<T>(g, p, x_nxt, it == 0, true);
-                launch_iteration<T>(g, p, /*resid=*/false, 0.0, 0);
+                launch_iteration<T>(g, p, /*resid=*/false, 0.0, 0, rs);
                 std::swap(x_cur, x_nxt);
             }
         };
@@ -305,7 +406,8 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
         rwr_graph::IterGraph& ig = g->iter_graph[Prec<T>::id];
         const u64 fr_budget = fr_on ? ws.fw.budget : 0;
         const void* key[9] = {xa, xb, y_out, ws.ctl.p, ws.head.p, ws.carry.p, ws.slot_S.p, ws.slot_R.p, fr_on ? ws.fr.p : nullptr};
-        const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1;
+        // a restart-set run launches kernel by kernel: the graphs are keyed for seeded and uniform runs only
+        const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1 && !set;
         const bool same = ig.n_iter == n_iter && ig.hub == p.hub && ig.c == c && ig.fr_budget == fr_budget &&
                           memcmp(ig.ptr, key, sizeof(key)) == 0;
         if (graphable && same && (ig.exec || ig.seen)) {
@@ -356,7 +458,7 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
                 p.x = x_cur; p.x_next = x_nxt; p.r_prev = r_cur; p.y = target;
                 set_peers<T>(g, p, x_nxt);
                 set_exchange<T>(g, p, x_nxt, launched == 0, true);
-                launch_iteration<T>(g, p, /*resid=*/true, thr, 1);
+                launch_iteration<T>(g, p, /*resid=*/true, thr, 1, rs);
                 std::swap(x_cur, x_nxt);
                 r_cur = target;
                 launched++;
@@ -399,17 +501,21 @@ static void check_exchange_fault(rwr_graph* g, const IterCtl* ctl) {
 }
 
 // probe RWR_FRONTIER_TRACE: how many iterations of the run just finished the frontier kernels did (host sync per seed)
-static void trace_frontier(rwr_graph* g, const RunWorkspace& ws, int seed_orig) {
+static void trace_frontier(rwr_graph* g, const RunWorkspace& ws, int seed_orig, const RestartDev* set) {
     IterCtl h{};
     CUDA_CHECK(cudaMemcpyAsync(&h, ws.ctl.p, sizeof(h), cudaMemcpyDeviceToHost, g->stream));
     CUDA_CHECK(cudaStreamSynchronize(g->stream));
-    fprintf(stderr, "[rwr frontier] seed %d: %d of %d iterations sparse (budget %llu links)\n", seed_orig, h.sparse_iters, h.iters,
-            (unsigned long long)ws.fw.budget);
+    if (set)
+        fprintf(stderr, "[rwr frontier] restart set of %d nodes: %d of %d iterations sparse (budget %llu links)\n", set->rs.m,
+                h.sparse_iters, h.iters, (unsigned long long)ws.fw.budget);
+    else
+        fprintf(stderr, "[rwr frontier] seed %d: %d of %d iterations sparse (budget %llu links)\n", seed_orig, h.sparse_iters, h.iters,
+                (unsigned long long)ws.fw.budget);
 }
 
 template <typename T>
 static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_seeds, double c, int mode, int n_iter,
-                    double thr, int max_iter, int32_t* iters_out) {
+                    double thr, int max_iter, int32_t* iters_out, const RestartDev* set) {
     cudaStream_t st = g->stream;
     const size_t n = (size_t)g->n;
     if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
@@ -418,7 +524,7 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     if (Prec<T>::ybuf(res).n != std::max<size_t>(1, ld * (size_t)n_seeds))      // a re-run keeps its rank buffers
         Prec<T>::ybuf(res).alloc(std::max<size_t>(1, ld * (size_t)n_seeds), nullptr);
     RunWorkspace ws;
-    ws.alloc<T>(g, (n + 8) * sizeof(T), mode == 0 ? frontier_budget(g) : 0);
+    ws.alloc<T>(g, (n + 8) * sizeof(T), (mode == 0 && !set) ? frontier_budget(g) : 0);
     DevEvent ev0, ev1, evA, evB;
     const int64_t launches0 = g->pool.launches;
     CUDA_CHECK(cudaEventRecord(evA, st));
@@ -427,11 +533,11 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
         int it = 0;
         double rs = NAN;
         run_one<T>(g, ws, seeds[s], c, mode, n_iter, thr, max_iter, Prec<T>::ybuf(res).p + (size_t)s * ld, &it, &rs,
-                   &res->iterate_ms, ev0, ev1);
+                   &res->iterate_ms, ev0, ev1, set);
         res->iters[s] = it;
         res->residual = rs;
         if (iters_out) iters_out[s] = it;
-        if (getenv("RWR_FRONTIER_TRACE")) trace_frontier(g, ws, seeds[s]);
+        if (getenv("RWR_FRONTIER_TRACE")) trace_frontier(g, ws, seeds[s], set);
     }
     CUDA_CHECK(cudaEventRecord(evB, st));
     CUDA_CHECK(cudaEventSynchronize(evB));
@@ -519,8 +625,63 @@ void iterate_single_into(rwr_graph* g, int seed_orig, double c, int n_iter, T* y
 template void iterate_single_into<double>(rwr_graph*, int, double, int, double*, float*, int64_t*, cudaEvent_t, cudaEvent_t);
 template void iterate_single_into<float>(rwr_graph*, int, double, int, float*, float*, int64_t*, cudaEvent_t, cudaEvent_t);
 
+// The arguments of rwr_run_*_restart: q = weights at nodes (original labels), the initial rank `init`
+struct RestartArgs {
+    const int32_t* nodes;
+    const double* weights;
+    int32_t m;
+    int32_t init;
+    int32_t init_node;
+};
+
+// the argument rules of the restart-set entry points (host only, before anything touches the device)
+static void restart_validate(const rwr_graph* g, const RestartArgs& a) {
+    if (!a.nodes || !a.weights) RWR_FAIL(RWR_E_INVALID, "restart set: NULL node list or weights");
+    if (a.m < 1) RWR_FAIL(RWR_E_INVALID, "restart set: %d nodes (at least one is needed)", a.m);
+    if (a.init != RWR_INIT_UNIFORM && a.init != RWR_INIT_NODE && a.init != RWR_INIT_RESTART)
+        RWR_FAIL(RWR_E_INVALID, "restart set: unknown init %d", a.init);
+    if (a.init == RWR_INIT_NODE && (a.init_node < 0 || a.init_node >= g->n))
+        RWR_FAIL(RWR_E_BADSEED, "restart set: init_node %d outside [0, %d)", a.init_node, g->n);
+    for (int32_t k = 0; k < a.m; k++) {
+        if (a.nodes[k] < 0 || a.nodes[k] >= g->n) RWR_FAIL(RWR_E_BADSEED, "restart set: node %d outside [0, %d)", a.nodes[k], g->n);
+        if (!std::isfinite(a.weights[k]) || a.weights[k] < 0.0)
+            RWR_FAIL(RWR_E_INVALID, "restart set: weight %g of node %d is negative or not finite", a.weights[k], a.nodes[k]);
+    }
+    std::vector<int32_t> sorted(a.nodes, a.nodes + a.m);
+    std::sort(sorted.begin(), sorted.end());
+    const auto dup = std::adjacent_find(sorted.begin(), sorted.end());
+    if (dup != sorted.end()) RWR_FAIL(RWR_E_INVALID, "restart set: node %d is listed twice", *dup);
+    if (dist_n_ranks(g->comm) > 1 || g->part_build) RWR_FAIL(RWR_E_UNSUPPORTED, "restart sets do not run on row-partitioned graphs");
+}
+
+// uploads the node list and the weights once and builds the bitmap, the word counts and q in internal labels
+static void restart_prepare(rwr_graph* g, const RestartArgs& a, RestartDev& d) {
+    cudaStream_t st = g->stream;
+    const int m = a.m, words = (g->n + 31) / 32;
+    d.nodes.alloc(&g->scratch, m); d.lbl.alloc(&g->scratch, m); d.w.alloc(&g->scratch, m); d.q.alloc(&g->scratch, m);
+    d.bits.alloc(&g->scratch, words); d.word_base.alloc(&g->scratch, (size_t)words + 1);
+    CUDA_CHECK(cudaMemcpyAsync(d.nodes.p, a.nodes, (size_t)m * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CUDA_CHECK(cudaMemcpyAsync(d.w.p, a.weights, (size_t)m * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_CHECK(cudaMemsetAsync(d.bits.p, 0, (size_t)words * sizeof(u32), st));
+    k_restart_mark<<<div_up(m, 256), 256, 0, st>>>(d.nodes.p, m, g->new_of_old.p, d.lbl.p, d.bits.p);
+    KERNEL_CHECK();
+    k_restart_popc<<<div_up(words, 256), 256, 0, st>>>(d.bits.p, words, d.word_base.p);
+    KERNEL_CHECK();
+    prim::exclusive_scan<u32>(d.word_base.p, d.word_base.p, words, d.word_base.p + words, st, &g->pool);
+    d.rs.bits = d.bits.p; d.rs.word_base = d.word_base.p; d.rs.q = d.q.p; d.rs.m = m; d.rs.words = words;
+    k_restart_place<<<div_up(m, 256), 256, 0, st>>>(d.lbl.p, d.w.p, m, d.rs, d.q.p);
+    KERNEL_CHECK();
+    g->pool.launches += 3;
+    d.init = a.init;
+    d.init_node = -1;
+    if (a.init == RWR_INIT_NODE)
+        CUDA_CHECK(cudaMemcpyAsync(&d.init_node, g->new_of_old.p + a.init_node, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+}
+
 static int run_entry(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, int mode, int32_t n_iter, double thr,
-                     int32_t max_iter, int32_t precision, int32_t* iters_out, rwr_result** out, rwr_result* reuse = nullptr) {
+                     int32_t max_iter, int32_t precision, int32_t* iters_out, rwr_result** out, rwr_result* reuse = nullptr,
+                     const RestartArgs* restart = nullptr) {
     rwr_result* res = nullptr;
     try {
         if (!out && !reuse) RWR_FAIL(RWR_E_INVALID, "out is NULL");
@@ -533,6 +694,9 @@ static int run_entry(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double
         if (!(c == c)) RWR_FAIL(RWR_E_INVALID, "c is NaN");
         for (int s = 0; s < n_seeds; s++)
             if (seeds[s] < -1 || seeds[s] >= g->n) RWR_FAIL(RWR_E_BADSEED, "seed %d outside [0, %d)", seeds[s], g->n);
+        if (restart) restart_validate(g, *restart);
+        if (reuse && !reuse->restart_nodes.empty())
+            RWR_FAIL(RWR_E_INVALID, "a restart-set result cannot be re-run with seeds: call rwr_run_*_restart again");
         CUDA_CHECK(cudaSetDevice(g->device));
         if (mode == 1 && !(thr > 0.0)) thr = (1.0 / 1.7976931348623157e308) * (double)g->n;   // Model.cs:53
         AllocStream alloc_on(g->stream);
@@ -545,8 +709,14 @@ static int run_entry(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double
         res->precision = precision;
         res->seeds.assign(seeds, seeds + n_seeds);
         res->iters.assign(n_seeds, 0);
-        if (precision == RWR_FP64) run_all<double>(g, res, seeds, n_seeds, c, mode, n_iter, thr, max_iter, iters_out);
-        else run_all<float>(g, res, seeds, n_seeds, c, mode, n_iter, thr, max_iter, iters_out);
+        RestartDev set;
+        if (restart) {
+            restart_prepare(g, *restart, set);
+            res->restart_nodes.assign(restart->nodes, restart->nodes + restart->m);
+        }
+        const RestartDev* sp = restart ? &set : nullptr;
+        if (precision == RWR_FP64) run_all<double>(g, res, seeds, n_seeds, c, mode, n_iter, thr, max_iter, iters_out, sp);
+        else run_all<float>(g, res, seeds, n_seeds, c, mode, n_iter, thr, max_iter, iters_out, sp);
         if (out) *out = res;
         return RWR_OK;
     } catch (const RwrError& e) {
@@ -569,6 +739,22 @@ int rwr_run_fixed(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c,
 int rwr_run_threshold(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, double thr, int32_t max_iter,
                       int32_t precision, int32_t* iters_out, rwr_result** out) {
     return run_entry(g, seeds, n_seeds, c, 1, 0, thr, max_iter, precision, iters_out, out);
+}
+
+// `model.restart = q; model.run(n)` with q = weights at nodes: a Model whose restart vector the caller overwrote
+int rwr_run_fixed_restart(rwr_graph* g, const int32_t* nodes, const double* weights, int32_t n_restart, int32_t init,
+                          int32_t init_node, double c, int32_t n_iter, int32_t precision, rwr_result** out) {
+    const int32_t none = -1;
+    const RestartArgs a{nodes, weights, n_restart, init, init_node};
+    return run_entry(g, &none, 1, c, 0, n_iter, 0.0, 0, precision, nullptr, out, nullptr, &a);
+}
+
+int rwr_run_threshold_restart(rwr_graph* g, const int32_t* nodes, const double* weights, int32_t n_restart, int32_t init,
+                              int32_t init_node, double c, double thr, int32_t max_iter, int32_t precision, int32_t* iters_out,
+                              rwr_result** out) {
+    const int32_t none = -1;
+    const RestartArgs a{nodes, weights, n_restart, init, init_node};
+    return run_entry(g, &none, 1, c, 1, 0, thr, max_iter, precision, iters_out, out, nullptr, &a);
 }
 
 // `new Model(graph, c, seed).run(n)` again on a live Model object: same graph, seed count and precision, the rank

@@ -25,6 +25,7 @@ struct rwr_result {
     int32_t n_seeds = 0;
     int32_t precision = RWR_FP64;
     std::vector<int32_t> seeds;        // original labels (-1: uniform restart)
+    std::vector<int32_t> restart_nodes; // restart-set run (rwr_run_*_restart): the listed nodes, original labels; else empty
     std::vector<int32_t> iters;
     double residual = 0.0;
     float iterate_ms = 0.f, total_ms = 0.f;

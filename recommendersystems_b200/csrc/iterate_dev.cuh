@@ -71,8 +71,20 @@ struct IterParams {
     int chk_pairs;          // compact blocks: vpair entries are < this
 };
 
+// The restart vector q of a restart-set run (rwr_run_fixed_restart / rwr_run_threshold_restart), in internal labels: bit i
+// of `bits` is set for the m rows with a listed weight; word_base[w] counts the members in the words before w, so the weight
+// of member i is q[word_base[i >> 5] + popc(bits[i >> 5] below bit i)] -- q holds the weights in label order.
+struct RestartSet {
+    const u32* bits;        // [words]
+    const u32* word_base;   // [words]
+    const double* q;        // [m]
+    int m;
+    int words;
+};
+
 // Checked build: an index outside its array leaves a code in IterCtl.fault (2 gather source, 3 row-sum store, 4 virtual row
-// of the epilogue) and the access is skipped; the run then fails with RWR_E_INVALID instead of corrupting memory.
+// of the epilogue, 5 restart-set bitmap word, 6 restart-set weight) and the access is skipped; the run then fails with
+// RWR_E_INVALID instead of corrupting memory.
 #ifdef RWR_CHECKED
 #define RWR_CHK(cond, ctl, code) ((cond) ? true : ((ctl)->fault = (code), false))
 #else

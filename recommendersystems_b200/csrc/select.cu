@@ -2,6 +2,7 @@
 //
 // Restates Recommenders/RWRBased/Recommender.cs:
 //   :19-24  exclusion list = targets of the seed's raw LIKE links            -> k_mark_excluded (bitmap)
+//           (a restart set: the union over its nodes)                        -> k_mark_excluded_set
 //   :27-31  candidates = ITEM nodes not excluded, as (node.id, rank[i])       -> filter inside the scan
 //   :34-38  order by score descending, ties by id descending                 -> 64-bit order-preserving score key, id
 //   :42-51  first topN of that order                                         -> k_topk_scan + k_topk_merge (k <= 16)
@@ -198,6 +199,25 @@ __global__ void k_mark_excluded(const int32_t* __restrict__ raw_dst, const u8* _
     }
 }
 
+// A restart set (rwr_run_*_restart): Recommender.cs:20-24 for each listed node, one warp per node -- the union of the
+// targets of their raw LIKE links
+__global__ void k_mark_excluded_set(const int32_t* __restrict__ raw_dst, const u8* __restrict__ raw_type, const u32* __restrict__ raw_ptr,
+                                    const int32_t* __restrict__ nodes /* original labels */, int m, const int32_t* __restrict__ new_of_old,
+                                    int n, u32* __restrict__ excl) {
+    const int k = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (k >= m) return;
+    const int node = nodes[k];
+    const u32 b = raw_ptr[node], e = raw_ptr[node + 1];
+    for (u32 i = b + lane; i < e; i += 32) {
+        if (raw_type[i] == RWR_EDGE_LIKE) {
+            const int32_t d = raw_dst[i];
+            if (d >= 0 && d < n) {
+                const int j = new_of_old[d];
+                atomicOr(&excl[j >> 5], 1u << (j & 31));
+            }
+        }
+    }
+}
 
 // ------------------------------------------------------------------------------------------------ top-k of a whole seed tile
 // The batched path keeps the ranks of B seeds row-major, Y[n, B].  Scanning one column at a time reads every 32-byte
@@ -415,6 +435,21 @@ static void mark_excluded(rwr_graph* g, int seed, u32* excl, size_t words) {
     g->pool.launches += 1;
 }
 
+// the exclusion bitmap of a result: its seed's LIKE targets, or the union over the nodes of a restart set
+static void mark_excluded_for(rwr_graph* g, const rwr_result* r, int slot, u32* excl, size_t words) {
+    if (r->restart_nodes.empty()) { mark_excluded(g, r->seeds[slot], excl, words); return; }
+    const int m = (int)r->restart_nodes.size();
+    Scratch<int32_t> nodes;
+    nodes.alloc(&g->scratch, m);
+    CUDA_CHECK(cudaMemcpyAsync(nodes.p, r->restart_nodes.data(), (size_t)m * sizeof(int32_t), cudaMemcpyHostToDevice, g->stream));
+    CUDA_CHECK(cudaMemsetAsync(excl, 0, words * sizeof(u32), g->stream));
+    k_mark_excluded_set<<<div_up((size_t)m * 32, 256), 256, 0, g->stream>>>(g->raw_dst.p, g->raw_type.p, g->raw_ptr.p, nodes.p, m,
+                                                                           g->new_of_old.p, g->n, excl);
+    KERNEL_CHECK();
+    CUDA_CHECK(cudaStreamSynchronize(g->stream));          // the host list is the caller's until the copy has run
+    g->pool.launches += 1;
+}
+
 // blocks of the top-k scans over a rank vector or a seed tile
 static int topk_grid(const rwr_graph* g) {
     return std::max(1, std::min(std::min(g->sm_count * 4, TOPK_MAX_GRID), (int)div_up((size_t)std::max(g->n, 1), TOPK_THREADS)));
@@ -484,14 +519,17 @@ static void ensure_items_by_id(rwr_graph* g) {
 }
 
 // Full ranking of one seed on the device; returns the candidate count, fills up to `cap` pairs on the host.
+// (rset: a restart-set result, whose exclusion is the union over its nodes; seed is then unused)
 template <typename T>
-static int64_t rank_all_one(rwr_graph* g, const T* y, int seed, int64_t* ids, double* scores, int64_t cap) {
+static int64_t rank_all_one(rwr_graph* g, const T* y, int seed, int64_t* ids, double* scores, int64_t cap,
+                            const rwr_result* rset = nullptr) {
     cudaStream_t st = g->stream;
     ensure_items_by_id(g);
     const size_t words = ((size_t)g->n + 31) / 32 + 1;
     DevBuf<u32> excl;
     excl.alloc(words);
-    mark_excluded(g, seed, excl.p, words);
+    if (rset) mark_excluded_for(g, rset, 0, excl.p, words);
+    else mark_excluded(g, seed, excl.p, words);
     const int m = g->n_items;
     DevBuf<u32> pos, total;
     pos.alloc(m); total.alloc(1);
@@ -533,19 +571,21 @@ int rwr_topk(rwr_result* r, int32_t k, int64_t* out_ids, double* out_scores, int
     CUDA_CHECK(cudaSetDevice(g->device));
     cudaStream_t st = g->stream;
     const int S = r->n_seeds;
+    const rwr_result* rset = r->restart_nodes.empty() ? nullptr : r;
     if (k > TOPK_MAX) {                                  // large k: truncate the full ranking
         for (int s = 0; s < S; s++) {
             int64_t cnt = (r->precision == RWR_FP64)
-                ? rank_all_one<double>(g, r->y64.p + (size_t)s * r->ld, r->seeds[s], out_ids + (size_t)s * k, out_scores + (size_t)s * k, k)
-                : rank_all_one<float>(g, r->y32.p + (size_t)s * r->ld, r->seeds[s], out_ids + (size_t)s * k, out_scores + (size_t)s * k, k);
+                ? rank_all_one<double>(g, r->y64.p + (size_t)s * r->ld, r->seeds[s], out_ids + (size_t)s * k, out_scores + (size_t)s * k, k, rset)
+                : rank_all_one<float>(g, r->y32.p + (size_t)s * r->ld, r->seeds[s], out_ids + (size_t)s * k, out_scores + (size_t)s * k, k, rset);
             out_counts[s] = (int32_t)std::min<int64_t>(cnt, k);
         }
         return RWR_OK;
     }
     TopkScratch ts(g, k, S);
     for (int s = 0; s < S; s++) {
-        if (r->precision == RWR_FP64) topk_one<double>(g, ts, s, r->y64.p + (size_t)s * r->ld, 1, r->seeds[s]);
-        else topk_one<float>(g, ts, s, r->y32.p + (size_t)s * r->ld, 1, r->seeds[s]);
+        if (rset) mark_excluded_for(g, r, s, ts.excl.p, ts.words);
+        if (r->precision == RWR_FP64) topk_one<double>(g, ts, s, r->y64.p + (size_t)s * r->ld, 1, r->seeds[s], rset != nullptr);
+        else topk_one<float>(g, ts, s, r->y32.p + (size_t)s * r->ld, 1, r->seeds[s], rset != nullptr);
     }
     ts.copy_out(st, out_ids, out_scores, out_counts);
     CUDA_CHECK(cudaStreamSynchronize(st));
@@ -560,9 +600,10 @@ int rwr_rank_all(rwr_result* r, int32_t seed_slot, int64_t* ids, double* scores,
     rwr_graph* g = r->g;
     CUDA_CHECK(cudaSetDevice(g->device));
     if (cap < 0) cap = 0;
+    const rwr_result* rset = r->restart_nodes.empty() ? nullptr : r;
     *count = (r->precision == RWR_FP64)
-        ? rank_all_one<double>(g, r->y64.p + (size_t)seed_slot * r->ld, r->seeds[seed_slot], ids, scores, cap)
-        : rank_all_one<float>(g, r->y32.p + (size_t)seed_slot * r->ld, r->seeds[seed_slot], ids, scores, cap);
+        ? rank_all_one<double>(g, r->y64.p + (size_t)seed_slot * r->ld, r->seeds[seed_slot], ids, scores, cap, rset)
+        : rank_all_one<float>(g, r->y32.p + (size_t)seed_slot * r->ld, r->seeds[seed_slot], ids, scores, cap, rset);
     return RWR_OK;
     RWR_API_END
 }

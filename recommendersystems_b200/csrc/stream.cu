@@ -1056,6 +1056,83 @@ __global__ void __launch_bounds__(FIN_THREADS) k_finish_ws(const IterParams<T> p
     }
 }
 
+// The epilogue of a restart-set run (rwr_run_*_restart): k_finish_ws with the sparse restart vector q of a RestartSet in
+// place of e_seed or 1/N, Model.cs:92-93 / :96-97 with `restart` = q.  A member row adds S * q_r in double and rounds once,
+// as the seed row adds S; its membership bit comes from one coalesced word per 32 rows, and q_r is read for member rows
+// only.  A separate kernel, so that the seeded and uniform instantiations stay exactly what they were.  BMODE 0 and 1 only:
+// a restart set never runs on a row-partitioned graph (no peers, no compact blocks, no allReduce of the sums).
+template <typename T, bool RESID, int BMODE>
+__global__ void __launch_bounds__(FIN_THREADS) k_finish_set_ws(const IterParams<T> p, double thr, int use_thr, const RestartSet rs) {
+    __shared__ double scratch[2 * FIN_THREADS / 32];
+    __shared__ int is_last;
+    IterCtl* ctl = p.ctl;
+    if (ctl->done || p.iter < ctl->sparse_iters) return;       // (done sparsely: frontier.cu)
+    const double S = ctl->S;
+    // the rows outside the set add `S * 0`: nothing, unless S is NaN or Inf (see k_finish_ws)
+    const bool poisoned = !((S * 0.0) == 0.0);
+    const u64 pol_first = policy_evict_first(), pol_last = policy_evict_last();
+    double accS = 0.0, accR = 0.0;
+    for (int row = p.row_begin + blockIdx.x * FIN_THREADS + threadIdx.x; row < p.row_end; row += gridDim.x * FIN_THREADS) {
+        T y;
+        if (BMODE == 1) {
+            const T* part = p.yv + (row - p.row_begin);
+            y = ld_stream(part, pol_first);
+            for (int b = 1; b < p.x_blocks; b++) y = add_rn(y, ld_stream(part + (size_t)b * (size_t)p.v_rows, pol_first));
+        } else {
+            y = ld_stream(p.y + row, pol_first);
+        }
+        const T invr = ld_stream(p.inv + row, pol_first);
+        const int w = row >> 5;
+        const u32 word = RWR_CHK(w < rs.words, ctl, 5) ? __ldg(rs.bits + w) : 0u;
+        if ((word >> (row & 31)) & 1u) {
+            const u32 k = __ldg(rs.word_base + w) + (u32)__popc(word & ((1u << (row & 31)) - 1u));
+            const double qr = RWR_CHK(k < (u32)rs.m, ctl, 6) ? __ldg(rs.q + k) : 0.0;
+            y = (T)__dadd_rn((double)y, __dmul_rn(S, qr));
+            p.y[row] = y;
+        } else if (poisoned) {
+            y = (T)(S * 0.0);
+            p.y[row] = y;
+        }
+        if (BMODE != 0) p.y[row] = y;
+        const T rw = mul_rn(p.omc, y);
+        // the next iteration gathers x_next: hot rows should still be in L2 then, cold rows are streamed
+        const T xn = mul_rn(rw, invr);
+        st_policy(p.x_next + row, xn, row < p.n_hot ? pol_last : pol_first);
+        accS += (invr == (T)0) ? (double)y : (double)sub_rn(y, rw);
+        if (RESID) {
+            const T rp = ld_stream(p.r_prev + row, pol_first);
+            accR += (double)((rp > y) ? sub_rn(rp, y) : sub_rn(y, rp));
+        }
+    }
+    block_sum2<FIN_THREADS>(accS, accR, scratch);
+    if (threadIdx.x == 0) {
+        p.slot_S[blockIdx.x] = accS;
+        p.slot_R[blockIdx.x] = accR;
+        __threadfence();
+        const unsigned tk = atomicAdd(&ctl->ticket, 1u);
+        is_last = (tk == gridDim.x - 1);
+    }
+    __syncthreads();
+    if (is_last) {
+        __threadfence();
+        double a = 0.0, b = 0.0;
+        for (int i = threadIdx.x; i < (int)gridDim.x; i += FIN_THREADS) {
+            a += __ldcg(p.slot_S + i);
+            b += __ldcg(p.slot_R + i);
+        }
+        __syncthreads();
+        block_sum2<FIN_THREADS>(a, b, scratch);
+        if (threadIdx.x == 0) {
+            ctl->iters += 1;
+            ctl->ticket = 0;
+            ctl->tile_ctr = 0;                            // the next k_spmv_ws hands its tiles out from the start
+            ctl->S = a;
+            ctl->resid = b;
+            if (use_thr && b < thr) ctl->done = 1;        // strict `<` (Model.cs:114)
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ launch
 int ws_main_grid(const rwr_graph* g) {
     return std::max(1, std::min(g->sm_count, (g->ws_tiles + WS_WARPS - 1) / WS_WARPS));
@@ -1096,8 +1173,21 @@ void ws_launch_spmv_only(rwr_graph* g, const IterParams<T>& p) {
     kern<<<ws_main_grid(g), threads, smem_launch, g->stream>>>(pv);
     KERNEL_CHECK();
 }
+// the epilogue of a restart-set run (never on a partitioned graph: no compact blocks)
 template <typename T>
-void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr) {
+static void launch_finish_set(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet& rs) {
+    const int grid = ws_fin_grid(g);
+    if (p.x_blocks > 1) {
+        if (resid) k_finish_set_ws<T, true, 1><<<grid, FIN_THREADS, 0, g->stream>>>(p, thr, use_thr, rs);
+        else k_finish_set_ws<T, false, 1><<<grid, FIN_THREADS, 0, g->stream>>>(p, thr, use_thr, rs);
+    } else {
+        if (resid) k_finish_set_ws<T, true, 0><<<grid, FIN_THREADS, 0, g->stream>>>(p, thr, use_thr, rs);
+        else k_finish_set_ws<T, false, 0><<<grid, FIN_THREADS, 0, g->stream>>>(p, thr, use_thr, rs);
+    }
+}
+
+template <typename T>
+void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet* rs) {
     if (p.x_blocks > 1) {
         IterParams<T> pv = p;
         pv.y = p.yv;
@@ -1107,7 +1197,9 @@ void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, dou
         IterParams<T> pf = p;
         pf.chk_pairs = g->v_compact;
         k_cutrows_ws<T><<<ws_fix_grid(g), FIX_THREADS, 0, g->stream>>>(pv);
-        if (p.compact) {
+        if (rs) {
+            launch_finish_set<T>(g, p, resid, thr, use_thr, *rs);
+        } else if (p.compact) {
             if (resid) k_finish_ws<T, true, 2><<<ws_fin_grid(g), FIN_THREADS, 0, g->stream>>>(pf, thr, use_thr);
             else k_finish_ws<T, false, 2><<<ws_fin_grid(g), FIN_THREADS, 0, g->stream>>>(pf, thr, use_thr);
         } else {
@@ -1121,22 +1213,23 @@ void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, dou
     pc.chk_y_begin = g->row_begin;
     pc.chk_y_end = g->row_end;
     k_cutrows_ws<T><<<ws_fix_grid(g), FIX_THREADS, 0, g->stream>>>(pc);
-    if (resid) k_finish_ws<T, true, 0><<<ws_fin_grid(g), FIN_THREADS, 0, g->stream>>>(p, thr, use_thr);
+    if (rs) launch_finish_set<T>(g, p, resid, thr, use_thr, *rs);
+    else if (resid) k_finish_ws<T, true, 0><<<ws_fin_grid(g), FIN_THREADS, 0, g->stream>>>(p, thr, use_thr);
     else k_finish_ws<T, false, 0><<<ws_fin_grid(g), FIN_THREADS, 0, g->stream>>>(p, thr, use_thr);
     KERNEL_CHECK();
 }
 template <typename T>
-void ws_launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr) {
+void ws_launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet* rs) {
     ws_launch_spmv_only<T>(g, p);
-    ws_launch_finish_only<T>(g, p, resid, thr, use_thr);
+    ws_launch_finish_only<T>(g, p, resid, thr, use_thr, rs);
     g->pool.launches += 3;
 }
-template void ws_launch_iteration<double>(rwr_graph*, const IterParams<double>&, bool, double, int);
-template void ws_launch_iteration<float>(rwr_graph*, const IterParams<float>&, bool, double, int);
+template void ws_launch_iteration<double>(rwr_graph*, const IterParams<double>&, bool, double, int, const RestartSet*);
+template void ws_launch_iteration<float>(rwr_graph*, const IterParams<float>&, bool, double, int, const RestartSet*);
 template void ws_launch_spmv_only<double>(rwr_graph*, const IterParams<double>&);
 template void ws_launch_spmv_only<float>(rwr_graph*, const IterParams<float>&);
-template void ws_launch_finish_only<double>(rwr_graph*, const IterParams<double>&, bool, double, int);
-template void ws_launch_finish_only<float>(rwr_graph*, const IterParams<float>&, bool, double, int);
+template void ws_launch_finish_only<double>(rwr_graph*, const IterParams<double>&, bool, double, int, const RestartSet*);
+template void ws_launch_finish_only<float>(rwr_graph*, const IterParams<float>&, bool, double, int, const RestartSet*);
 
 #ifdef RWR_PROFILE_CLOCKS
 extern "C" int rwr_debug_clocks_ws(unsigned long long* out16, int reset) {

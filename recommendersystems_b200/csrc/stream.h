@@ -23,14 +23,17 @@ constexpr size_t WS_HUB_AUTO_BYTES_FP32 = 163 * 1024;   // same, FP32: the 164 K
 static_assert(WS_R == 2, "ws_consume is written for two rounds (8 links per lane) per stage");
 
 template <typename T> struct IterParams;
+struct RestartSet;
 
 void stream_prepare(rwr_graph* g);               // builds ws_src / ws_val64 / ws_tile from the pull CSR
 int ws_hub_entries(const rwr_graph* g, int precision);
 int ws_main_grid(const rwr_graph* g);
 int ws_fix_grid(const rwr_graph* g);
 int ws_fin_grid(const rwr_graph* g);
-// one iteration = k_spmv_ws (row sums) + k_cutrows_ws (rows cut by a tile boundary) + k_finish_ws (fused epilogue)
+// one iteration = k_spmv_ws (row sums) + k_cutrows_ws (rows cut by a tile boundary) + k_finish_ws (fused epilogue); a
+// restart-set run (rs) gets the epilogue k_finish_set_ws
 template <typename T>
-void ws_launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr);
+void ws_launch_iteration(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet* rs = nullptr);
 template <typename T> void ws_launch_spmv_only(rwr_graph* g, const IterParams<T>& p);
-template <typename T> void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr);
+template <typename T>
+void ws_launch_finish_only(rwr_graph* g, const IterParams<T>& p, bool resid, double thr, int use_thr, const RestartSet* rs = nullptr);

@@ -18,6 +18,8 @@ import numpy as np
 from . import _native as N
 
 FP64, FP32 = N.FP64, N.FP32
+# initial rank of a restart-set run (include/rwr_b200.h RWR_INIT_*): 1 everywhere, N at one node, fl(N * q_i)
+INIT_UNIFORM, INIT_NODE, INIT_RESTART = N.INIT_UNIFORM, N.INIT_NODE, N.INIT_RESTART
 
 
 class NodeType(enum.IntEnum):      # Recommender.cs:4
@@ -388,8 +390,41 @@ def run_threshold(graph: Graph, seeds: Sequence[int], c: float, thr: float, max_
     return _Result(h, len(s), graph.size(), graph), it
 
 
+def _restart_args(nodes: Sequence[int], weights: Sequence[float]):
+    n = np.ascontiguousarray(nodes, np.int32)
+    w = np.ascontiguousarray(weights, np.float64)
+    if n.ndim != 1 or n.shape != w.shape:
+        raise ValueError("one weight per node")
+    return n, w
+
+
+def run_fixed_restart(graph: Graph, nodes: Sequence[int], weights: Sequence[float], c: float, n_iter: int,
+                      init: int = INIT_RESTART, init_node: int = 0, precision: int = FP64) -> _Result:
+    """`Model.restart` = `weights` at `nodes` (0 elsewhere, not normalised), then run(n_iter): a walk that restarts over a
+    weighted node set (personalized PageRank with a preference vector).  `init`: the initial rank, INIT_UNIFORM (1
+    everywhere), INIT_NODE (N at `init_node`) or INIT_RESTART (fl(N * weight)).  One rank vector (slot 0); its top-k and
+    ranking exclude the LIKE targets of every listed node."""
+    n, w = _restart_args(nodes, weights)
+    h = C.c_void_p()
+    _check(N.lib().rwr_run_fixed_restart(graph._h, _p(n), _p(w), len(n), int(init), int(init_node), float(c), int(n_iter),
+                                         precision, C.byref(h)))
+    return _Result(h, 1, graph.size(), graph)
+
+
+def run_threshold_restart(graph: Graph, nodes: Sequence[int], weights: Sequence[float], c: float, thr: float,
+                          max_iter: int = 0, init: int = INIT_RESTART, init_node: int = 0, precision: int = FP64):
+    """run_fixed_restart with Model.run(double threshold) (Model.cs:57-66) -> (result, iterations)."""
+    n, w = _restart_args(nodes, weights)
+    it = np.zeros(1, np.int32)
+    h = C.c_void_p()
+    _check(N.lib().rwr_run_threshold_restart(graph._h, _p(n), _p(w), len(n), int(init), int(init_node), float(c), float(thr),
+                                             int(max_iter), precision, _p(it), C.byref(h)))
+    return _Result(h, 1, graph.size(), graph), int(it[0])
+
+
 class Model:
-    """Model.cs:5-116.  `Model(graph, d)` = uniform restart, `Model(graph, d, targetNode)` = seeded."""
+    """Model.cs:5-116.  `Model(graph, d)` = uniform restart, `Model(graph, d, targetNode)` = seeded.  `restart` (Model.cs:9)
+    may be assigned an N-vector: every run then restarts over its nonzeros, from the constructor's initial rank."""
 
     def __init__(self, graph: Graph, dampingFactor: float, targetNode: Optional[int] = None, precision: int = FP64):
         self.graph = graph
@@ -402,29 +437,49 @@ class Model:
         self._res: Optional[_Result] = None
         self.residual = float("nan")
         self.nextRank = np.zeros(self.nNodes)         # Model.cs:8
+        self._restart: Optional[np.ndarray] = None    # None: the constructor's restart vector
 
     def _seed(self) -> int:
         return -1 if self.targetNode is None else int(self.targetNode)
+
+    def _set(self):
+        """the nonzeros of an assigned `restart` that differs from the constructor's, else None"""
+        if self._restart is None or np.array_equal(self._restart, self._constructor_restart()):
+            return None
+        nz = np.flatnonzero(self._restart)
+        return nz, self._restart[nz]
+
+    def _run_fixed(self, n_iter: int) -> _Result:
+        s = self._set()
+        if s is None:
+            return run_fixed(self.graph, [self._seed()], self.dampingFactor, n_iter, self.precision)
+        init = INIT_UNIFORM if self.targetNode is None else INIT_NODE
+        return run_fixed_restart(self.graph, s[0], s[1], self.dampingFactor, n_iter, init, max(self._seed(), 0), self.precision)
 
     def run(self, arg=None, max_iter: int = 0) -> None:
         """run(int nIterations) / run(double threshold) / run() -- Model.cs:68-73, :57-66, :52-55."""
         if isinstance(arg, (int, np.integer)) and not isinstance(arg, bool):
             # successive run(int) calls accumulate in the reference; re-run from the constructor state
             self._fixed_total += max(int(arg), 0)
-            self._res = run_fixed(self.graph, [self._seed()], self.dampingFactor, self._fixed_total, self.precision)
+            self._res = self._run_fixed(self._fixed_total)
             self.nIterations = self._fixed_total
             return
         if self._fixed_total:
             raise NotImplementedError("threshold run after run(int) on the same Model is not supported")
         thr = 0.0 if arg is None else float(arg)      # thr <= 0 selects Model.run(): (1/double.MaxValue) * N
-        self._res, it = run_threshold(self.graph, [self._seed()], self.dampingFactor, thr, max_iter, self.precision)
-        self.nIterations = int(it[0])
+        s = self._set()
+        if s is None:
+            self._res, it = run_threshold(self.graph, [self._seed()], self.dampingFactor, thr, max_iter, self.precision)
+            self.nIterations = int(it[0])
+        else:
+            init = INIT_UNIFORM if self.targetNode is None else INIT_NODE
+            self._res, self.nIterations = run_threshold_restart(self.graph, s[0], s[1], self.dampingFactor, thr, max_iter, init,
+                                                                max(self._seed(), 0), self.precision)
         self.residual = self._res.info().residual
 
     # -- the step methods of Model.cs:76-115.  Nobody in the reference calls them one by one; here each deliverRanks()
     #    re-runs the device loop from the constructor state (O(step) per call) so that the surface stays usable.
-    @property
-    def restart(self) -> np.ndarray:      # Model.cs:9, :25, :45-48
+    def _constructor_restart(self) -> np.ndarray:     # Model.cs:25, :45-48
         r = np.zeros(self.nNodes)
         if self.targetNode is None:
             r[:] = 1.0 / self.nNodes
@@ -432,15 +487,26 @@ class Model:
             r[self.targetNode] = 1.0
         return r
 
+    @property
+    def restart(self) -> np.ndarray:      # Model.cs:9
+        return self._constructor_restart() if self._restart is None else self._restart
+
+    @restart.setter
+    def restart(self, value) -> None:
+        r = np.array(value, np.float64)
+        if r.shape != (self.nNodes,):
+            raise ValueError(f"restart must hold {self.nNodes} weights")
+        self._restart = r
+
     def deliverRanks(self) -> None:
-        res = run_fixed(self.graph, [self._seed()], self.dampingFactor, self._fixed_total + 1, self.precision)
+        res = self._run_fixed(self._fixed_total + 1)
         self.nextRank = res.scores(0)
         res.close()
 
     def updateRanks(self) -> None:
         self._fixed_total += 1
         self.nIterations = self._fixed_total
-        self._res = run_fixed(self.graph, [self._seed()], self.dampingFactor, self._fixed_total, self.precision)
+        self._res = self._run_fixed(self._fixed_total)
         self.nextRank = np.zeros(self.nNodes)
 
     def checkConvergence(self, threshold: float) -> bool:
@@ -486,6 +552,25 @@ class Recommender:
                 m = int(cnt[0])
                 return list(zip(ids[0, :m].tolist(), sc[0, :m].tolist()))
             # 3-argument overload; the 4-argument one returns the whole list too when topN <= 0 (Recommender.cs:47)
+            ids, sc, _ = res.rank_all(0)
+            return list(zip(ids.tolist(), sc.tolist()))
+        finally:
+            res.close()
+
+    def RecommendationForSet(self, nodes: Sequence[int], weights: Sequence[float], dampingFactor: float, nIteration: int,
+                             topN: Optional[int] = None) -> List[Tuple[int, float]]:
+        """Not in the reference: the ranking for a weighted node set -- a group of users, a session of items -- from a Model
+        whose `restart` is `weights` at `nodes`, initial rank fl(N * weight).  The candidates are the ITEM nodes none of the
+        listed nodes has liked (Recommender.cs:20-24 for each of them), in the (score desc, id desc) order of
+        Recommender.cs:34-38; topN > 0 keeps the first topN.  `dampingFactor` is widened from float as in Recommendation."""
+        res = run_fixed_restart(self.graph, nodes, weights, widen_float(dampingFactor), int(nIteration), INIT_RESTART, 0,
+                                self.precision)
+        try:
+            self.last_info = res.info()
+            if topN is not None and topN > 0:
+                ids, sc, cnt = res.topk(int(topN))
+                m = int(cnt[0])
+                return list(zip(ids[0, :m].tolist(), sc[0, :m].tolist()))
             ids, sc, _ = res.rank_all(0)
             return list(zip(ids.tolist(), sc.tolist()))
         finally:
