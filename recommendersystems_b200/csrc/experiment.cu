@@ -270,45 +270,35 @@ extern "C" int rwr_graph_hold_out(rwr_graph* g, const int32_t* users, int32_t n_
     if (n_users == 0 || e0 == 0) return RWR_OK;
 
     DevBuf<int32_t> d_users;
-    DevBuf<u32> off, toff, total;
-    d_users.alloc(n_users); off.alloc((size_t)n_users + 1); toff.alloc((size_t)n_users + 1); total.alloc(1);
+    DevBuf<u32> off, toff;
+    d_users.alloc(n_users); off.alloc((size_t)n_users + 1); toff.alloc((size_t)n_users + 1);
     CUDA_CHECK(cudaMemcpyAsync(d_users.p, users, (size_t)n_users * 4, cudaMemcpyHostToDevice, st));
     const unsigned wgrid = grid_of((size_t)n_users * 32);
     k_ho_count<<<wgrid, 256, 0, st>>>(d_users.p, n_users, g->raw_ptr.p, g->raw_dst.p, g->raw_type.p, g->node_type.p, n, off.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(off.p, off.p, n_users, total.p, st, &g->pool);
-    u32 m32 = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&m32, total.p, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(off.p + n_users, total.p, 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    const size_t m = m32;
+    const size_t m = prim::scan_total<u32>(off.p, off.p, n_users, true, st, &g->pool);
     if (m == 0) return RWR_OK;
 
     // ---- (user slot, tweet id) order of the candidate likes: LSD sort by id, then a stable pass by slot
-    DevBuf<u64> k0, k1;
-    DevBuf<u32> v0, v1, link, slot, s0, s1, w0, w1;
-    k0.alloc(m); k1.alloc(m); v0.alloc(m); v1.alloc(m); link.alloc(m); slot.alloc(m);
+    prim::SortBuffers<u64> by_id;
+    DevBuf<u32> link, slot;
+    by_id.alloc(m, true); link.alloc(m); slot.alloc(m);
     k_ho_fill<<<wgrid, 256, 0, st>>>(d_users.p, n_users, g->raw_ptr.p, g->raw_dst.p, g->raw_type.p, g->node_type.p, g->node_id.p, n,
-                                     off.p, k0.p, v0.p, link.p, slot.p);
+                                     off.p, by_id.keys(), by_id.vals(), link.p, slot.p);
     KERNEL_CHECK();
-    const bool f1 = prim::radix_sort<u64>(k0.p, k1.p, v0.p, v1.p, m, 64, st, &g->pool);
-    const u32* perm1 = f1 ? v1.p : v0.p;
-    s0.alloc(m); s1.alloc(m); w0.alloc(m); w1.alloc(m);
-    k_ho_slot_keys<<<grid_of(m), 256, 0, st>>>(perm1, slot.p, m, s0.p);
+    by_id.sort(m, 64, st, &g->pool);
+    prim::SortBuffers<u32> by_slot;
+    by_slot.alloc(m, true);
+    k_ho_slot_keys<<<grid_of(m), 256, 0, st>>>(by_id.vals(), slot.p, m, by_slot.keys());
     KERNEL_CHECK();
-    CUDA_CHECK(cudaMemcpyAsync(w0.p, perm1, m * 4, cudaMemcpyDeviceToDevice, st));
-    const bool f2 = prim::radix_sort<u32>(s0.p, s1.p, w0.p, w1.p, m, std::max(1, ceil_log2_u64((u64)n_users)), st, &g->pool);
-    const u32* perm2 = f2 ? w1.p : w0.p;
+    CUDA_CHECK(cudaMemcpyAsync(by_slot.vals(), by_id.vals(), m * 4, cudaMemcpyDeviceToDevice, st));
+    by_slot.sort(m, std::max(1, ceil_log2_u64((u64)n_users)), st, &g->pool);
+    const u32* perm2 = by_slot.vals();
 
     // ---- fold windows -> test sets, removed flags, reverse links
     k_ho_tcount<<<grid_of(n_users), 256, 0, st>>>(off.p, n_users, n_folds, fold, toff.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(toff.p, toff.p, n_users, total.p, st, &g->pool);
-    u32 held32 = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&held32, total.p, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(toff.p + n_users, total.p, 4, cudaMemcpyDeviceToDevice, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    const size_t held = held32;
+    const size_t held = prim::scan_total<u32>(toff.p, toff.p, n_users, true, st, &g->pool);
     std::vector<u32> h_toff((size_t)n_users + 1);
     CUDA_CHECK(cudaMemcpyAsync(h_toff.data(), toff.p, ((size_t)n_users + 1) * 4, cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaStreamSynchronize(st));
@@ -362,10 +352,7 @@ extern "C" int rwr_graph_hold_out(rwr_graph* g, const int32_t* users, int32_t n_
     pos.alloc(e0);
     k_ho_keep_flags<<<grid_of(e0), 256, 0, st>>>(removed.p, e0, pos.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(pos.p, pos.p, e0, total.p, st, &g->pool);
-    u32 kept = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&kept, total.p, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    const u32 kept = prim::scan_total<u32>(pos.p, pos.p, e0, false, st, &g->pool);
     DevBuf<int32_t> src2, dst2;
     DevBuf<u8> type2;
     DevBuf<double> w2;

@@ -200,7 +200,7 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_expand(const FrDev d, const T
 }
 
 // ------------------------------------------------------------------------------------------------ radix sort
-// One stable 8-bit pass of an LSD sort over the sc[1] entries (the same scheme as prim::radix_sort, with the count on the
+// One stable 8-bit pass of an LSD sort over the sc[1] entries (the same scheme as prim::SortBuffers, with the count on the
 // device).  The digit table is digit-major over the tiles that hold entries.
 __global__ void __launch_bounds__(FR_THREADS) k_fr_hist(const FrDev d, const u32* __restrict__ keys, int shift) {
     __shared__ u32 h[256];

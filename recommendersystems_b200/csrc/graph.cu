@@ -447,6 +447,13 @@ void graph_init_device(rwr_graph* g, const rwr_opts* opts) {
     }
 }
 
+void graph_rebuild_raw_ptr(rwr_graph* g) {
+    g->raw_ptr.alloc((size_t)g->n + 1, &g->pool);
+    k_lower_bounds<int32_t><<<grid_for((size_t)g->n + 1), 256, 0, g->stream>>>(g->raw_src.p, (size_t)g->e0, g->n, g->raw_ptr.p);
+    KERNEL_CHECK();
+    CUDA_CHECK(cudaStreamSynchronize(g->stream));
+}
+
 // Canonicalise the raw links: stable sort by source when needed, then raw_ptr.
 void graph_finish_create(rwr_graph* g) {
     cudaStream_t st = g->stream;
@@ -464,30 +471,25 @@ void graph_finish_create(rwr_graph* g) {
     if (h[0]) RWR_FAIL(RWR_E_BADINDEX, "link source outside [0, %d)", g->n);
     if (h[1]) {
         // not source-ascending: stable sort by source keeps each source's insertion order
-        DevBuf<u32> keys, keys_alt, ord, ord_alt;
-        keys.alloc(e0); keys_alt.alloc(e0); ord.alloc(e0); ord_alt.alloc(e0);
-        CUDA_CHECK(cudaMemcpyAsync(keys.p, g->raw_src.p, e0 * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-        k_iota<<<grid_for(e0), 256, 0, st>>>(ord.p, e0);
+        prim::SortBuffers<u32> sb;
+        sb.alloc(e0, true);
+        CUDA_CHECK(cudaMemcpyAsync(sb.keys(), g->raw_src.p, e0 * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+        k_iota<<<grid_for(e0), 256, 0, st>>>(sb.vals(), e0);
         KERNEL_CHECK();
-        bool fl = prim::radix_sort<u32>(keys.p, keys_alt.p, ord.p, ord_alt.p, e0, ceil_log2_u64((u64)g->n), st, &g->pool);
-        u32* order = fl ? ord_alt.p : ord.p;
-        u32* sorted = fl ? keys_alt.p : keys.p;
+        sb.sort(e0, ceil_log2_u64((u64)g->n), st, &g->pool);
         DevBuf<int32_t> dst2; DevBuf<u8> type2; DevBuf<double> w2;
         dst2.alloc(e0, &g->pool); type2.alloc(e0, &g->pool); w2.alloc(e0, &g->pool);
-        k_gather<int32_t><<<grid_for(e0), 256, 0, st>>>(g->raw_dst.p, order, dst2.p, e0);
-        k_gather<u8><<<grid_for(e0), 256, 0, st>>>(g->raw_type.p, order, type2.p, e0);
-        k_gather<double><<<grid_for(e0), 256, 0, st>>>(g->raw_w.p, order, w2.p, e0);
+        k_gather<int32_t><<<grid_for(e0), 256, 0, st>>>(g->raw_dst.p, sb.vals(), dst2.p, e0);
+        k_gather<u8><<<grid_for(e0), 256, 0, st>>>(g->raw_type.p, sb.vals(), type2.p, e0);
+        k_gather<double><<<grid_for(e0), 256, 0, st>>>(g->raw_w.p, sb.vals(), w2.p, e0);
         KERNEL_CHECK();
-        CUDA_CHECK(cudaMemcpyAsync(g->raw_src.p, sorted, e0 * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(g->raw_src.p, sb.keys(), e0 * sizeof(u32), cudaMemcpyDeviceToDevice, st));
         CUDA_CHECK(cudaStreamSynchronize(st));
         g->raw_dst = std::move(dst2);
         g->raw_type = std::move(type2);
         g->raw_w = std::move(w2);
     }
-    g->raw_ptr.alloc((size_t)g->n + 1, &g->pool);
-    k_lower_bounds<int32_t><<<grid_for((size_t)g->n + 1), 256, 0, st>>>(g->raw_src.p, e0, g->n, g->raw_ptr.p);
-    KERNEL_CHECK();
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    graph_rebuild_raw_ptr(g);
 }
 
 // probe knob RWR_BUILD_TRACE=1: wall time of the build phases on stderr (each mark synchronises the stream)
@@ -505,13 +507,6 @@ struct BuildTrace {
         t0 = t1;
     }
 };
-
-void graph_rebuild_raw_ptr(rwr_graph* g) {
-    g->raw_ptr.alloc((size_t)g->n + 1, &g->pool);
-    k_lower_bounds<int32_t><<<grid_for((size_t)g->n + 1), 256, 0, g->stream>>>(g->raw_src.p, (size_t)g->e0, g->n, g->raw_ptr.p);
-    KERNEL_CHECK();
-    CUDA_CHECK(cudaStreamSynchronize(g->stream));
-}
 
 static void graph_build_impl(rwr_graph* g) {
     if (g->built) RWR_FAIL(RWR_E_ALREADY_BUILT, "buildGraph() called twice (ArgumentException at Graph.cs:86)");
@@ -538,9 +533,8 @@ static void graph_build_impl(rwr_graph* g) {
 
     BuildTrace trace(st, dist_rank(g->comm));
     // ---- K1 + K2: explicit flags, exclusive scan
-    DevBuf<u32> pos, total;
+    DevBuf<u32> pos;
     pos.alloc(e0);
-    total.alloc(1);
     DevBuf<u8> carrier;                    // sources that hold an explicit link of a type outside zero_weight_type_mask
     const u32 zero_mask = (u32)g->opts.zero_weight_type_mask;
     if (e0) {
@@ -554,14 +548,10 @@ static void graph_build_impl(rwr_graph* g) {
                                                       zero_mask, carrier.p, pos.p, bad.p);
         KERNEL_CHECK();
     }
-    prim::exclusive_scan<u32>(pos.p, pos.p, e0, total.p, st, &g->pool);
-    u32 h_total = 0;
     int h_bad = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&h_total, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));   // complete once the scan returns
+    const size_t nnz = prim::scan_total<u32>(pos.p, pos.p, e0, false, st, &g->pool);
     if (h_bad) RWR_FAIL(RWR_E_BADINDEX, "link target outside [0, %d) (IndexOutOfRangeException at Model.cs:87)", n);
-    const size_t nnz = h_total;
     g->nnz = (int64_t)nnz;
 
     // ---- K3: stable scatter (skipped when no UNDEFINED link exists: the raw arrays already are the CSR)
@@ -621,11 +611,9 @@ static void graph_build_impl(rwr_graph* g) {
     }
     if (pb) {
         // deg[n] carries "this rank saw a row with unequal weights"
-        const u32 nonuni = 0;
         CUDA_CHECK(cudaMemcpyAsync(&hs, stats.p, sizeof(hs), cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaStreamSynchronize(st));
         const u32 flag = hs.all_uniform ? 0u : 1u;
-        (void)nonuni;
         CUDA_CHECK(cudaMemcpyAsync(deg.p + n, &flag, sizeof(u32), cudaMemcpyHostToDevice, st));
         dist_allreduce_sum(g, deg.p, (size_t)n + 1, DIST_U32);
         dist_allreduce_sum(g, first_nb.p, (size_t)n, DIST_U32);
@@ -676,34 +664,33 @@ static void graph_build_impl(rwr_graph* g) {
     g->relabelled = (g->opts.relabel == 0) && n > 1;
     g->n_hot = n;
     if (g->relabelled) {
-        DevBuf<u32> k0, k1, v0, v1;
-        k0.alloc(n); k1.alloc(n); v0.alloc(n); v1.alloc(n);
-        k_degree_keys<<<grid_for(n), 256, 0, st>>>(deg.p, n, hs.max_out, k0.p, v0.p);
+        prim::SortBuffers<u32> sb;
+        sb.alloc(n, true);
+        k_degree_keys<<<grid_for(n), 256, 0, st>>>(deg.p, n, hs.max_out, sb.keys(), sb.vals());
         KERNEL_CHECK();
-        bool fl = prim::radix_sort<u32>(k0.p, k1.p, v0.p, v1.p, n, ceil_log2_u64((u64)hs.max_out + 1), st, &g->pool);
-        k_invert_perm<<<grid_for(n), 256, 0, st>>>(fl ? v1.p : v0.p, n, g->old_of_new.p, g->new_of_old.p);
+        sb.sort(n, ceil_log2_u64((u64)hs.max_out + 1), st, &g->pool);
+        k_invert_perm<<<grid_for(n), 256, 0, st>>>(sb.vals(), n, g->old_of_new.p, g->new_of_old.p);
         KERNEL_CHECK();
         const u32 hot_min = g->opts.hot_min_degree > 0 ? (u32)g->opts.hot_min_degree : 8u;   // profiles/microbench/hotmin_sweep.py
         if (hot_min > 1) {
-            DevBuf<u32> counts, pos, total;
-            counts.alloc(2); pos.alloc(n); total.alloc(1);
+            DevBuf<u32> counts, pos;
+            counts.alloc(2); pos.alloc(n);
             CUDA_CHECK(cudaMemsetAsync(counts.p, 0, 2 * sizeof(u32), st));
             k_cold_flags<<<grid_for(n), 256, 0, st>>>(deg.p, n, hot_min, pos.p, counts.p);
             KERNEL_CHECK();
-            prim::exclusive_scan<u32>(pos.p, pos.p, n, total.p, st, &g->pool);
-            u32 hc[2] = {0, 0}, n_cold = 0;
-            CUDA_CHECK(cudaMemcpyAsync(hc, counts.p, sizeof(hc), cudaMemcpyDeviceToHost, st));
-            CUDA_CHECK(cudaMemcpyAsync(&n_cold, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            CUDA_CHECK(cudaStreamSynchronize(st));
+            u32 hc[2] = {0, 0};
+            CUDA_CHECK(cudaMemcpyAsync(hc, counts.p, sizeof(hc), cudaMemcpyDeviceToHost, st));   // complete once the scan returns
+            const u32 n_cold = prim::scan_total<u32>(pos.p, pos.p, n, false, st, &g->pool);
             const u32 n_hot = hc[0];
             g->n_hot = (int32_t)n_hot;
             if (n_cold) {
-                DevBuf<u32> ck0, ck1, cv0, cv1;
-                ck0.alloc(n_cold); ck1.alloc(n_cold); cv0.alloc(n_cold); cv1.alloc(n_cold);
-                k_cold_keys<<<grid_for(n), 256, 0, st>>>(deg.p, first_nb.p, g->new_of_old.p, n, hot_min, n_hot, pos.p, ck0.p, cv0.p);
+                prim::SortBuffers<u32> cold;
+                cold.alloc(n_cold, true);
+                k_cold_keys<<<grid_for(n), 256, 0, st>>>(deg.p, first_nb.p, g->new_of_old.p, n, hot_min, n_hot, pos.p, cold.keys(),
+                                                         cold.vals());
                 KERNEL_CHECK();
-                bool f2 = prim::radix_sort<u32>(ck0.p, ck1.p, cv0.p, cv1.p, n_cold, ceil_log2_u64((u64)n_hot + (u64)n + 1), st, &g->pool);
-                k_assign_cold<<<grid_for(n_cold), 256, 0, st>>>(f2 ? cv1.p : cv0.p, n_cold, n_hot, g->new_of_old.p, g->old_of_new.p);
+                cold.sort(n_cold, ceil_log2_u64((u64)n_hot + (u64)n + 1), st, &g->pool);
+                k_assign_cold<<<grid_for(n_cold), 256, 0, st>>>(cold.vals(), n_cold, n_hot, g->new_of_old.p, g->old_of_new.p);
                 KERNEL_CHECK();
             }
         }
@@ -757,18 +744,16 @@ static void graph_build_impl(rwr_graph* g) {
         g->in_src.alloc(nnz + IDX_PAD, &g->pool);
         CUDA_CHECK(cudaMemsetAsync(g->in_src.p, 0, (nnz + IDX_PAD) * sizeof(int32_t), st));
         if (layout == RWR_LAYOUT_VALUED) g->in_val64.alloc(nnz + IDX_PAD, &g->pool);   // k_spmm reads whole groups of 4
-        DevBuf<u32> k0, k1, v0, v1;
-        k0.alloc(nnz); k1.alloc(nnz); v0.alloc(nnz); v1.alloc(nnz);
+        prim::SortBuffers<u32> sb;
+        sb.alloc(nnz, true);
         if (nnz) {
-            k_transpose_keys<<<grid_for(nnz), 256, 0, st>>>(g->col, g->new_of_old.p, nnz, k0.p, v0.p);
+            k_transpose_keys<<<grid_for(nnz), 256, 0, st>>>(g->col, g->new_of_old.p, nnz, sb.keys(), sb.vals());
             KERNEL_CHECK();
         }
-        bool fl = prim::radix_sort<u32>(k0.p, k1.p, v0.p, v1.p, nnz, ceil_log2_u64((u64)n), st, &g->pool);
-        const u32* sorted = fl ? k1.p : k0.p;
-        const u32* order = fl ? v1.p : v0.p;
-        k_lower_bounds<u32><<<grid_for((size_t)n + 1), 256, 0, st>>>(sorted, nnz, n, g->in_ptr.p);
+        sb.sort(nnz, ceil_log2_u64((u64)n), st, &g->pool);
+        k_lower_bounds<u32><<<grid_for((size_t)n + 1), 256, 0, st>>>(sb.keys(), nnz, n, g->in_ptr.p);
         if (nnz)
-            k_fill_pull<<<grid_for(nnz), 256, 0, st>>>(order, g->src_of, g->new_of_old.p, g->val.p, nnz, g->in_src.p,
+            k_fill_pull<<<grid_for(nnz), 256, 0, st>>>(sb.vals(), g->src_of, g->new_of_old.p, g->val.p, nnz, g->in_src.p,
                                                       layout == RWR_LAYOUT_VALUED ? g->in_val64.p : nullptr);
         KERNEL_CHECK();
         CUDA_CHECK(cudaStreamSynchronize(st));
@@ -789,15 +774,15 @@ static void graph_build_impl(rwr_graph* g) {
         send_pairs.alloc(nnz);
         if (valued) send_val.alloc(nnz);
         {
-            DevBuf<u32> k0, k1, v0, v1;
-            k0.alloc(nnz); k1.alloc(nnz); v0.alloc(nnz); v1.alloc(nnz);
+            prim::SortBuffers<u32> sb;
+            sb.alloc(nnz, true);
             if (nnz) {
-                k_dest_keys<<<grid_for(nnz), 256, 0, st>>>(g->col, g->new_of_old.p, nnz, parts, d_rows.p, k0.p, v0.p, d_cnt.p);
+                k_dest_keys<<<grid_for(nnz), 256, 0, st>>>(g->col, g->new_of_old.p, nnz, parts, d_rows.p, sb.keys(), sb.vals(), d_cnt.p);
                 KERNEL_CHECK();
             }
-            const bool fl = prim::radix_sort<u32>(k0.p, k1.p, v0.p, v1.p, nnz, std::max(1, ceil_log2_u64((u64)parts)), st, &g->pool);
+            sb.sort(nnz, std::max(1, ceil_log2_u64((u64)parts)), st, &g->pool);
             if (nnz) {
-                k_pack_links<<<grid_for(nnz), 256, 0, st>>>(fl ? v1.p : v0.p, g->col, g->src_of, g->new_of_old.p, g->val.p, nnz,
+                k_pack_links<<<grid_for(nnz), 256, 0, st>>>(sb.vals(), g->col, g->src_of, g->new_of_old.p, g->val.p, nnz,
                                                            send_pairs.p, valued ? send_val.p : nullptr);
                 KERNEL_CHECK();
             }
@@ -841,23 +826,18 @@ static void graph_build_impl(rwr_graph* g) {
         CUDA_CHECK(cudaMemsetAsync(g->in_src.p, 0, (m + IDX_PAD) * sizeof(int32_t), st));
         if (valued) g->in_val64.alloc(m + IDX_PAD, &g->pool);
         {
-            DevBuf<u32> k0, k1, v0, v1;
-            k0.alloc(m); k1.alloc(m); v0.alloc(m); v1.alloc(m);
-            if (m) k_pair_field<<<grid_for(m), 256, 0, st>>>(recv_pairs.p, nullptr, m, 1, k0.p, v0.p);
+            prim::SortBuffers<u32> sb;
+            sb.alloc(m, true);
+            if (m) k_pair_field<<<grid_for(m), 256, 0, st>>>(recv_pairs.p, nullptr, m, 1, sb.keys(), sb.vals());
             KERNEL_CHECK();
-            const bool f1 = prim::radix_sort<u32>(k0.p, k1.p, v0.p, v1.p, m, ceil_log2_u64((u64)n), st, &g->pool);
-            u32* ord1 = f1 ? v1.p : v0.p;
-            u32* ord_alt = f1 ? v0.p : v1.p;
-            u32* kk = f1 ? k0.p : k1.p;         // the key buffer that does not hold the sorted keys: reuse for the target keys
-            u32* kk_alt = f1 ? k1.p : k0.p;
-            if (m) k_pair_field<<<grid_for(m), 256, 0, st>>>(recv_pairs.p, ord1, m, 0, kk, nullptr);
+            sb.sort(m, ceil_log2_u64((u64)n), st, &g->pool);
+            u32* target_keys = sb.rekey();
+            if (m) k_pair_field<<<grid_for(m), 256, 0, st>>>(recv_pairs.p, sb.vals(), m, 0, target_keys, nullptr);
             KERNEL_CHECK();
-            const bool f2 = prim::radix_sort<u32>(kk, kk_alt, ord1, ord_alt, m, ceil_log2_u64((u64)n), st, &g->pool);
-            const u32* sorted = f2 ? kk_alt : kk;
-            const u32* order = f2 ? ord_alt : ord1;
-            k_lower_bounds<u32><<<grid_for((size_t)n + 1), 256, 0, st>>>(sorted, m, n, g->in_ptr.p);
+            sb.sort(m, ceil_log2_u64((u64)n), st, &g->pool);
+            k_lower_bounds<u32><<<grid_for((size_t)n + 1), 256, 0, st>>>(sb.keys(), m, n, g->in_ptr.p);
             if (m)
-                k_fill_pull_recv<<<grid_for(m), 256, 0, st>>>(order, recv_pairs.p, valued ? recv_val.p : nullptr, g->new_of_old.p, m,
+                k_fill_pull_recv<<<grid_for(m), 256, 0, st>>>(sb.vals(), recv_pairs.p, valued ? recv_val.p : nullptr, g->new_of_old.p, m,
                                                              g->in_src.p, valued ? g->in_val64.p : nullptr);
             KERNEL_CHECK();
             CUDA_CHECK(cudaStreamSynchronize(st));

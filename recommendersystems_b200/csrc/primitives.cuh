@@ -74,12 +74,18 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_apply(const InT* __r
     }
 }
 
-// out[i] = sum(in[0..i)), out may alias in when InT is u32; optional total (device pointer) = sum of all.
+// out[i] = sum(in[0..i)), out may alias in when InT is u32; optional total (device pointer) = sum of all, and with
+// total_host (which needs total_dev) a copy of it on the host, enqueued before the final synchronisation.
 // Temp memory is allocated internally (tile sums, a few hundred KB at most).
 template <typename InT>
-inline void exclusive_scan(const InT* in, u32* out, size_t n, u32* total_dev, cudaStream_t st, DevPool* pool) {
+inline void exclusive_scan(const InT* in, u32* out, size_t n, u32* total_dev, cudaStream_t st, DevPool* pool,
+                           u32* total_host = nullptr) {
     if (n == 0) {
         if (total_dev) CUDA_CHECK(cudaMemsetAsync(total_dev, 0, sizeof(u32), st));
+        if (total_host) {
+            *total_host = 0;
+            CUDA_CHECK(cudaStreamSynchronize(st));
+        }
         return;
     }
     size_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
@@ -98,7 +104,19 @@ inline void exclusive_scan(const InT* in, u32* out, size_t n, u32* total_dev, cu
     k_scan_tile_apply<InT><<<(unsigned)tiles, SCAN_THREADS, 0, st>>>(in, out, sums.p, n);
     KERNEL_CHECK();
     if (pool) pool->launches++;
+    if (total_host) CUDA_CHECK(cudaMemcpyAsync(total_host, total_dev, sizeof(u32), cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaStreamSynchronize(st));   // `sums` is freed on return
+}
+
+// The scan for a caller that needs the total on the host: returns it, after the stream has synchronised.  With `csr`,
+// out holds n + 1 words and out[n] receives the total as well (CSR offsets).
+template <typename InT>
+inline u32 scan_total(const InT* in, u32* out, size_t n, bool csr, cudaStream_t st, DevPool* pool) {
+    DevBuf<u32> word;
+    if (!csr) word.alloc(1);
+    u32 total = 0;
+    exclusive_scan<InT>(in, out, n, csr ? out + n : word.p, st, pool, &total);
+    return total;
 }
 
 // ======================================================================================= LSD radix sort
@@ -178,35 +196,51 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const KeyT* __restric
     }
 }
 
-// Sorts `n` (< 2^32) keys ascending on bits [0, end_bit), stable.  keys/vals are ping-ponged with the alt buffers;
-// returns true when the result ended up in the alt buffers.
+// The buffers of a stable radix sort: two for the keys and, for a sort that carries u32 values, two for the values.
+// sort() ping-pongs between each pair; keys() and vals() are the current buffers, which hold the result after a sort.
 template <typename KeyT>
-inline bool radix_sort(KeyT* keys, KeyT* keys_alt, u32* vals, u32* vals_alt, size_t n, int end_bit, cudaStream_t st,
-                       DevPool* pool) {
-    if (n == 0 || end_bit <= 0) return false;
-    if (n >= (1ULL << 32)) RWR_FAIL(RWR_E_UNSUPPORTED, "radix_sort: more than 2^32-1 elements");
-    u32 tiles = (u32)((n + RS_TILE - 1) / RS_TILE);
-    DevBuf<u32> table;
-    table.alloc((size_t)tiles * 256);
-    bool flipped = false;
-    for (int shift = 0; shift < end_bit; shift += 8) {
-        KeyT* ki = flipped ? keys_alt : keys;
-        KeyT* ko = flipped ? keys : keys_alt;
-        u32* vi = flipped ? vals_alt : vals;
-        u32* vo = flipped ? vals : vals_alt;
-        k_rs_hist<KeyT><<<tiles, RS_THREADS, 0, st>>>(ki, table.p, n, shift, tiles);
-        KERNEL_CHECK();
-        exclusive_scan<u32>(table.p, table.p, (size_t)tiles * 256, nullptr, st, pool);
-        if (vals)
-            k_rs_scatter<KeyT, true><<<tiles, RS_THREADS, 0, st>>>(ki, ko, vi, vo, table.p, n, shift, tiles);
-        else
-            k_rs_scatter<KeyT, false><<<tiles, RS_THREADS, 0, st>>>(ki, ko, nullptr, nullptr, table.p, n, shift, tiles);
-        KERNEL_CHECK();
-        if (pool) pool->launches += 2;
-        flipped = !flipped;
+struct SortBuffers {
+    DevBuf<KeyT> k[2];
+    DevBuf<u32> v[2];
+    int kc = 0, vc = 0;   // current key / value buffer
+
+    void alloc(size_t n, bool with_vals) {
+        k[0].alloc(n); k[1].alloc(n);
+        if (with_vals) { v[0].alloc(n); v[1].alloc(n); }
     }
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return flipped;
-}
+    KeyT* keys() const { return k[kc].p; }
+    u32* vals() const { return v[vc].p; }
+    // The spare key buffer becomes the current one, for the caller to fill with new keys: the next sort is a stable pass
+    // over them that keeps the current order of the values.
+    KeyT* rekey() { kc ^= 1; return keys(); }
+    void release_spare() { k[kc ^ 1].release(); v[vc ^ 1].release(); }
+    void release() { release_spare(); k[kc].release(); v[vc].release(); }
+    DevBuf<u32> take_vals() { return std::move(v[vc]); }
+
+    // Sorts the first `n` (< 2^32) current keys ascending on bits [0, end_bit), stable, with their values.
+    void sort(size_t n, int end_bit, cudaStream_t st, DevPool* pool) {
+        if (n == 0 || end_bit <= 0) return;
+        if (n >= (1ULL << 32)) RWR_FAIL(RWR_E_UNSUPPORTED, "radix_sort: more than 2^32-1 elements");
+        u32 tiles = (u32)((n + RS_TILE - 1) / RS_TILE);
+        DevBuf<u32> table;
+        table.alloc((size_t)tiles * 256);
+        for (int shift = 0; shift < end_bit; shift += 8) {
+            KeyT* ki = k[kc].p;
+            KeyT* ko = k[kc ^ 1].p;
+            k_rs_hist<KeyT><<<tiles, RS_THREADS, 0, st>>>(ki, table.p, n, shift, tiles);
+            KERNEL_CHECK();
+            exclusive_scan<u32>(table.p, table.p, (size_t)tiles * 256, nullptr, st, pool);
+            if (v[vc].p)
+                k_rs_scatter<KeyT, true><<<tiles, RS_THREADS, 0, st>>>(ki, ko, v[vc].p, v[vc ^ 1].p, table.p, n, shift, tiles);
+            else
+                k_rs_scatter<KeyT, false><<<tiles, RS_THREADS, 0, st>>>(ki, ko, nullptr, nullptr, table.p, n, shift, tiles);
+            KERNEL_CHECK();
+            if (pool) pool->launches += 2;
+            kc ^= 1;
+            vc ^= 1;
+        }
+        CUDA_CHECK(cudaStreamSynchronize(st));
+    }
+};
 
 }  // namespace prim

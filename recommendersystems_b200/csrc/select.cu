@@ -498,22 +498,18 @@ static void ensure_items_by_id(rwr_graph* g) {
     if (g->items_by_id_desc.p) return;
     cudaStream_t st = g->stream;
     const int n = g->n;
-    DevBuf<u32> pos, total;
-    pos.alloc(n); total.alloc(1);
+    DevBuf<u32> pos;
+    pos.alloc(n);
     if (n) k_item_flags<<<div_up(n, 256), 256, 0, st>>>(g->node_type_int.p, n, pos.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(pos.p, pos.p, n, total.p, st, &g->pool);
-    u32 m = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&m, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    DevBuf<u64> k0, k1;
-    DevBuf<u32> v0, v1;
-    k0.alloc(m); k1.alloc(m); v0.alloc(m); v1.alloc(m);
-    if (n) k_item_keys<<<div_up(n, 256), 256, 0, st>>>(g->node_type_int.p, g->node_id_int.p, pos.p, n, k0.p, v0.p);
+    const u32 m = prim::scan_total<u32>(pos.p, pos.p, n, false, st, &g->pool);
+    prim::SortBuffers<u64> sb;
+    sb.alloc(m, true);
+    if (n) k_item_keys<<<div_up(n, 256), 256, 0, st>>>(g->node_type_int.p, g->node_id_int.p, pos.p, n, sb.keys(), sb.vals());
     KERNEL_CHECK();
-    bool fl = prim::radix_sort<u64>(k0.p, k1.p, v0.p, v1.p, m, 64, st, &g->pool);
+    sb.sort(m, 64, st, &g->pool);
     g->items_by_id_desc.alloc(m, &g->pool);
-    if (m) CUDA_CHECK(cudaMemcpyAsync(g->items_by_id_desc.p, fl ? v1.p : v0.p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
+    if (m) CUDA_CHECK(cudaMemcpyAsync(g->items_by_id_desc.p, sb.vals(), (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
     CUDA_CHECK(cudaStreamSynchronize(st));
     g->n_items = (int)m;
 }
@@ -531,27 +527,23 @@ static int64_t rank_all_one(rwr_graph* g, const T* y, int seed, int64_t* ids, do
     if (rset) mark_excluded_for(g, rset, 0, excl.p, words);
     else mark_excluded(g, seed, excl.p, words);
     const int m = g->n_items;
-    DevBuf<u32> pos, total;
-    pos.alloc(m); total.alloc(1);
+    DevBuf<u32> pos;
+    pos.alloc(m);
     if (m) k_cand_flags<<<div_up(m, 256), 256, 0, st>>>(g->items_by_id_desc.p, m, excl.p, pos.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(pos.p, pos.p, m, total.p, st, &g->pool);
-    u32 cnt = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&cnt, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    const u32 cnt = prim::scan_total<u32>(pos.p, pos.p, m, false, st, &g->pool);
     if (cnt == 0) return 0;
-    DevBuf<u64> k0, k1;
-    DevBuf<u32> v0, v1;
-    k0.alloc(cnt); k1.alloc(cnt); v0.alloc(cnt); v1.alloc(cnt);
-    k_cand_keys<T><<<div_up(m, 256), 256, 0, st>>>(g->items_by_id_desc.p, m, excl.p, pos.p, y, k0.p, v0.p);
+    prim::SortBuffers<u64> sb;
+    sb.alloc(cnt, true);
+    k_cand_keys<T><<<div_up(m, 256), 256, 0, st>>>(g->items_by_id_desc.p, m, excl.p, pos.p, y, sb.keys(), sb.vals());
     KERNEL_CHECK();
-    bool fl = prim::radix_sort<u64>(k0.p, k1.p, v0.p, v1.p, cnt, 64, st, &g->pool);
+    sb.sort(cnt, 64, st, &g->pool);
     const size_t emit = (size_t)std::min<int64_t>(cap, (int64_t)cnt);
     if (emit && ids && scores) {
         DevBuf<int64_t> d_ids;
         DevBuf<double> d_sc;
         d_ids.alloc(emit); d_sc.alloc(emit);
-        k_emit_ranking<T><<<div_up(emit, 256), 256, 0, st>>>(fl ? v1.p : v0.p, emit, y, g->node_id_int.p, d_ids.p, d_sc.p);
+        k_emit_ranking<T><<<div_up(emit, 256), 256, 0, st>>>(sb.vals(), emit, y, g->node_id_int.p, d_ids.p, d_sc.p);
         KERNEL_CHECK();
         CUDA_CHECK(cudaMemcpyAsync(ids, d_ids.p, emit * 8, cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaMemcpyAsync(scores, d_sc.p, emit * 8, cudaMemcpyDeviceToHost, st));
@@ -955,17 +947,16 @@ static void ensure_id_lookup(rwr_graph* g) {
     if (g->ids_sorted.p) return;
     cudaStream_t st = g->stream;
     const int n = g->n;
-    DevBuf<u64> k0, k1;
-    DevBuf<u32> v0, v1;
-    k0.alloc(n); k1.alloc(n); v0.alloc(n); v1.alloc(n);
-    if (n) k_ev_id_keys<<<div_up(n, 256), 256, 0, st>>>(g->node_id_int.p, n, k0.p, v0.p);
+    prim::SortBuffers<u64> sb;
+    sb.alloc(n, true);
+    if (n) k_ev_id_keys<<<div_up(n, 256), 256, 0, st>>>(g->node_id_int.p, n, sb.keys(), sb.vals());
     KERNEL_CHECK();
-    const bool fl = prim::radix_sort<u64>(k0.p, k1.p, v0.p, v1.p, n, 64, st, &g->pool);
+    sb.sort(n, 64, st, &g->pool);
     g->ids_sorted.alloc(n, &g->pool);
     g->label_of_sorted.alloc(n, &g->pool);
     if (n) {
-        CUDA_CHECK(cudaMemcpyAsync(g->ids_sorted.p, fl ? k1.p : k0.p, (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
-        CUDA_CHECK(cudaMemcpyAsync(g->label_of_sorted.p, fl ? v1.p : v0.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(g->ids_sorted.p, sb.keys(), (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(g->label_of_sorted.p, sb.vals(), (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
     }
     CUDA_CHECK(cudaStreamSynchronize(st));
 }

@@ -291,16 +291,11 @@ void stream_prepare(rwr_graph* g) {
     }
     const u64 nnz2_max = (u64)g->nnz_in + (u64)n;
     if (nnz2_max + WS_TILE >= (1ull << 32)) RWR_FAIL(RWR_E_UNSUPPORTED, "edge stream of %llu links exceeds 32-bit offsets", (unsigned long long)nnz2_max);
-    DevBuf<u32> ptr2, total;
+    DevBuf<u32> ptr2;
     ptr2.alloc((size_t)n + 1);
-    total.alloc(1);
     k_ws_len<<<div_up(n, 256), 256, 0, st>>>(g->in_ptr.p, n, ptr2.p);
     KERNEL_CHECK();
-    prim::exclusive_scan<u32>(ptr2.p, ptr2.p, n, total.p, st, &g->pool);
-    u32 nnz2 = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&nnz2, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaMemcpyAsync(ptr2.p + n, total.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    u32 nnz2 = prim::scan_total<u32>(ptr2.p, ptr2.p, n, true, st, &g->pool);
     // row-partitioned graph: this rank keeps the rows [row_begin, row_end) of W^T
     u32 q0 = 0;
     g->row_begin = 0;
@@ -318,8 +313,7 @@ void stream_prepare(rwr_graph* g) {
         nnz2 = lim[1] - lim[0];
     }
     // column blocking (experimental): the stream is rebuilt over x_blocks * (row_end - row_begin) virtual rows
-    DevBuf<u32> ptr2v, cnt_ptr, perm, perm_alt;
-    const u32* perm_sorted = nullptr;
+    DevBuf<u32> ptr2v, cnt_ptr, perm;
     u32 link_base = 0;
     g->x_blocks = 1;
     g->v_rows = g->row_end - g->row_begin;
@@ -341,25 +335,21 @@ void stream_prepare(rwr_graph* g) {
                 const u32 lb = lim[0], le = lim[1];
                 const size_t er = (size_t)(le - lb);
                 if ((u64)er + V64 + WS_TILE >= (1ull << 32)) RWR_FAIL(RWR_E_UNSUPPORTED, "blocked edge stream exceeds 32-bit offsets");
-                DevBuf<u32> keys, keys_alt, total_v;
-                cnt_ptr.alloc(V + 1); ptr2v.alloc(V + 1); total_v.alloc(1);
-                keys.alloc(er); keys_alt.alloc(er); perm.alloc(er); perm_alt.alloc(er);
+                prim::SortBuffers<u32> sb;
+                cnt_ptr.alloc(V + 1); ptr2v.alloc(V + 1);
+                sb.alloc(er, true);
                 CUDA_CHECK(cudaMemsetAsync(cnt_ptr.p, 0, (V + 1) * sizeof(u32), st));
                 if (er) {
                     k_vrow_count<<<div_up(er, 256), 256, 0, st>>>(g->in_ptr.p, g->in_src.p, g->row_begin, g->row_end, lb, le, block_size,
-                                                                 R, cnt_ptr.p, keys.p, perm.p);
+                                                                 R, cnt_ptr.p, sb.keys(), sb.vals());
                     KERNEL_CHECK();
                 }
                 k_vrow_len<<<div_up(V, 256), 256, 0, st>>>(cnt_ptr.p, V, ptr2v.p);
                 KERNEL_CHECK();
-                prim::exclusive_scan<u32>(ptr2v.p, ptr2v.p, V, total_v.p, st, &g->pool);
-                CUDA_CHECK(cudaMemcpyAsync(&nnz2, total_v.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(ptr2v.p + V, total_v.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-                prim::exclusive_scan<u32>(cnt_ptr.p, cnt_ptr.p, V, total_v.p, st, &g->pool);
-                CUDA_CHECK(cudaMemcpyAsync(cnt_ptr.p + V, total_v.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-                const bool fl = prim::radix_sort<u32>(keys.p, keys_alt.p, perm.p, perm_alt.p, er, ceil_log2_u64((u64)xb), st, &g->pool);
-                CUDA_CHECK(cudaStreamSynchronize(st));
-                perm_sorted = fl ? perm_alt.p : perm.p;
+                nnz2 = prim::scan_total<u32>(ptr2v.p, ptr2v.p, V, true, st, &g->pool);
+                prim::exclusive_scan<u32>(cnt_ptr.p, cnt_ptr.p, V, cnt_ptr.p + V, st, &g->pool);
+                sb.sort(er, ceil_log2_u64((u64)xb), st, &g->pool);
+                perm = sb.take_vals();
                 link_base = lb;
                 q0 = 0;
                 g->x_blocks = xb;
@@ -385,25 +375,20 @@ void stream_prepare(rwr_graph* g) {
             smap.parts = parts;
             smap.rank = dist_rank(g->comm);
             for (int r = 0; r <= parts; r++) smap.start[r] = g->part_rows[r];
-            DevBuf<u32> cnt, keys, keys_alt, total_v;
-            cnt.alloc(V + 1); ptr2v.alloc(V + 1); cidx.alloc(V + 1); total_v.alloc(1);
-            keys.alloc(er); keys_alt.alloc(er); perm.alloc(er); perm_alt.alloc(er);
+            DevBuf<u32> cnt;
+            prim::SortBuffers<u32> sb;
+            cnt.alloc(V + 1); ptr2v.alloc(V + 1); cidx.alloc(V + 1);
+            sb.alloc(er, true);
             CUDA_CHECK(cudaMemsetAsync(cnt.p, 0, (V + 1) * sizeof(u32), st));
             k_pair_count<<<div_up(er, 256), 256, 0, st>>>(g->in_ptr.p, g->in_src.p, g->row_begin, g->row_end, lb, le, smap, R, cnt.p,
-                                                         keys.p, perm.p);
+                                                         sb.keys(), sb.vals());
             KERNEL_CHECK();
-            prim::exclusive_scan<u32>(cnt.p, ptr2v.p, V, total_v.p, st, &g->pool);
-            CUDA_CHECK(cudaMemcpyAsync(&nnz2, total_v.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            CUDA_CHECK(cudaMemcpyAsync(ptr2v.p + V, total_v.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
+            nnz2 = prim::scan_total<u32>(cnt.p, ptr2v.p, V, true, st, &g->pool);
             k_pair_flags<<<div_up(V, 256), 256, 0, st>>>(cnt.p, V, cidx.p);
             KERNEL_CHECK();
-            prim::exclusive_scan<u32>(cidx.p, cidx.p, V, total_v.p, st, &g->pool);
-            u32 vc = 0;
-            CUDA_CHECK(cudaMemcpyAsync(&vc, total_v.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            CUDA_CHECK(cudaMemcpyAsync(cidx.p + V, total_v.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
-            const bool fl = prim::radix_sort<u32>(keys.p, keys_alt.p, perm.p, perm_alt.p, er, ceil_log2_u64((u64)parts), st, &g->pool);
-            CUDA_CHECK(cudaStreamSynchronize(st));
-            perm_sorted = fl ? perm_alt.p : perm.p;
+            const u32 vc = prim::scan_total<u32>(cidx.p, cidx.p, V, true, st, &g->pool);
+            sb.sort(er, ceil_log2_u64((u64)parts), st, &g->pool);
+            perm = sb.take_vals();
             link_base = lb;
             q0 = 0;
             g->x_blocks = parts;
@@ -413,8 +398,7 @@ void stream_prepare(rwr_graph* g) {
             g->vpair.alloc((size_t)vc + 1, &g->pool);
             k_pair_row_counts<<<div_up((size_t)R, 256), 256, 0, st>>>(cnt.p, R, parts, g->vrow_ptr.p);
             KERNEL_CHECK();
-            prim::exclusive_scan<u32>(g->vrow_ptr.p, g->vrow_ptr.p, R, total_v.p, st, &g->pool);
-            CUDA_CHECK(cudaMemcpyAsync(g->vrow_ptr.p + R, total_v.p, sizeof(u32), cudaMemcpyDeviceToDevice, st));
+            prim::exclusive_scan<u32>(g->vrow_ptr.p, g->vrow_ptr.p, R, g->vrow_ptr.p + R, st, &g->pool);
             k_pair_row_fill<<<div_up((size_t)R, 256), 256, 0, st>>>(cnt.p, cidx.p, g->vrow_ptr.p, R, parts, g->vpair.p);
             KERNEL_CHECK();
             // first stream position of every block -> the tile that holds it (k_spmv_ws waits for a block's slice there)
@@ -468,7 +452,7 @@ void stream_prepare(rwr_graph* g) {
         for (int k = 0; k < 8; k++)
             if (g->blk_first_tile[k] != INT32_MAX) g->blk_first_tile[k] /= tile_links;
         if (padded)
-            k_ws_fill_compact<<<div_up(padded, 256), 256, 0, st>>>(ptr2v.p, perm_sorted, g->in_src.p + link_base,
+            k_ws_fill_compact<<<div_up(padded, 256), 256, 0, st>>>(ptr2v.p, perm.p, g->in_src.p + link_base,
                                                                   valued ? g->in_val64.p + link_base : nullptr, V, n, nnz2, padded, hm,
                                                                   g->ws_src.p, valued ? g->ws_val64.p : nullptr);
         k_ws_tiles_compact<<<div_up((size_t)n_tiles + 1, 256), 256, 0, st>>>(ptr2v.p, cidx.p, V, (u32)g->v_compact, n_tiles,
@@ -476,7 +460,7 @@ void stream_prepare(rwr_graph* g) {
     } else if (blocked) {
         const int V = g->x_blocks * g->v_rows;
         if (padded)
-            k_ws_fill_blocked<<<div_up(padded, 256), 256, 0, st>>>(ptr2v.p, cnt_ptr.p, perm_sorted, g->in_src.p + link_base,
+            k_ws_fill_blocked<<<div_up(padded, 256), 256, 0, st>>>(ptr2v.p, cnt_ptr.p, perm.p, g->in_src.p + link_base,
                                                                   valued ? g->in_val64.p + link_base : nullptr, V, n, nnz2, padded, hm,
                                                                   g->ws_src.p, valued ? g->ws_val64.p : nullptr);
         k_ws_tiles<<<div_up((size_t)n_tiles + 1, 256), 256, 0, st>>>(ptr2v.p, V, 0u, V, n_tiles, (u32)tile_links, g->ws_tile.p);

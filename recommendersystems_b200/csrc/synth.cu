@@ -215,7 +215,7 @@ void synth_generate_device(rwr_graph* g, const rwr_synth_spec* spec) {
     k_synth_nodes<<<div_up(N, 256), 256, 0, st>>>(s.U, s.T, N, g->node_id.p, g->node_type.p);
     KERNEL_CHECK();
 
-    DevBuf<u64> keys, keys_alt;
+    prim::SortBuffers<u64> sb;
     if (owned) {
         DevBuf<unsigned long long> counter;
         counter.alloc(1);
@@ -225,7 +225,7 @@ void synth_generate_device(rwr_graph* g, const rwr_synth_spec* spec) {
             CUDA_CHECK(cudaMemsetAsync(counter.p, 0, sizeof(unsigned long long), st));
             for (u64 j0 = 0; j0 < s.nrel; j0 += CH) {
                 const u64 j1 = std::min(s.nrel, j0 + CH);
-                k_synth_keys_owned<<<div_up((size_t)(j1 - j0), 256), 256, 0, st>>>(s, g->own, j0, j1, pass ? keys.p : nullptr, counter.p);
+                k_synth_keys_owned<<<div_up((size_t)(j1 - j0), 256), 256, 0, st>>>(s, g->own, j0, j1, pass ? sb.keys() : nullptr, counter.p);
                 KERNEL_CHECK();
             }
             if (pass == 0) {
@@ -233,35 +233,27 @@ void synth_generate_device(rwr_graph* g, const rwr_synth_spec* spec) {
                 CUDA_CHECK(cudaStreamSynchronize(st));
                 if (mine >= (1ULL << 32) - 65536) RWR_FAIL(RWR_E_UNSUPPORTED, "more than 2^32-65537 link slots on one rank");
                 slots = (size_t)mine;
-                keys.alloc(slots);
-                keys_alt.alloc(slots);
+                sb.alloc(slots, false);
             }
         }
     } else {
-        keys.alloc(slots);
-        keys_alt.alloc(slots);
+        sb.alloc(slots, false);
         if (s.nrel) {
-            k_synth_keys<<<div_up((size_t)s.nrel, 256), 256, 0, st>>>(s, keys.p);
+            k_synth_keys<<<div_up((size_t)s.nrel, 256), 256, 0, st>>>(s, sb.keys());
             KERNEL_CHECK();
         }
     }
-    const int end_bit = 31 + ceil_log2_u64(N);
     // the all-ones sentinel must sort last: include every bit when any slot can be invalid
-    bool fl = prim::radix_sort<u64>(keys.p, keys_alt.p, nullptr, nullptr, slots, 64, st, &g->pool);
-    (void)end_bit;
-    const u64* sorted = fl ? keys_alt.p : keys.p;
-    (fl ? keys : keys_alt).release();
-    DevBuf<u32> pos, total;
+    sb.sort(slots, 64, st, &g->pool);
+    sb.release_spare();
+    const u64* sorted = sb.keys();
+    DevBuf<u32> pos;
     pos.alloc(slots);
-    total.alloc(1);
     if (slots) {
         k_unique_flags<<<div_up(slots, 256), 256, 0, st>>>(sorted, slots, pos.p);
         KERNEL_CHECK();
     }
-    prim::exclusive_scan<u32>(pos.p, pos.p, slots, total.p, st, &g->pool);
-    u32 e0 = 0;
-    CUDA_CHECK(cudaMemcpyAsync(&e0, total.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
+    const u32 e0 = prim::scan_total<u32>(pos.p, pos.p, slots, false, st, &g->pool);
     g->e0 = (int64_t)e0;
     g->raw_src.alloc(e0, &g->pool);
     g->raw_dst.alloc(e0, &g->pool);
@@ -274,8 +266,7 @@ void synth_generate_device(rwr_graph* g, const rwr_synth_spec* spec) {
     CUDA_CHECK(cudaStreamSynchronize(st));
     g->pool.launches += 4;
     pos.release();
-    keys.release();
-    keys_alt.release();
+    sb.release();
     graph_finish_create(g);     // already source-ascending: only raw_ptr is built
     CUDA_CHECK(cudaEventRecord(ev1, st));
     CUDA_CHECK(cudaEventSynchronize(ev1));
