@@ -23,10 +23,9 @@
 #include "stream.h"
 #include "dist.h"
 
+// The bitmap and scan kernels work on prim's scan tiles, the sort kernels on its radix-sort tiles; k_fr_expand and k_fr_sum
+// go over their entries with FR_THREADS per block.
 constexpr int FR_THREADS = 256;
-constexpr int FR_ITEMS = 8;
-constexpr int FR_TILE = FR_THREADS * FR_ITEMS;   // 2048
-constexpr int FR_WARPS = FR_THREADS / 32;
 
 struct FrDev {
     IterCtl* ctl;
@@ -46,31 +45,32 @@ struct FrDev {
 __device__ __forceinline__ bool fr_off(const FrDev& d) { return d.ctl->sparse == 0; }
 
 // sum of bsum[0, b) over the block (result in every thread)
-__device__ __forceinline__ u32 fr_prefix(const u32* bsum, int b, u32* red /* FR_WARPS + 1 */) {
+__device__ __forceinline__ u32 fr_prefix(const u32* bsum, int b, u32* red /* SCAN_THREADS / 32 + 1 */) {
+    constexpr int WARPS = prim::SCAN_THREADS / 32;
     u32 s = 0;
-    for (int i = threadIdx.x; i < b; i += FR_THREADS) s += bsum[i];
+    for (int i = threadIdx.x; i < b; i += prim::SCAN_THREADS) s += bsum[i];
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
     __syncthreads();
     if (threadIdx.x == 0) {
         u32 t = 0;
-        for (int w = 0; w < FR_WARPS; w++) t += red[w];
-        red[FR_WARPS] = t;
+        for (int w = 0; w < WARPS; w++) t += red[w];
+        red[WARPS] = t;
     }
     __syncthreads();
-    const u32 r = red[FR_WARPS];
+    const u32 r = red[WARPS];
     __syncthreads();
     return r;
 }
 
 // ------------------------------------------------------------------------------------------------ frontier
-__global__ void __launch_bounds__(FR_THREADS) k_fr_count(const FrDev d) {
+__global__ void __launch_bounds__(prim::SCAN_THREADS) k_fr_count(const FrDev d) {
     __shared__ u32 sm[9];
     if (fr_off(d)) return;
-    const size_t base = (size_t)blockIdx.x * FR_TILE + (size_t)threadIdx.x * FR_ITEMS;
+    const size_t base = (size_t)blockIdx.x * prim::SCAN_TILE + (size_t)threadIdx.x * prim::SCAN_ITEMS;
     u32 c = 0;
 #pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++)
+    for (int k = 0; k < prim::SCAN_ITEMS; k++)
         if (base + k < d.words) c += __popc(d.bits[base + k]);
     u32 total;
     prim::block_exclusive_scan_256(c, &total, sm);
@@ -80,9 +80,9 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_count(const FrDev d) {
 // bitmap -> frontier list (ascending) and out-degrees; clears the bitmap
 // This kernel may clear ctl->sparse itself: every block reads the flag once, behind a barrier, so that all its threads
 // agree and reach the barriers below together.
-__global__ void __launch_bounds__(FR_THREADS) k_fr_extract(const FrDev d) {
+__global__ void __launch_bounds__(prim::SCAN_THREADS) k_fr_extract(const FrDev d) {
     __shared__ u32 sm[9];
-    __shared__ u32 red[FR_WARPS + 1];
+    __shared__ u32 red[prim::SCAN_THREADS / 32 + 1];
     __shared__ int off;
     if (threadIdx.x == 0) off = fr_off(d);
     __syncthreads();
@@ -94,18 +94,18 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_extract(const FrDev d) {
     }
     const u32 pre = fr_prefix(d.bsum, blockIdx.x, red);
     if (blockIdx.x == 0 && threadIdx.x == 0) d.sc[0] = nf;
-    const size_t base = (size_t)blockIdx.x * FR_TILE + (size_t)threadIdx.x * FR_ITEMS;
-    u32 w[FR_ITEMS];
+    const size_t base = (size_t)blockIdx.x * prim::SCAN_TILE + (size_t)threadIdx.x * prim::SCAN_ITEMS;
+    u32 w[prim::SCAN_ITEMS];
     u32 c = 0;
 #pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++) {
+    for (int k = 0; k < prim::SCAN_ITEMS; k++) {
         w[k] = (base + k < d.words) ? d.bits[base + k] : 0u;
         c += __popc(w[k]);
     }
     u32 total;
     u32 pos = prim::block_exclusive_scan_256(c, &total, sm) + pre;
 #pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++) {
+    for (int k = 0; k < prim::SCAN_ITEMS; k++) {
         u32 m = w[k];
         if (!m) continue;
         d.bits[base + k] = 0u;
@@ -121,50 +121,30 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_extract(const FrDev d) {
 }
 
 // ------------------------------------------------------------------------------------------------ device-sized scan
-// Exclusive scan of in[0, *len) into out (in place allowed), out[*len] = total.  Pass A: one sum per 2048-entry block;
-// pass B: every block adds the sums of the blocks before it.
-__global__ void __launch_bounds__(FR_THREADS) k_fr_scan_a(const FrDev d, const u32* __restrict__ in, const u32* len_ptr) {
+// Exclusive scan of in[0, *len) into out (in place allowed), out[*len] = total, on prim's scan tiles.  Pass A: one sum per
+// tile; pass B: every tile adds the sums of the tiles before it.
+__global__ void __launch_bounds__(prim::SCAN_THREADS) k_fr_scan_a(const FrDev d, const u32* __restrict__ in, const u32* len_ptr) {
     __shared__ u32 sm[9];
     if (fr_off(d)) return;
     const u32 len = *len_ptr;
-    const size_t base = (size_t)blockIdx.x * FR_TILE + (size_t)threadIdx.x * FR_ITEMS;
-    if ((size_t)blockIdx.x * FR_TILE >= len) return;
-    u32 s = 0;
-#pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++)
-        if (base + k < len) s += in[base + k];
-    u32 total;
-    prim::block_exclusive_scan_256(s, &total, sm);
+    if ((size_t)blockIdx.x * prim::SCAN_TILE >= len) return;
+    const u32 total = prim::scan_tile_total<u32>(in, len, sm);
     if (threadIdx.x == 0) d.bsum[blockIdx.x] = total;
 }
 
-__global__ void __launch_bounds__(FR_THREADS) k_fr_scan_b(const FrDev d, const u32* in, u32* out, const u32* len_ptr) {
+__global__ void __launch_bounds__(prim::SCAN_THREADS) k_fr_scan_b(const FrDev d, const u32* in, u32* out, const u32* len_ptr) {
     __shared__ u32 sm[9];
-    __shared__ u32 red[FR_WARPS + 1];
+    __shared__ u32 red[prim::SCAN_THREADS / 32 + 1];
     if (fr_off(d)) return;
     const u32 len = *len_ptr;
     if (len == 0) {
         if (blockIdx.x == 0 && threadIdx.x == 0) out[0] = 0;
         return;
     }
-    if ((size_t)blockIdx.x * FR_TILE >= len) return;
+    if ((size_t)blockIdx.x * prim::SCAN_TILE >= len) return;
     const u32 pre = fr_prefix(d.bsum, blockIdx.x, red);
-    const size_t base = (size_t)blockIdx.x * FR_TILE + (size_t)threadIdx.x * FR_ITEMS;
-    u32 v[FR_ITEMS];
-    u32 s = 0;
-#pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++) {
-        v[k] = (base + k < len) ? in[base + k] : 0u;
-        s += v[k];
-    }
-    u32 total;
-    u32 ex = prim::block_exclusive_scan_256(s, &total, sm) + pre;
-#pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++) {
-        if (base + k < len) out[base + k] = ex;
-        ex += v[k];
-    }
-    if (threadIdx.x == 0 && (size_t)(blockIdx.x + 1) * FR_TILE >= len) out[len] = pre + total;
+    const u32 total = prim::scan_tile_apply<u32>(in, out, len, [=] { return pre; }, sm);
+    if (threadIdx.x == 0 && (size_t)(blockIdx.x + 1) * prim::SCAN_TILE >= len) out[len] = pre + total;
 }
 
 // ------------------------------------------------------------------------------------------------ expand
@@ -200,79 +180,28 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_expand(const FrDev d, const T
 }
 
 // ------------------------------------------------------------------------------------------------ radix sort
-// One stable 8-bit pass of an LSD sort over the sc[1] entries (the same scheme as prim::SortBuffers, with the count on the
-// device).  The digit table is digit-major over the tiles that hold entries.
-__global__ void __launch_bounds__(FR_THREADS) k_fr_hist(const FrDev d, const u32* __restrict__ keys, int shift) {
+// One stable 8-bit pass of prim's LSD sort over the sc[1] entries, with the count on the device: the kernels return in the
+// blocks past the tiles that hold entries, over which the digit table is digit-major.
+__device__ __forceinline__ u32 fr_sort_tiles(const FrDev& d) { return (d.sc[1] + prim::RS_TILE - 1) / prim::RS_TILE; }
+
+__global__ void __launch_bounds__(prim::RS_THREADS) k_fr_hist(const FrDev d, const u32* __restrict__ keys, int shift) {
     __shared__ u32 h[256];
     if (fr_off(d)) return;
-    const u32 ne = d.sc[1];
-    const u32 tiles = (ne + FR_TILE - 1) / FR_TILE;
+    const u32 tiles = fr_sort_tiles(d);
     if (blockIdx.x >= tiles) return;
     if (blockIdx.x == 0 && threadIdx.x == 0) d.sc[2] = 256u * tiles;
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    const size_t base = (size_t)blockIdx.x * FR_TILE;
-#pragma unroll
-    for (int k = 0; k < FR_ITEMS; k++) {
-        const size_t i = base + (size_t)k * FR_THREADS + threadIdx.x;
-        if (i < ne) atomicAdd(&h[(keys[i] >> shift) & 255u], 1u);
-    }
-    __syncthreads();
-    d.table[(size_t)threadIdx.x * tiles + blockIdx.x] = h[threadIdx.x];
+    prim::rs_hist_tile<u32>(keys, d.table, d.sc[1], shift, tiles, h);
 }
 
 template <typename T>
-__global__ void __launch_bounds__(FR_THREADS) k_fr_scatter(const FrDev d, const u32* __restrict__ keys_in, u32* __restrict__ keys_out,
-                                                          const T* __restrict__ vals_in, T* __restrict__ vals_out, int shift) {
-    __shared__ u32 wh[FR_WARPS][256];
+__global__ void __launch_bounds__(prim::RS_THREADS) k_fr_scatter(const FrDev d, const u32* __restrict__ keys_in, u32* __restrict__ keys_out,
+                                                                const T* __restrict__ vals_in, T* __restrict__ vals_out, int shift) {
+    __shared__ u32 wh[prim::RS_WARPS][256];
     if (fr_off(d)) return;
-    const u32 ne = d.sc[1];
-    const u32 tiles = (ne + FR_TILE - 1) / FR_TILE;
+    const u32 tiles = fr_sort_tiles(d);
     if (blockIdx.x >= tiles) return;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int i = threadIdx.x; i < FR_WARPS * 256; i += FR_THREADS) (&wh[0][0])[i] = 0;
-    __syncthreads();
-    // element order inside a tile is (warp, round, lane): ranking in that order keeps the sort stable
-    const size_t wbase = (size_t)blockIdx.x * FR_TILE + (size_t)warp * (32 * FR_ITEMS);
-    u32 key[FR_ITEMS], rank[FR_ITEMS];
-    const u32 lt = (1u << lane) - 1u;
-#pragma unroll
-    for (int r = 0; r < FR_ITEMS; r++) {
-        const size_t i = wbase + (size_t)r * 32 + lane;
-        const bool valid = i < ne;
-        key[r] = valid ? keys_in[i] : 0u;
-        const u32 dg = valid ? ((key[r] >> shift) & 255u) : 256u;
-        const u32 peers = __match_any_sync(0xffffffffu, dg);
-        const int leader = __ffs(peers) - 1;
-        u32 b = 0;
-        if (valid && lane == leader) {
-            b = wh[warp][dg];
-            wh[warp][dg] = b + __popc(peers);
-        }
-        b = __shfl_sync(0xffffffffu, b, leader);
-        rank[r] = b + __popc(peers & lt);
-        __syncwarp();
-    }
-    __syncthreads();
-    {
-        u32 run = d.table[(size_t)threadIdx.x * tiles + blockIdx.x];
-#pragma unroll
-        for (int w = 0; w < FR_WARPS; w++) {
-            const u32 t = wh[w][threadIdx.x];
-            wh[w][threadIdx.x] = run;
-            run += t;
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < FR_ITEMS; r++) {
-        const size_t i = wbase + (size_t)r * 32 + lane;
-        if (i < ne) {
-            const u32 pos = wh[warp][(key[r] >> shift) & 255u] + rank[r];
-            keys_out[pos] = key[r];
-            vals_out[pos] = vals_in[i];
-        }
-    }
+    prim::rs_scatter_tile<u32, T, true>(keys_in, keys_out, vals_in, vals_out, d.table, d.sc[1], shift, tiles, wh,
+                                        threadIdx.x);
 }
 
 // ------------------------------------------------------------------------------------------------ sum + epilogue
@@ -281,7 +210,7 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_scatter(const FrDev d, const 
 template <typename T>
 __global__ void __launch_bounds__(FR_THREADS) k_fr_sum(const FrDev d, const u32* __restrict__ key, const T* __restrict__ prod,
                                                       const IterParams<T> p, int emit) {
-    __shared__ double scratch[2 * FR_WARPS];
+    __shared__ double scratch[2 * FR_THREADS / 32];
     __shared__ int is_last;
     IterCtl* ctl = p.ctl;
     if (fr_off(d)) return;
@@ -308,26 +237,11 @@ __global__ void __launch_bounds__(FR_THREADS) k_fr_sum(const FrDev d, const u32*
             atomicOr(&d.bits[o >> 5], 1u << (o & 31));
         }
     }
-    block_sum2<FR_THREADS>(accS, unused, scratch);
-    if (threadIdx.x == 0) {
-        p.slot_S[blockIdx.x] = accS;
-        __threadfence();
-        const unsigned tk = atomicAdd(&ctl->ticket, 1u);
-        is_last = (tk == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (is_last) {
-        __threadfence();
-        double a = 0.0, b = 0.0;
-        for (int i = threadIdx.x; i < (int)gridDim.x; i += FR_THREADS) a += __ldcg(p.slot_S + i);
-        __syncthreads();
-        block_sum2<FR_THREADS>(a, b, scratch);
-        if (threadIdx.x == 0) {
-            ctl->S = a;
-            ctl->iters += 1;
-            ctl->sparse_iters += 1;               // the dense kernels of this iteration return at once
-            ctl->ticket = 0;
-        }
+    if (grid_sum2<FR_THREADS, false>(accS, unused, p.slot_S, nullptr, ctl, scratch, &is_last) && threadIdx.x == 0) {
+        ctl->S = accS;
+        ctl->iters += 1;
+        ctl->sparse_iters += 1;                   // the dense kernels of this iteration return at once
+        ctl->ticket = 0;
     }
 }
 
@@ -372,10 +286,10 @@ size_t frontier_carve(const rwr_graph* g, u64 budget, size_t elt, void* base, Fr
     fw.budget = budget;
     fw.cap = (size_t)budget + 1;
     fw.words = (u32)(((size_t)g->n + 31) / 32);
-    fw.g_words = (int)div_up(fw.words, FR_TILE);
-    fw.g_scan_f = (int)div_up((size_t)budget + 1, FR_TILE);
-    fw.t_max = (int)div_up(fw.cap, FR_TILE);
-    fw.g_scan_t = (int)div_up((size_t)fw.t_max * 256, FR_TILE);
+    fw.g_words = (int)div_up(fw.words, prim::SCAN_TILE);
+    fw.g_scan_f = (int)div_up((size_t)budget + 1, prim::SCAN_TILE);
+    fw.t_max = (int)div_up(fw.cap, prim::RS_TILE);
+    fw.g_scan_t = (int)div_up((size_t)fw.t_max * 256, prim::SCAN_TILE);
     fw.g_exp = (int)std::min<size_t>(div_up(fw.cap, FR_THREADS), (size_t)g->sm_count * 8);
     fw.g_sum = (int)std::min<size_t>(div_up(fw.cap, FR_THREADS), (size_t)g->sm_count * 8);   // <= the slots of the workspace
     fw.passes = (ceil_log2_u64((u64)g->n) + 7) / 8;
@@ -407,19 +321,19 @@ int frontier_launch(rwr_graph* g, const FrontierWs& fw, const IterParams<T>& p, 
     d.n = g->n; d.words = fw.words; d.nnz = (u64)g->nnz; d.budget = fw.budget;
     d.bits = fw.bits; d.fid = fw.fid; d.fdeg = fw.fdeg; d.foff = fw.foff; d.bsum = fw.bsum; d.table = fw.table;
     int launches = 0;
-    k_fr_count<<<fw.g_words, FR_THREADS, 0, st>>>(d);
-    k_fr_extract<<<fw.g_words, FR_THREADS, 0, st>>>(d);
-    k_fr_scan_a<<<fw.g_scan_f, FR_THREADS, 0, st>>>(d, fw.fdeg, fw.sc);
-    k_fr_scan_b<<<fw.g_scan_f, FR_THREADS, 0, st>>>(d, fw.fdeg, fw.foff, fw.sc);
+    k_fr_count<<<fw.g_words, prim::SCAN_THREADS, 0, st>>>(d);
+    k_fr_extract<<<fw.g_words, prim::SCAN_THREADS, 0, st>>>(d);
+    k_fr_scan_a<<<fw.g_scan_f, prim::SCAN_THREADS, 0, st>>>(d, fw.fdeg, fw.sc);
+    k_fr_scan_b<<<fw.g_scan_f, prim::SCAN_THREADS, 0, st>>>(d, fw.fdeg, fw.foff, fw.sc);
     k_fr_expand<T><<<fw.g_exp, FR_THREADS, 0, st>>>(d, p.x, fw.key[0], (T*)fw.val[0]);
     launches += 5;
     int cur = 0;
     for (int pass = 0; pass < fw.passes; pass++) {
-        k_fr_hist<<<fw.t_max, FR_THREADS, 0, st>>>(d, fw.key[cur], pass * 8);
-        k_fr_scan_a<<<fw.g_scan_t, FR_THREADS, 0, st>>>(d, fw.table, fw.sc + 2);
-        k_fr_scan_b<<<fw.g_scan_t, FR_THREADS, 0, st>>>(d, fw.table, fw.table, fw.sc + 2);
-        k_fr_scatter<T><<<fw.t_max, FR_THREADS, 0, st>>>(d, fw.key[cur], fw.key[cur ^ 1], (const T*)fw.val[cur], (T*)fw.val[cur ^ 1],
-                                                          pass * 8);
+        k_fr_hist<<<fw.t_max, prim::RS_THREADS, 0, st>>>(d, fw.key[cur], pass * 8);
+        k_fr_scan_a<<<fw.g_scan_t, prim::SCAN_THREADS, 0, st>>>(d, fw.table, fw.sc + 2);
+        k_fr_scan_b<<<fw.g_scan_t, prim::SCAN_THREADS, 0, st>>>(d, fw.table, fw.table, fw.sc + 2);
+        k_fr_scatter<T><<<fw.t_max, prim::RS_THREADS, 0, st>>>(d, fw.key[cur], fw.key[cur ^ 1], (const T*)fw.val[cur],
+                                                                (T*)fw.val[cur ^ 1], pass * 8);
         cur ^= 1;
         launches += 4;
     }

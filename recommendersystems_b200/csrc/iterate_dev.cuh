@@ -1,5 +1,5 @@
-// iterate_dev.cuh -- device-side pieces shared by iterate.cu and stream.cu: the launch parameters of an iteration, PTX
-// helpers (mbarrier, TMA bulk copy, cache-hinted loads) and the fixed-order block reduction.
+// iterate_dev.cuh -- device-side pieces shared by iterate.cu, stream.cu and frontier.cu: the launch parameters of an
+// iteration, PTX helpers (mbarrier, TMA bulk copy, cache-hinted loads) and the fixed-order block and grid reductions.
 #pragma once
 
 #include "iterate.h"
@@ -121,6 +121,34 @@ __device__ __forceinline__ void block_sum2(double& a, double& b, double* scratch
         for (int w = 0; w < THREADS / 32; w++) { sa += scratch[w]; sb += scratch[THREADS / 32 + w]; }
         a = sa; b = sb;
     }
+}
+
+// Fixed-order reduction over the blocks of a grid: every block reduces its partials a (and, with TWO, b), stores them in
+// slot_a[blockIdx.x] (slot_b) and takes a ticket on ctl->ticket.  Returns true in the last block to arrive, where thread 0
+// then holds the sums of all slots, added in block order, in a (and b); that block's caller resets ctl->ticket.
+template <int THREADS, bool TWO>
+__device__ __forceinline__ bool grid_sum2(double& a, double& b, double* slot_a, double* slot_b, IterCtl* ctl,
+                                          double* scratch /* 2 * THREADS/32 */, int* is_last /* shared */) {
+    block_sum2<THREADS>(a, b, scratch);
+    if (threadIdx.x == 0) {
+        slot_a[blockIdx.x] = a;
+        if (TWO) slot_b[blockIdx.x] = b;
+        __threadfence();
+        const unsigned tk = atomicAdd(&ctl->ticket, 1u);
+        *is_last = (tk == gridDim.x - 1);
+    }
+    __syncthreads();
+    if (!*is_last) return false;
+    __threadfence();
+    a = 0.0;
+    b = 0.0;
+    for (int i = threadIdx.x; i < (int)gridDim.x; i += THREADS) {
+        a += __ldcg(slot_a + i);
+        if (TWO) b += __ldcg(slot_b + i);
+    }
+    __syncthreads();
+    block_sum2<THREADS>(a, b, scratch);
+    return true;
 }
 
 // ------------------------------------------------------------------------------------------------ shared-space PTX

@@ -1,5 +1,6 @@
 // primitives.cuh -- device-wide exclusive scan (K2) and stable LSD radix sort used by the graph build (K3, K5),
-// the synthetic generator (K0) and the full ranking (A9).  Hand-written; no CUB/Thrust.
+// the synthetic generator (K0), the full ranking (A9) and, through their tile bodies, the sparse prefix of a single-seed run
+// (frontier.cu, counts on the device).  Hand-written; no CUB/Thrust.
 #pragma once
 
 #include "common.cuh"
@@ -40,9 +41,12 @@ __device__ __forceinline__ u32 block_exclusive_scan_256(u32 v, u32* total, u32* 
     return res;
 }
 
+// The tile bodies below serve the host-sized kernels here and the device-sized ones of the sparse prefix (frontier.cu):
+// block b works on tile b of the n items, and the shared arrays belong to the calling kernel.
+
+// sum of the block's tile of in[0, n), in every thread
 template <typename InT>
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_sums(const InT* __restrict__ in, u32* __restrict__ sums, size_t n) {
-    __shared__ u32 sm[9];
+__device__ __forceinline__ u32 scan_tile_total(const InT* __restrict__ in, size_t n, u32* sm /*>=9*/) {
     size_t base = (size_t)blockIdx.x * SCAN_TILE + (size_t)threadIdx.x * SCAN_ITEMS;
     u32 s = 0;
 #pragma unroll
@@ -50,13 +54,14 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_sums(const InT* __re
         if (base + k < n) s += (u32)in[base + k];
     u32 total;
     block_exclusive_scan_256(s, &total, sm);
-    if (threadIdx.x == 0) sums[blockIdx.x] = total;
+    return total;
 }
 
-template <typename InT>
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_apply(const InT* __restrict__ in, u32* __restrict__ out,
-                                                                 const u32* __restrict__ tile_off, size_t n) {
-    __shared__ u32 sm[9];
+// exclusive scan of the block's tile of in[0, n) into out, every entry plus the tile's offset off(); returns the tile's sum.
+// off() is called after the block scan: k_scan_tile_apply loads the offset there, k_fr_scan_b has computed it before.
+template <typename InT, typename Off>
+__device__ __forceinline__ u32 scan_tile_apply(const InT* __restrict__ in, u32* __restrict__ out, size_t n, Off off,
+                                               u32* sm /*>=9*/) {
     size_t base = (size_t)blockIdx.x * SCAN_TILE + (size_t)threadIdx.x * SCAN_ITEMS;
     u32 v[SCAN_ITEMS];
     u32 s = 0;
@@ -66,12 +71,27 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_apply(const InT* __r
         s += v[k];
     }
     u32 total;
-    u32 ex = block_exclusive_scan_256(s, &total, sm) + (tile_off ? tile_off[blockIdx.x] : 0);
+    u32 ex = block_exclusive_scan_256(s, &total, sm) + off();
 #pragma unroll
     for (int k = 0; k < SCAN_ITEMS; k++) {
         if (base + k < n) out[base + k] = ex;
         ex += v[k];
     }
+    return total;
+}
+
+template <typename InT>
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_sums(const InT* __restrict__ in, u32* __restrict__ sums, size_t n) {
+    __shared__ u32 sm[9];
+    u32 total = scan_tile_total<InT>(in, n, sm);
+    if (threadIdx.x == 0) sums[blockIdx.x] = total;
+}
+
+template <typename InT>
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_apply(const InT* __restrict__ in, u32* __restrict__ out,
+                                                                 const u32* __restrict__ tile_off, size_t n) {
+    __shared__ u32 sm[9];
+    scan_tile_apply<InT>(in, out, n, [&] { return tile_off ? tile_off[blockIdx.x] : 0u; }, sm);
 }
 
 // out[i] = sum(in[0..i)), out may alias in when InT is u32; optional total (device pointer) = sum of all, and with
@@ -125,10 +145,10 @@ constexpr int RS_ITEMS = 8;
 constexpr int RS_TILE = RS_THREADS * RS_ITEMS;   // 2048 keys per CTA
 constexpr int RS_WARPS = RS_THREADS / 32;
 
+// digit histogram of the block's tile of keys[0, n) into its column of the digit-major table of `tiles` tiles
 template <typename KeyT>
-__global__ void __launch_bounds__(RS_THREADS) k_rs_hist(const KeyT* __restrict__ keys, u32* __restrict__ table, size_t n,
-                                                        int shift, u32 tiles) {
-    __shared__ u32 h[256];
+__device__ __forceinline__ void rs_hist_tile(const KeyT* __restrict__ keys, u32* __restrict__ table, size_t n, int shift, u32 tiles,
+                                             u32* h /*256*/) {
     h[threadIdx.x] = 0;
     __syncthreads();
     size_t base = (size_t)blockIdx.x * RS_TILE;
@@ -141,16 +161,17 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_hist(const KeyT* __restrict__
     table[(size_t)threadIdx.x * tiles + blockIdx.x] = h[threadIdx.x];   // digit-major
 }
 
-// Stable scatter.  Element order inside a tile is (warp, round, lane): warp w owns the contiguous sub-tile
-// [w*32*ITEMS, (w+1)*32*ITEMS), read in rounds of 32 consecutive keys, so ranking by (warp, round, lane)
-// preserves the input order.
-template <typename KeyT, bool HAS_VAL>
-__global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out,
-                                                           const u32* __restrict__ vals_in, u32* __restrict__ vals_out,
-                                                           const u32* __restrict__ table, size_t n, int shift, u32 tiles) {
-    __shared__ u32 wh[RS_WARPS][256];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int i = threadIdx.x; i < RS_WARPS * 256; i += RS_THREADS) (&wh[0][0])[i] = 0;
+// Stable scatter of the block's tile, with the table scanned.  Element order inside a tile is (warp, round, lane): warp w owns
+// the contiguous sub-tile [w*32*ITEMS, (w+1)*32*ITEMS), read in rounds of 32 consecutive keys, so ranking by (warp, round,
+// lane) preserves the input order.  `tid` is the kernel's threadIdx.x: read in the kernel, it carries the range of the
+// launch bounds, which lets the compiler form the warp's first key as tile base | warp offset.
+template <typename KeyT, typename ValT, bool HAS_VAL>
+__device__ __forceinline__ void rs_scatter_tile(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out,
+                                                const ValT* __restrict__ vals_in, ValT* __restrict__ vals_out,
+                                                const u32* __restrict__ table, size_t n, int shift, u32 tiles,
+                                                u32 (*wh)[256] /*[RS_WARPS]*/, const u32 tid) {
+    const int lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i < RS_WARPS * 256; i += RS_THREADS) (&wh[0][0])[i] = 0;
     __syncthreads();
     const size_t wbase = (size_t)blockIdx.x * RS_TILE + (size_t)warp * (32 * RS_ITEMS);
     KeyT key[RS_ITEMS];
@@ -174,12 +195,12 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const KeyT* __restric
         __syncwarp();
     }
     __syncthreads();
-    {   // digit d = threadIdx.x: exclusive prefix over the warps, seeded with the global offset of (d, tile)
-        u32 run = table[(size_t)threadIdx.x * tiles + blockIdx.x];
+    {   // digit d = tid: exclusive prefix over the warps, seeded with the global offset of (d, tile)
+        u32 run = table[(size_t)tid * tiles + blockIdx.x];
 #pragma unroll
         for (int w = 0; w < RS_WARPS; w++) {
-            u32 t = wh[w][threadIdx.x];
-            wh[w][threadIdx.x] = run;
+            u32 t = wh[w][tid];
+            wh[w][tid] = run;
             run += t;
         }
     }
@@ -194,6 +215,21 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const KeyT* __restric
             if (HAS_VAL) vals_out[pos] = vals_in[i];
         }
     }
+}
+
+template <typename KeyT>
+__global__ void __launch_bounds__(RS_THREADS) k_rs_hist(const KeyT* __restrict__ keys, u32* __restrict__ table, size_t n,
+                                                        int shift, u32 tiles) {
+    __shared__ u32 h[256];
+    rs_hist_tile<KeyT>(keys, table, n, shift, tiles, h);
+}
+
+template <typename KeyT, bool HAS_VAL>
+__global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out,
+                                                           const u32* __restrict__ vals_in, u32* __restrict__ vals_out,
+                                                           const u32* __restrict__ table, size_t n, int shift, u32 tiles) {
+    __shared__ u32 wh[RS_WARPS][256];
+    rs_scatter_tile<KeyT, u32, HAS_VAL>(keys_in, keys_out, vals_in, vals_out, table, n, shift, tiles, wh, threadIdx.x);
 }
 
 // The buffers of a stable radix sort: two for the keys and, for a sort that carries u32 values, two for the values.

@@ -1006,36 +1006,17 @@ __global__ void __launch_bounds__(FIN_THREADS) k_finish_ws(const IterParams<T> p
         }
     }
     if (p.n_peers) __threadfence_system();                 // peer stores are visible before this kernel is seen complete
-    block_sum2<FIN_THREADS>(accS, accR, scratch);
-    if (threadIdx.x == 0) {
-        p.slot_S[blockIdx.x] = accS;
-        p.slot_R[blockIdx.x] = accR;
-        __threadfence();
-        const unsigned tk = atomicAdd(&ctl->ticket, 1u);
-        is_last = (tk == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (is_last) {
-        __threadfence();
-        double a = 0.0, b = 0.0;
-        for (int i = threadIdx.x; i < (int)gridDim.x; i += FIN_THREADS) {
-            a += __ldcg(p.slot_S + i);
-            b += __ldcg(p.slot_R + i);
-        }
-        __syncthreads();
-        block_sum2<FIN_THREADS>(a, b, scratch);
-        if (threadIdx.x == 0) {
-            ctl->iters += 1;
-            ctl->ticket = 0;
-            ctl->tile_ctr = 0;                            // the next k_spmv_ws hands its tiles out from the start
-            if (p.parted) {                               // partial sums of this rank's rows: k_after_reduce finishes the job
-                ctl->red[0] = a;
-                ctl->red[1] = b;
-            } else {
-                ctl->S = a;
-                ctl->resid = b;
-                if (use_thr && b < thr) ctl->done = 1;    // strict `<` (Model.cs:114)
-            }
+    if (grid_sum2<FIN_THREADS, true>(accS, accR, p.slot_S, p.slot_R, ctl, scratch, &is_last) && threadIdx.x == 0) {
+        ctl->iters += 1;
+        ctl->ticket = 0;
+        ctl->tile_ctr = 0;                                // the next k_spmv_ws hands its tiles out from the start
+        if (p.parted) {                                   // partial sums of this rank's rows: k_after_reduce finishes the job
+            ctl->red[0] = accS;
+            ctl->red[1] = accR;
+        } else {
+            ctl->S = accS;
+            ctl->resid = accR;
+            if (use_thr && accR < thr) ctl->done = 1;     // strict `<` (Model.cs:114)
         }
     }
 }
@@ -1088,32 +1069,13 @@ __global__ void __launch_bounds__(FIN_THREADS) k_finish_set_ws(const IterParams<
             accR += (double)((rp > y) ? sub_rn(rp, y) : sub_rn(y, rp));
         }
     }
-    block_sum2<FIN_THREADS>(accS, accR, scratch);
-    if (threadIdx.x == 0) {
-        p.slot_S[blockIdx.x] = accS;
-        p.slot_R[blockIdx.x] = accR;
-        __threadfence();
-        const unsigned tk = atomicAdd(&ctl->ticket, 1u);
-        is_last = (tk == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (is_last) {
-        __threadfence();
-        double a = 0.0, b = 0.0;
-        for (int i = threadIdx.x; i < (int)gridDim.x; i += FIN_THREADS) {
-            a += __ldcg(p.slot_S + i);
-            b += __ldcg(p.slot_R + i);
-        }
-        __syncthreads();
-        block_sum2<FIN_THREADS>(a, b, scratch);
-        if (threadIdx.x == 0) {
-            ctl->iters += 1;
-            ctl->ticket = 0;
-            ctl->tile_ctr = 0;                            // the next k_spmv_ws hands its tiles out from the start
-            ctl->S = a;
-            ctl->resid = b;
-            if (use_thr && b < thr) ctl->done = 1;        // strict `<` (Model.cs:114)
-        }
+    if (grid_sum2<FIN_THREADS, true>(accS, accR, p.slot_S, p.slot_R, ctl, scratch, &is_last) && threadIdx.x == 0) {
+        ctl->iters += 1;
+        ctl->ticket = 0;
+        ctl->tile_ctr = 0;                                // the next k_spmv_ws hands its tiles out from the start
+        ctl->S = accS;
+        ctl->resid = accR;
+        if (use_thr && accR < thr) ctl->done = 1;         // strict `<` (Model.cs:114)
     }
 }
 
