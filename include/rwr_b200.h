@@ -120,7 +120,8 @@ typedef struct rwr_run_info {
     int32_t n_seeds;
     int32_t n_nodes;
     int32_t precision;
-    int32_t iterations;      /* deliverRanks() calls of the last (or only) seed                                 */
+    int32_t iterations;      /* deliverRanks() calls of the last (or only) seed since its constructor state or the
+                              * rank last written into it (rwr_set_rank)                                         */
     double residual;         /* last L1 residual (threshold mode), else NaN                                     */
     float iterate_ms;        /* device time of the power-iteration loop only (CUDA events on the stream)        */
     float total_ms;          /* init + iterations (+ top-k for rwr_recommend)                                   */
@@ -190,6 +191,24 @@ int rwr_run_threshold_restart(rwr_graph* g, const int32_t* nodes, const double* 
 /* the same Model re-run from the constructor state with other seeds (same count): rank buffers are reused, no
  * device allocation happens on the call.  The graph handle must still be alive.                             */
 int rwr_rerun_fixed(rwr_result* r, const int32_t* seeds, double c, int32_t n_iter);
+/* ---- a Model that has run, run again: `run(5); run(5)` is ten iterations (Model.cs:68-73), `run(double)` iterates
+ * from whatever `rank` holds (Model.cs:57-66), and a caller-written `rank` (Model.cs:7) is a warm start.  A result keeps
+ * per seed slot its rank, the restart mass the next iteration adds, and -- for a restart-set result -- its nodes and
+ * weights; every seed slot continues from its own rank, on the device, with the precision, layout and options of the
+ * run that made the result.  rwr_scores, rwr_topk and rwr_rank_all work on a continued or written result unchanged
+ * (a restart-set result keeps its union LIKE exclusion); rwr_rerun_fixed still starts from the constructor state.
+ * RWR_E_INVALID: a NULL r / v / iters_out, a slot outside [0, n_seeds); RWR_E_UNSUPPORTED: a result of a
+ * row-partitioned handle (continuing there would be a collective call).
+ * Model.run(int) on a Model that has already run: n_iter more deliverRanks() from the ranks r holds, for every slot.
+ * Bit-identical to one run of the total count (same precision, layout, options).  n_iter <= 0: nothing happens. */
+int rwr_continue_fixed(rwr_result* r, int32_t n_iter);
+/* Model.run(double) / run() (thr <= 0) from the ranks r holds; iters_out[n_seeds] = deliverRanks() calls of THIS call;
+ * max_iter <= 0: unbounded, as in rwr_run_threshold. */
+int rwr_continue_threshold(rwr_result* r, double thr, int32_t max_iter, int32_t* iters_out);
+/* `model.rank = v` (Model.cs:7): overwrite slot `seed_slot` with v[N] (original labels; rounded to float in FP32).
+ * The next continuation starts from v, with S recomputed from it.  Any double is accepted, as the reference accepts
+ * any: NaN / Inf entries poison every node one iteration later, as they do today. */
+int rwr_set_rank(rwr_result* r, int32_t seed_slot, const double* v);
 int rwr_result_get_info(rwr_result* r, rwr_run_info* info);
 /* `Model.rank` (Model.cs:7) of one seed, widened to double in FP32 mode                                    */
 int rwr_scores(rwr_result* r, int32_t seed_slot, double* out_n);

@@ -70,6 +70,9 @@ SYMBOLS = {
     "rwr_run_fixed_restart": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _f64, _i32, _i32, _pp]),
     "rwr_run_threshold_restart": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _f64, _f64, _i32, _i32, _vp, _pp]),
     "rwr_rerun_fixed": (C.c_int, [_vp, _vp, _f64, _i32]),
+    "rwr_continue_fixed": (C.c_int, [_vp, _i32]),
+    "rwr_continue_threshold": (C.c_int, [_vp, _f64, _i32, _vp]),
+    "rwr_set_rank": (C.c_int, [_vp, _i32, _vp]),
     "rwr_result_get_info": (C.c_int, [_vp, C.POINTER(rwr_run_info)]),
     "rwr_scores": (C.c_int, [_vp, _i32, _vp]),
     "rwr_topk": (C.c_int, [_vp, _i32, _vp, _vp, _vp]),

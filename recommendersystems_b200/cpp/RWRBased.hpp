@@ -21,6 +21,7 @@
 #pragma once
 
 #include <cstdint>
+#include <cstring>
 #include <limits>
 #include <map>
 #include <stdexcept>
@@ -57,6 +58,7 @@ struct ForwardLink {                                                            
 struct KeyNotFoundException : std::runtime_error { using std::runtime_error::runtime_error; };        // Recommender.cs:21, Model.cs:79
 struct ArgumentException : std::runtime_error { using std::runtime_error::runtime_error; };           // Graph.cs:86 (buildGraph twice)
 struct IndexOutOfRangeException : std::runtime_error { using std::runtime_error::runtime_error; };    // Model.cs:87
+struct NotSupportedException : std::runtime_error { using std::runtime_error::runtime_error; };       // Model.run(double), see Model
 struct RwrException : std::runtime_error {                                                            // everything else (CUDA, NCCL, ...)
     int code;
     RwrException(int code, const std::string& what) : std::runtime_error(what), code(code) {}
@@ -179,9 +181,13 @@ private:
 class Model {                                                                                            // Model.cs:5-116
 public:
     Graph* graph;
+    // Model.cs:7.  A caller may overwrite it: the next run starts from the written vector (a warm start).  Detected by
+    // comparison with the vector the last run delivered, as a changed `restart` is.
     std::vector<double> rank;
     // Model.cs:9: e_seed, or 1/N everywhere.  A caller may overwrite it: a vector that differs from the constructor's runs
-    // as a restart set (its nonzeros, rwr_run_*_restart) from the constructor's initial rank
+    // as a restart set (its nonzeros, rwr_run_*_restart).  A run after `restart` changed starts from the constructor state:
+    // run(int) for the run(int) iterations so far (threshold iterations are not replayed), and run(double) throws
+    // NotSupportedException once run(int) has run.
     std::vector<double> restart;
     int nNodes;
     double dampingFactor;
@@ -190,6 +196,7 @@ public:
     Model(Graph& graph, double dampingFactor) : graph(&graph), nNodes(graph.size()), dampingFactor(dampingFactor), seed_(-1) {
         rank.assign((size_t)nNodes, 1.0);                                                                // Model.cs:24
         restart.assign((size_t)nNodes, 1.0 / nNodes);                                                    // Model.cs:25
+        delivered_ = rank;
     }
     Model(Graph& graph, double dampingFactor, int targetNode)
         : graph(&graph), nNodes(graph.size()), dampingFactor(dampingFactor), seed_(targetNode) {
@@ -199,31 +206,59 @@ public:
             rank[(size_t)targetNode] = nNodes;
             restart[(size_t)targetNode] = 1.0;
         }
+        delivered_ = rank;
     }
     // a C# class variable is a reference: `new Model(graph, c, seed)` with `Graph* graph` reads the same here
     Model(Graph* graph, double dampingFactor) : Model(*graph, dampingFactor) {}
     Model(Graph* graph, double dampingFactor, int targetNode) : Model(*graph, dampingFactor, targetNode) {}
+    // the Model owns the result its runs continue from: moved, never copied
+    Model(const Model&) = delete;
+    Model& operator=(const Model&) = delete;
+    Model(Model&& o) noexcept { *this = std::move(o); }
+    Model& operator=(Model&& o) noexcept {
+        if (this != &o) {
+            rwr_result_destroy(res_);
+            graph = o.graph; rank = std::move(o.rank); restart = std::move(o.restart); nNodes = o.nNodes;
+            dampingFactor = o.dampingFactor; nIterations = o.nIterations; seed_ = o.seed_; total_ = o.total_;
+            res_ = o.res_; ran_restart_ = std::move(o.ran_restart_); delivered_ = std::move(o.delivered_);
+            o.res_ = nullptr;
+        }
+        return *this;
+    }
+    ~Model() { rwr_result_destroy(res_); }
 
     void run() { run_threshold(0.0); }                                    // Model.cs:52-55: (1 / double.MaxValue) * N, chosen by the library
     void run(double threshold) { run_threshold(threshold); }              // Model.cs:57-66
     void run(int nIterations) {                                           // Model.cs:68-73; successive calls accumulate, as in the reference
-        total_ += nIterations > 0 ? nIterations : 0;
-        rwr_result* r = nullptr;
-        std::vector<int32_t> nodes;
-        std::vector<double> weights;
-        if (restart_set(nodes, weights))
-            check(rwr_run_fixed_restart(graph->handle(), nodes.data(), weights.data(), (int32_t)nodes.size(), init_kind(), seed_,
-                                        dampingFactor, total_, RWR_FP64, &r));
-        else
-            check(rwr_run_fixed(graph->handle(), &seed_, 1, dampingFactor, total_, RWR_FP64, &r));
-        fetch(r);
-        this->nIterations = total_;
+        const int n = nIterations > 0 ? nIterations : 0;
+        total_ += n;
+        if (!res_ && !written()) {
+            fresh(total_);
+        } else if (live()) {
+            write_rank();
+            check(rwr_continue_fixed(res_, n));
+            fetch();
+        } else {
+            fresh(total_);
+            this->nIterations = total_;
+            return;
+        }
+        this->nIterations += n;
     }
 
 private:
     void run_threshold(double thr) {
-        rwr_result* r = nullptr;
         int32_t iters = 0;
+        if (live()) {
+            write_rank();
+            check(rwr_continue_threshold(res_, thr, 0, &iters));
+            fetch();
+            nIterations += iters;
+            return;
+        }
+        if (total_) throw NotSupportedException("run(double) after run(int) / a changed `restart`: a run from the constructor state "
+                                                "would not start from `rank`");
+        rwr_result* r = nullptr;
         std::vector<int32_t> nodes;
         std::vector<double> weights;
         if (restart_set(nodes, weights))
@@ -231,8 +266,46 @@ private:
                                             dampingFactor, thr, 0, RWR_FP64, &iters, &r));
         else
             check(rwr_run_threshold(graph->handle(), &seed_, 1, dampingFactor, thr, 0, RWR_FP64, &iters, &r));
-        fetch(r);
+        own(r);
         nIterations = iters;
+    }
+    // a run of n_iter iterations from the constructor state becomes the live result
+    void fresh(int n_iter) {
+        rwr_result* r = nullptr;
+        std::vector<int32_t> nodes;
+        std::vector<double> weights;
+        if (restart_set(nodes, weights))
+            check(rwr_run_fixed_restart(graph->handle(), nodes.data(), weights.data(), (int32_t)nodes.size(), init_kind(), seed_,
+                                        dampingFactor, n_iter, RWR_FP64, &r));
+        else
+            check(rwr_run_fixed(graph->handle(), &seed_, 1, dampingFactor, n_iter, RWR_FP64, &r));
+        own(r);
+    }
+    void own(rwr_result* r) {
+        rwr_result_destroy(res_);
+        res_ = r;
+        ran_restart_ = restart;
+        fetch();
+    }
+    // the live result can be continued: `restart` has not changed since it ran (a written rank is written into it first;
+    // one written before the first run gets a result of the constructor state to be written into)
+    bool live() {
+        if (!res_) {
+            if (!written()) return false;
+            const std::vector<double> w = rank;
+            fresh(0);
+            rank = w;
+            return true;
+        }
+        return same_bits(restart, ran_restart_);
+    }
+    bool written() const { return !same_bits(rank, delivered_); }
+    void write_rank() {
+        if ((int)rank.size() != nNodes) throw ArgumentException("rank must hold one value per node");
+        if (written()) check(rwr_set_rank(res_, 0, rank.data()));
+    }
+    static bool same_bits(const std::vector<double>& a, const std::vector<double>& b) {
+        return a.size() == b.size() && (a.empty() || std::memcmp(a.data(), b.data(), a.size() * sizeof(double)) == 0);
     }
     // the nonzeros of `restart` when it differs from the constructor's vector; false: unchanged
     bool restart_set(std::vector<int32_t>& nodes, std::vector<double>& weights) const {
@@ -246,13 +319,16 @@ private:
         return true;
     }
     int32_t init_kind() const { return seed_ < 0 ? RWR_INIT_UNIFORM : RWR_INIT_NODE; }
-    void fetch(rwr_result* r) {
-        const int rc = rwr_scores(r, 0, rank.data());
-        rwr_result_destroy(r);
-        check(rc);
+    void fetch() {
+        rank.resize((size_t)nNodes);
+        check(rwr_scores(res_, 0, rank.data()));
+        delivered_ = rank;
     }
-    int32_t seed_;
-    int total_ = 0;
+    int32_t seed_ = -1;
+    int total_ = 0;                 // run(int) iterations so far: the count a run after `restart` changed replays
+    rwr_result* res_ = nullptr;
+    std::vector<double> ran_restart_;   // `restart` as it was when res_ ran
+    std::vector<double> delivered_;     // `rank` as the last run delivered it
 };
 
 class Recommender {                                                                                      // Recommender.cs:7-52

@@ -1,9 +1,11 @@
 // Model.cs -- drop-in for Recommenders/RWRBased/Model.cs: constructors, run() / run(double) / run(int), the public
-// fields rank / nextRank / restart and the three step methods.  deliverRanks / updateRanks / checkConvergence run on
-// the device inside the run* calls; called one by one (nobody in the reference does) they are served by re-running the
-// device loop from the constructor state, which costs O(step) per call but keeps the surface.  A caller who overwrites
-// `restart` (Model.cs:9 is a public field) gets a walk that restarts over that weighted node set: every run path passes its
-// nonzeros to rwr_run_*_restart, with the constructor's initial rank.  Source only.
+// fields rank / nextRank / restart and the three step methods.  The Model keeps its result on the device: run(int) and
+// run(double) continue from the rank it holds (rwr_continue_fixed / rwr_continue_threshold; `run(5); run(5)` is `run(10)`
+// bit for bit), a caller-written `rank` is written into it first (rwr_set_rank: a warm start), and a deliverRanks() /
+// updateRanks() pair is one continued iteration.  A caller who overwrites `restart` (Model.cs:9 is a public field) gets a
+// walk that restarts over that weighted node set: a run passes its nonzeros to rwr_run_*_restart; a run after `restart`
+// changed starts from the constructor state: run(int) for the run(int) and updateRanks() iterations so far (threshold
+// iterations are not replayed), and run(double) throws NotSupportedException once either has run.  Source only.
 using System;
 using System.Collections.Generic;
 using Recommenders.RWRBased.Native;
@@ -17,8 +19,12 @@ namespace Recommenders.RWRBased {
         public double[] nextRank;               // Model.cs:8: zero except between deliverRanks() and updateRanks()
         public double[] restart;                // Model.cs:9: e_seed, or 1/N everywhere (uniform constructor); writable
         readonly int seed;                      // -1: uniform restart (Model.cs:14-31)
-        ResultHandle result;
-        double[] rankCache;
+        ResultHandle result;                    // the live result the runs continue from
+        double[] rankCache;                     // `rank` as the result holds it (a caller may write into it)
+        double[] delivered;                     // a copy of rankCache as read: a difference is a caller-written rank
+        double[] ranRestart;                    // `restart` as it was when `result` ran
+        double[] beforeDeliver;                 // deliverRanks() advanced `result`: the rank before it
+        int total;                              // run(int) and updateRanks() iterations so far: the count a run after `restart` changed replays
 
         public Model(Graph graph, double dampingFactor) : this(graph, dampingFactor, -1) { }
         public Model(Graph graph, double dampingFactor, int targetNode) {
@@ -31,7 +37,16 @@ namespace Recommenders.RWRBased {
         public void run() { runThreshold(0.0); }                    // thr <= 0 selects (1/double.MaxValue) * N, Model.cs:53
         public void run(double threshold) { runThreshold(threshold); }
         public void run(int nIterations) {                          // Model.cs:68-73; successive calls accumulate
-            runFixed(this.nIterations + Math.Max(nIterations, 0));
+            graph.RequireBuilt();
+            Settle();
+            int n = Math.Max(nIterations, 0);
+            total += n;
+            if (result == null && !Written()) { Fresh(total); this.nIterations = total; return; }
+            if (!Live()) { Fresh(total); this.nIterations = total; return; }
+            WriteRank();
+            RwrNative.Check(RwrNative.rwr_continue_fixed(result, n));
+            rankCache = null;
+            this.nIterations += n;
         }
         // the nonzeros of `restart` when the caller changed it from the constructor's vector; false: unchanged
         bool restartSet(out int[] nodes, out double[] weights) {
@@ -47,47 +62,107 @@ namespace Recommenders.RWRBased {
         }
         int initKind { get { return seed < 0 ? RwrNative.INIT_UNIFORM : RwrNative.INIT_NODE; } }
 
-        void runFixedInto(int total, out ResultHandle res) {
+        void runFixedInto(int nIter, out ResultHandle res) {
             int[] nodes; double[] weights;
             if (restartSet(out nodes, out weights))
                 RwrNative.Check(RwrNative.rwr_run_fixed_restart(graph.handle, nodes, weights, nodes.Length, initKind, seed, dampingFactor,
-                                                                total, RwrNative.FP64, out res));
+                                                                nIter, RwrNative.FP64, out res));
             else
-                RwrNative.Check(RwrNative.rwr_run_fixed(graph.handle, new[] { seed }, 1, dampingFactor, total, RwrNative.FP64, out res));
+                RwrNative.Check(RwrNative.rwr_run_fixed(graph.handle, new[] { seed }, 1, dampingFactor, nIter, RwrNative.FP64, out res));
         }
-        void runFixed(int total) {
-            graph.RequireBuilt();
+        // a run of nIter iterations from the constructor state becomes the live result
+        void Fresh(int nIter) {
             Release();
-            runFixedInto(total, out result);
-            nIterations = total;
+            runFixedInto(nIter, out result);
+            ranRestart = (double[])restart.Clone();
         }
+        // the live result can be continued: `restart` has not changed since it ran.  A rank written before the first run gets
+        // a result of the constructor state to be written into.
+        bool Live() {
+            if (result == null) {
+                if (!Written()) return false;
+                double[] w = rankCache;
+                Fresh(0);
+                rankCache = w;
+                return true;
+            }
+            if (restart == null || restart.Length != nNodes) return false;      // the run from the constructor state throws
+            for (int i = 0; i < nNodes; i++) if (restart[i] != ranRestart[i]) return false;
+            return true;
+        }
+        bool Written() {
+            if (rankCache == null) return false;
+            if (delivered == null) return true;
+            for (int i = 0; i < nNodes; i++)
+                if (BitConverter.DoubleToInt64Bits(rankCache[i]) != BitConverter.DoubleToInt64Bits(delivered[i])) return true;
+            return false;
+        }
+        void WriteRank() { if (Written()) RwrNative.Check(RwrNative.rwr_set_rank(result, 0, rankCache)); }
         void runThreshold(double thr) {
             graph.RequireBuilt();
-            if (nIterations != 0) throw new NotSupportedException("run(threshold) after run(int) / deliverRanks() on the same Model");
-            Release();
+            Settle();
             var iters = new int[1];
+            if (Live()) {
+                WriteRank();
+                RwrNative.Check(RwrNative.rwr_continue_threshold(result, thr, 0, iters));
+                rankCache = null;
+                nIterations += iters[0];
+                return;
+            }
+            if (total != 0)
+                throw new NotSupportedException("run(double) after run(int) / updateRanks() and a changed `restart`: a run from the " +
+                                                "constructor state would not start from `rank`");
+            Release();
             int[] nodes; double[] weights;
             if (restartSet(out nodes, out weights))
                 RwrNative.Check(RwrNative.rwr_run_threshold_restart(graph.handle, nodes, weights, nodes.Length, initKind, seed, dampingFactor,
                                                                     thr, 0, RwrNative.FP64, iters, out result));
             else
                 RwrNative.Check(RwrNative.rwr_run_threshold(graph.handle, new[] { seed }, 1, dampingFactor, thr, 0, RwrNative.FP64, iters, out result));
+            ranRestart = (double[])restart.Clone();
             nIterations = iters[0];
         }
+        // a deliverRanks() without its updateRanks(): `rank` is still the rank before it, put it back
+        void Settle() {
+            if (beforeDeliver == null) return;
+            RwrNative.Check(RwrNative.rwr_set_rank(result, 0, beforeDeliver));
+            rankCache = beforeDeliver; delivered = (double[])beforeDeliver.Clone(); beforeDeliver = null;
+            Array.Clear(nextRank, 0, nNodes);
+        }
 
-        // Model.cs:76-100: nextRank <- one more iteration from `rank`
+        // Model.cs:76-100: nextRank <- one more iteration from `rank`; `rank` is unchanged.  A second call before
+        // updateRanks() changes nothing.
         public void deliverRanks() {
             graph.RequireBuilt();
-            ResultHandle next;
-            runFixedInto(nIterations + 1, out next);
-            using (next) RwrNative.Check(RwrNative.rwr_scores(next, 0, nextRank));
+            if (beforeDeliver != null) return;
+            if (result == null && !Written()) Fresh(0);
+            if (!Live()) {                          // `restart` changed: from the constructor state, O(step) per call
+                ResultHandle next;
+                runFixedInto(total + 1, out next);
+                using (next) RwrNative.Check(RwrNative.rwr_scores(next, 0, nextRank));
+                return;
+            }
+            WriteRank();
+            double[] before = (double[])rank.Clone();
+            RwrNative.Check(RwrNative.rwr_continue_fixed(result, 1));
+            RwrNative.Check(RwrNative.rwr_scores(result, 0, nextRank));
+            beforeDeliver = before;
         }
         // Model.cs:103-108: rank <- nextRank, nextRank <- 0
         public void updateRanks() {
-            rankCache = (double[])nextRank.Clone();
+            total += 1;
+            if (beforeDeliver != null) {
+                rankCache = (double[])nextRank.Clone(); delivered = (double[])nextRank.Clone(); beforeDeliver = null;
+            } else if (Live()) {
+                WriteRank();
+                RwrNative.Check(RwrNative.rwr_continue_fixed(result, 1));
+                rankCache = null;
+            } else {
+                Fresh(total);
+                nIterations = total - 1;
+            }
             Array.Clear(nextRank, 0, nNodes);
             nIterations += 1;
-            if (result != null) { result.Dispose(); result = null; }
         }
         // Model.cs:110-115: sequential sum of |rank - nextRank|, strict `<`
         public bool checkConvergence(double threshold) {
@@ -97,20 +172,30 @@ namespace Recommenders.RWRBased {
             return diff < threshold;
         }
 
+        // Model.cs:7.  The array is the Model's: a caller may write into it, or assign a new one, and the next run starts from
+        // what it holds (a warm start).
         public double[] rank {
             get {
+                if (beforeDeliver != null) return beforeDeliver;
                 if (rankCache != null) return rankCache;
                 var r = new double[nNodes];
                 if (result == null) {               // constructor state, Model.cs:24 / :44
                     for (int i = 0; i < nNodes; i++) r[i] = seed < 0 ? 1.0 : (i == seed ? nNodes : 0.0);
-                    return rankCache = r;
+                } else {
+                    RwrNative.Check(RwrNative.rwr_scores(result, 0, r));
                 }
-                RwrNative.Check(RwrNative.rwr_scores(result, 0, r));
+                delivered = (double[])r.Clone();
                 return rankCache = r;
+            }
+            set {
+                if (value == null || value.Length != nNodes) throw new ArgumentException("rank must hold one value per node");
+                Settle();                           // a pending deliverRanks(): the result goes back to the rank before it
+                if (rankCache == null) { var unused = rank; }      // `delivered`: what the result holds
+                rankCache = value;
             }
         }
 
-        void Release() { rankCache = null; if (result != null) { result.Dispose(); result = null; } }
+        void Release() { rankCache = null; delivered = null; beforeDeliver = null; if (result != null) { result.Dispose(); result = null; } }
         public void Dispose() { Release(); }
     }
 }

@@ -89,6 +89,9 @@ namespace Recommenders.RWRBased.Native {
         [DllImport(Lib)] public static extern int rwr_run_threshold_restart(GraphHandle g, int[] nodes, double[] weights, int nRestart,
             int init, int initNode, double c, double thr, int maxIter, int precision, int[] itersOut, out ResultHandle result);
         [DllImport(Lib)] public static extern int rwr_rerun_fixed(ResultHandle r, int[] seeds, double c, int nIter);
+        [DllImport(Lib)] public static extern int rwr_continue_fixed(ResultHandle r, int nIter);
+        [DllImport(Lib)] public static extern int rwr_continue_threshold(ResultHandle r, double thr, int maxIter, int[] itersOut);
+        [DllImport(Lib)] public static extern int rwr_set_rank(ResultHandle r, int seedSlot, double[] v);
         [DllImport(Lib)] public static extern int rwr_result_get_info(ResultHandle r, out RwrRunInfo info);
         [DllImport(Lib)] public static extern int rwr_scores(ResultHandle r, int seedSlot, double[] outN);
         [DllImport(Lib)] public static extern int rwr_topk(ResultHandle r, int k, long[] outIds, double[] outScores, int[] outCounts);

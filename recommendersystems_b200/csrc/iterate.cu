@@ -125,6 +125,58 @@ __global__ void __launch_bounds__(FIN_THREADS) k_restart_s0(int n, T omc, const 
     if (threadIdx.x == 0) ctl->S = a;
 }
 
+// ---- continuing from the rank a result holds (rwr_continue_*, rwr_set_rank)
+// K6 of a continuation: x0 = fl(fl((1-c) r) inv) from the held rank r (internal labels) and the zero pad; ctl is reset as
+// k_init_set resets it, with S the restart mass kept after the slot's last run (or computed by k_resume_s from a written
+// rank).  Threshold mode (r_copy): r also goes to the buffer the residual of the first iteration reads.
+template <typename T>
+__global__ void k_init_resume(int n, int seed, T omc, const T* __restrict__ inv, const T* __restrict__ r, T* __restrict__ x0,
+                              T* __restrict__ x1, T* __restrict__ r_copy, IterCtl* ctl, const double* __restrict__ S) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < 8) { x0[n + j] = (T)0; x1[n + j] = (T)0; }
+    if (j == 0) {
+        ctl->resid = 0.0; ctl->done = 0; ctl->iters = 0; ctl->ticket = 0; ctl->fault = 0; ctl->wait_clk = 0;
+        ctl->tile_ctr = 0;
+        ctl->seed = RWR_CHK(seed < n, ctl, 7) ? seed : -1;
+        ctl->sparse = 0;
+        ctl->sparse_iters = 0;
+        ctl->S = *S;
+    }
+    if (j >= n) return;
+    const T rj = r[j];
+    x0[j] = mul_rn(mul_rn(omc, rj), inv[j]);
+    if (r_copy) r_copy[j] = rj;
+}
+
+// S of a caller-written rank r: the restart mass the epilogue sums (k_finish_ws), over the same grid (ws_fin_grid blocks
+// of FIN_THREADS), the same rows per thread and the same fixed-order reduction -- writing back the rank an epilogue
+// produced gives that epilogue's S bit for bit.
+template <typename T>
+__global__ void __launch_bounds__(FIN_THREADS) k_resume_s(int n, T omc, const T* __restrict__ inv, const T* __restrict__ r,
+                                                          double* __restrict__ slot, IterCtl* ctl, double* __restrict__ S_out) {
+    __shared__ double scratch[2 * FIN_THREADS / 32];
+    __shared__ int is_last;
+    double accS = 0.0, unused = 0.0;
+    for (int row = blockIdx.x * FIN_THREADS + threadIdx.x; row < n; row += gridDim.x * FIN_THREADS) {
+        const T y = r[row];
+        accS += (inv[row] == (T)0) ? (double)y : (double)sub_rn(y, mul_rn(omc, y));
+    }
+    if (grid_sum2<FIN_THREADS, false>(accS, unused, slot, nullptr, ctl, scratch, &is_last) && threadIdx.x == 0) {
+        *S_out = accS;
+        ctl->ticket = 0;
+    }
+}
+
+// `model.rank = v`: v (original labels, double) into the result column r (internal labels), rounded to T
+template <typename T>
+__global__ void k_set_rank(int n, const double* __restrict__ v, const int32_t* __restrict__ new_of_old, T* __restrict__ r,
+                           IterCtl* ctl) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int j = new_of_old[i];
+    if (RWR_CHK((unsigned)j < (unsigned)n, ctl, 7)) r[j] = (T)v[i];
+}
+
 __global__ void k_partition(const u32* __restrict__ in_ptr, int n, u32 nnz, int n_chunks, int2* __restrict__ part) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k > n_chunks) return;
@@ -349,11 +401,13 @@ struct RestartDev {
 };
 
 // Runs one seed (or the restart set `set`, seed_orig -1).  mode 0: fixed n_iter; mode 1: threshold.  Final rank lands in
-// y_out (internal labels).
+// y_out (internal labels).  The run starts from the constructor state (k_init, k_init_set) or, with held_S, from the rank
+// y_out holds and the restart mass *held_S (device; k_init_resume): such a run is dense from its first iteration.  cont
+// (a continuation of a result): launch kernel by kernel, neither using nor replacing the cached iteration graph.
 template <typename T>
 static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int mode, int n_iter, double thr, int max_iter,
                     T* y_out, int* iters_out, double* resid_out, float* iter_ms, cudaEvent_t ev0, cudaEvent_t ev1,
-                    const RestartDev* set = nullptr) {
+                    const RestartDev* set = nullptr, const double* held_S = nullptr, bool cont = false) {
     cudaStream_t st = g->stream;
     const int n = g->n;
     IterParams<T> p = iter_params<T>(g, ws, seed_orig, c);
@@ -367,8 +421,13 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
     // r0 goes to y_out in fixed mode (also the answer for n_iter == 0); threshold mode ping-pongs ya <-> y_out
     T* r_cur = (mode == 0) ? y_out : ya;
     // single-seed fixed-count run: the first iterations may be pushed from the frontier (frontier.cu)
-    const bool fr_on = mode == 0 && ws.fw.budget > 0 && seed_orig >= 0 && !set;
-    if (set) {
+    const bool fr_on = mode == 0 && ws.fw.budget > 0 && seed_orig >= 0 && !set && !held_S;
+    if (held_S) {
+        k_init_resume<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, p.seed, p.omc, p.inv, y_out, xa, xb,
+                                                                       mode == 0 ? nullptr : ya, ws.ctl.p, held_S);
+        KERNEL_CHECK();
+        g->pool.launches += 1;
+    } else if (set) {
         k_init_set<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, set->init, set->init_node, p.omc, p.inv, r_cur, xa, xb,
                                                                    ws.ctl.p, S_uniform, set->rs);
         KERNEL_CHECK();
@@ -407,7 +466,7 @@ static void run_one(rwr_graph* g, RunWorkspace& ws, int seed_orig, double c, int
         const u64 fr_budget = fr_on ? ws.fw.budget : 0;
         const void* key[9] = {xa, xb, y_out, ws.ctl.p, ws.head.p, ws.carry.p, ws.slot_S.p, ws.slot_R.p, fr_on ? ws.fr.p : nullptr};
         // a restart-set run launches kernel by kernel: the graphs are keyed for seeded and uniform runs only
-        const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1 && !set;
+        const bool graphable = n_iter >= 2 && dist_n_ranks(g->comm) == 1 && !no_graph && g->x_blocks == 1 && !set && !cont;
         const bool same = ig.n_iter == n_iter && ig.hub == p.hub && ig.c == c && ig.fr_budget == fr_budget &&
                           memcmp(ig.ptr, key, sizeof(key)) == 0;
         if (graphable && same && (ig.exec || ig.seen)) {
@@ -513,9 +572,14 @@ static void trace_frontier(rwr_graph* g, const RunWorkspace& ws, int seed_orig, 
                 (unsigned long long)ws.fw.budget);
 }
 
+// Runs every slot of `res` from the constructor state (seeds), or -- cont -- continues every slot from the rank it holds:
+// n_iter more iterations (mode 0) or a threshold run (mode 1).  A fixed-count continuation of a slot whose rank nobody
+// wrote runs from the constructor state for the total count when the slot holds that state or stopped inside the sparse
+// prefix (frontier.cu): the frontier kernels and the dense ones agree to the FP64 bar only, and a run of a + b iterations
+// must keep the bits of run(a + b).
 template <typename T>
 static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_seeds, double c, int mode, int n_iter,
-                    double thr, int max_iter, int32_t* iters_out, const RestartDev* set) {
+                    double thr, int max_iter, int32_t* iters_out, const RestartDev* set, bool cont = false) {
     cudaStream_t st = g->stream;
     const size_t n = (size_t)g->n;
     if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
@@ -523,6 +587,15 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     res->ld = ld;
     if (Prec<T>::ybuf(res).n != std::max<size_t>(1, ld * (size_t)n_seeds))      // a re-run keeps its rank buffers
         Prec<T>::ybuf(res).alloc(std::max<size_t>(1, ld * (size_t)n_seeds), nullptr);
+    if (res->s_keep.n != (size_t)std::max(1, n_seeds)) {
+        res->s_keep.alloc((size_t)std::max(1, n_seeds), nullptr);
+        res->sparse_keep.alloc((size_t)std::max(1, n_seeds), nullptr);
+    }
+    std::vector<int32_t> sparse((size_t)n_seeds, 0);
+    if (cont && n_seeds) {
+        CUDA_CHECK(cudaMemcpyAsync(sparse.data(), res->sparse_keep.p, sizeof(int32_t) * (size_t)n_seeds, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+    }
     RunWorkspace ws;
     ws.alloc<T>(g, (n + 8) * sizeof(T), (mode == 0 && !set) ? frontier_budget(g) : 0);
     DevEvent ev0, ev1, evA, evB;
@@ -532,11 +605,18 @@ static void run_all(rwr_graph* g, rwr_result* res, const int32_t* seeds, int n_s
     for (int s = 0; s < n_seeds; s++) {
         int it = 0;
         double rs = NAN;
-        run_one<T>(g, ws, seeds[s], c, mode, n_iter, thr, max_iter, Prec<T>::ybuf(res).p + (size_t)s * ld, &it, &rs,
-                   &res->iterate_ms, ev0, ev1, set);
-        res->iters[s] = it;
+        const int done = cont ? res->iters[s] : 0;
+        const bool replay = cont && mode == 0 && !set && !res->written[s] &&
+                            (done == 0 || (done < FR_ITERS && sparse[s] == done));
+        const double* held_S = (cont && !replay) ? res->s_keep.p + s : nullptr;
+        run_one<T>(g, ws, seeds[s], c, mode, replay ? done + n_iter : n_iter, thr, max_iter,
+                   Prec<T>::ybuf(res).p + (size_t)s * ld, &it, &rs, &res->iterate_ms, ev0, ev1, set, held_S, cont);
+        if (replay) it -= done;                    // the iterations of this call
+        res->iters[s] = done + it;
         res->residual = rs;
         if (iters_out) iters_out[s] = it;
+        CUDA_CHECK(cudaMemcpyAsync(res->s_keep.p + s, &ws.ctl.p->S, sizeof(double), cudaMemcpyDeviceToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(res->sparse_keep.p + s, &ws.ctl.p->sparse_iters, sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
         if (getenv("RWR_FRONTIER_TRACE")) trace_frontier(g, ws, seeds[s], set);
     }
     CUDA_CHECK(cudaEventRecord(evB, st));
@@ -703,16 +783,21 @@ static int run_entry(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double
         res = reuse ? reuse : new rwr_result();
         res->y64.plain = true;                    // rank buffers may be freed after the graph (and its stream) are gone
         res->y32.plain = true;
+        res->s_keep.plain = true;
+        res->sparse_keep.plain = true;
         res->g = g;
         res->device = g->device;
         res->n_seeds = n_seeds;
         res->precision = precision;
+        res->c = c;
         res->seeds.assign(seeds, seeds + n_seeds);
         res->iters.assign(n_seeds, 0);
+        res->written.assign(n_seeds, 0);
         RestartDev set;
         if (restart) {
             restart_prepare(g, *restart, set);
             res->restart_nodes.assign(restart->nodes, restart->nodes + restart->m);
+            res->restart_weights.assign(restart->weights, restart->weights + restart->m);
         }
         const RestartDev* sp = restart ? &set : nullptr;
         if (precision == RWR_FP64) run_all<double>(g, res, seeds, n_seeds, c, mode, n_iter, thr, max_iter, iters_out, sp);
@@ -729,7 +814,81 @@ static int run_entry(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double
     }
 }
 
+// the result rules of the continuation entry points (rwr_continue_*, rwr_set_rank)
+static void resume_validate(const rwr_result* r) {
+    if (!r || !r->g) RWR_FAIL(RWR_E_INVALID, "NULL result");
+    if (dist_n_ranks(r->g->comm) > 1 || r->g->part_build)
+        RWR_FAIL(RWR_E_UNSUPPORTED, "a result of a row-partitioned graph cannot be continued or written");
+}
+
+// Model.run(int) / run(double) on a Model that has run: every slot continues from the rank r holds (run_all, cont)
+static int continue_entry(rwr_result* r, int mode, int32_t n_iter, double thr, int32_t max_iter, int32_t* iters_out) {
+    RWR_API_BEGIN
+    resume_validate(r);
+    if (mode == 1 && !iters_out) RWR_FAIL(RWR_E_INVALID, "iters_out is NULL");
+    if (mode == 0 && n_iter <= 0) return RWR_OK;
+    rwr_graph* g = r->g;
+    CUDA_CHECK(cudaSetDevice(g->device));
+    if (mode == 1 && !(thr > 0.0)) thr = (1.0 / 1.7976931348623157e308) * (double)g->n;   // Model.cs:53
+    AllocStream alloc_on(g->stream);
+    RestartDev set;
+    if (!r->restart_nodes.empty()) {
+        const RestartArgs a{r->restart_nodes.data(), r->restart_weights.data(), (int32_t)r->restart_nodes.size(), RWR_INIT_RESTART, -1};
+        restart_prepare(g, a, set);
+    }
+    const RestartDev* sp = r->restart_nodes.empty() ? nullptr : &set;
+    if (r->precision == RWR_FP64) run_all<double>(g, r, r->seeds.data(), r->n_seeds, r->c, mode, n_iter, thr, max_iter, iters_out, sp, true);
+    else run_all<float>(g, r, r->seeds.data(), r->n_seeds, r->c, mode, n_iter, thr, max_iter, iters_out, sp, true);
+    return RWR_OK;
+    RWR_API_END
+}
+
+template <typename T>
+static void set_rank_impl(rwr_graph* g, rwr_result* r, int slot, const double* v) {
+    cudaStream_t st = g->stream;
+    const int n = g->n;
+    if (Prec<T>::id == RWR_FP32) ensure_fp32_arrays(g);
+    Scratch<double> vd, slots;
+    Scratch<IterCtl> ctl;
+    vd.alloc(&g->scratch, (size_t)n);
+    slots.alloc(&g->scratch, (size_t)ws_fin_grid(g));
+    ctl.alloc(&g->scratch, 1);
+    T* col = Prec<T>::ybuf(r).p + (size_t)slot * r->ld;
+    CUDA_CHECK(cudaMemsetAsync(ctl.p, 0, sizeof(IterCtl), st));
+    if (n) CUDA_CHECK(cudaMemcpyAsync(vd.p, v, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+    k_set_rank<T><<<div_up(std::max(n, 1), 256), 256, 0, st>>>(n, vd.p, g->new_of_old.p, col, ctl.p);
+    KERNEL_CHECK();
+    k_resume_s<T><<<ws_fin_grid(g), FIN_THREADS, 0, st>>>(n, (T)(1.0 - r->c), Prec<T>::inv(g), col, slots.p, ctl.p, r->s_keep.p + slot);
+    KERNEL_CHECK();
+    g->pool.launches += 2;
+    check_exchange_fault(g, ctl.p);
+}
+
 extern "C" {
+
+int rwr_continue_fixed(rwr_result* r, int32_t n_iter) {
+    return continue_entry(r, 0, n_iter, 0.0, 0, nullptr);
+}
+
+int rwr_continue_threshold(rwr_result* r, double thr, int32_t max_iter, int32_t* iters_out) {
+    return continue_entry(r, 1, 0, thr, max_iter, iters_out);
+}
+
+int rwr_set_rank(rwr_result* r, int32_t seed_slot, const double* v) {
+    RWR_API_BEGIN
+    resume_validate(r);
+    if (!v) RWR_FAIL(RWR_E_INVALID, "v is NULL");
+    if (seed_slot < 0 || seed_slot >= r->n_seeds) RWR_FAIL(RWR_E_INVALID, "seed slot %d outside [0, %d)", seed_slot, r->n_seeds);
+    rwr_graph* g = r->g;
+    CUDA_CHECK(cudaSetDevice(g->device));
+    AllocStream alloc_on(g->stream);
+    if (r->precision == RWR_FP64) set_rank_impl<double>(g, r, seed_slot, v);
+    else set_rank_impl<float>(g, r, seed_slot, v);
+    r->written[seed_slot] = 1;
+    r->iters[seed_slot] = 0;
+    return RWR_OK;
+    RWR_API_END
+}
 
 int rwr_run_fixed(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, int32_t n_iter, int32_t precision,
                   rwr_result** out) {

@@ -26,7 +26,15 @@ struct rwr_result {
     int32_t precision = RWR_FP64;
     std::vector<int32_t> seeds;        // original labels (-1: uniform restart)
     std::vector<int32_t> restart_nodes; // restart-set run (rwr_run_*_restart): the listed nodes, original labels; else empty
-    std::vector<int32_t> iters;
+    std::vector<double> restart_weights; // their weights (a continuation rebuilds the restart set from both)
+    double c = 0.0;                    // damping of the run
+    std::vector<int32_t> iters;        // per slot: deliverRanks() calls since the constructor state or the last written rank
+    std::vector<char> written;         // per slot: the rank was written by the caller (rwr_set_rank) since the last run from
+                                       // the constructor state
+    // per slot, the state a continuation starts from besides the rank: the restart mass S the next iteration adds
+    // (IterCtl.S) and the iterations the frontier kernels did (IterCtl.sparse_iters), copied on the device after each run
+    DevBuf<double> s_keep;
+    DevBuf<int32_t> sparse_keep;
     double residual = 0.0;
     float iterate_ms = 0.f, total_ms = 0.f;
     int64_t launches = 0;

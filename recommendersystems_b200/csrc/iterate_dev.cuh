@@ -83,7 +83,8 @@ struct RestartSet {
 };
 
 // Checked build: an index outside its array leaves a code in IterCtl.fault (2 gather source, 3 row-sum store, 4 virtual row
-// of the epilogue, 5 restart-set bitmap word, 6 restart-set weight) and the access is skipped; the run then fails with
+// of the epilogue, 5 restart-set bitmap word, 6 restart-set weight, 7 node label of a held or written rank) and the access
+// is skipped; the run then fails with
 // RWR_E_INVALID instead of corrupting memory.
 #ifdef RWR_CHECKED
 #define RWR_CHK(cond, ctl, code) ((cond) ? true : ((ctl)->fault = (code), false))

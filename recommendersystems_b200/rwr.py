@@ -352,6 +352,24 @@ class _Result:
             raise ValueError("rerun() needs the same number of seeds")
         _check(N.lib().rwr_rerun_fixed(self._h, _p(s), float(c), int(n_iter)))
 
+    def continue_fixed(self, n_iter: int) -> None:
+        """`Model.run(int)` again: n_iter more iterations of every slot from the rank it holds, bit-identical to one run of
+        the total count (n_iter <= 0: nothing)."""
+        _check(N.lib().rwr_continue_fixed(self._h, int(n_iter)))
+
+    def continue_threshold(self, thr: float = 0.0, max_iter: int = 0) -> np.ndarray:
+        """`Model.run(double)` (thr <= 0: `Model.run()`) from the rank every slot holds -> iterations of this call per slot."""
+        it = np.zeros(self.n_seeds, np.int32)
+        _check(N.lib().rwr_continue_threshold(self._h, float(thr), int(max_iter), _p(it)))
+        return it
+
+    def set_rank(self, slot: int, v) -> None:
+        """`model.rank = v`: the next continuation of `slot` starts from v (N doubles, original labels)."""
+        a = np.ascontiguousarray(v, np.float64)
+        if a.shape != (self.n_nodes,):
+            raise ValueError(f"rank must hold {self.n_nodes} values")
+        _check(N.lib().rwr_set_rank(self._h, int(slot), _p(a)))
+
     def scores(self, slot: int = 0) -> np.ndarray:
         out = np.empty(self.n_nodes, np.float64)
         _check(N.lib().rwr_scores(self._h, slot, _p(out)))
@@ -424,7 +442,12 @@ def run_threshold_restart(graph: Graph, nodes: Sequence[int], weights: Sequence[
 
 class Model:
     """Model.cs:5-116.  `Model(graph, d)` = uniform restart, `Model(graph, d, targetNode)` = seeded.  `restart` (Model.cs:9)
-    may be assigned an N-vector: every run then restarts over its nonzeros, from the constructor's initial rank."""
+    may be assigned an N-vector: every run then restarts over its nonzeros.  The Model keeps its live result on the device:
+    `run(int)` and `run(double)` continue from the rank it holds (`run(5); run(5)` is `run(10)`, bit for bit), and an
+    assigned `rank` (Model.cs:7) is where the next run starts -- a warm start.  On a row-partitioned graph, or after
+    `restart` changed since the last run, a run starts from the constructor state instead: run(int) for the run(int) and
+    updateRanks() iterations so far (threshold iterations are not replayed), and run(double) raises NotImplementedError once
+    either has run.  A rank cannot be written on a row-partitioned graph."""
 
     def __init__(self, graph: Graph, dampingFactor: float, targetNode: Optional[int] = None, precision: int = FP64):
         self.graph = graph
@@ -433,8 +456,11 @@ class Model:
         self.targetNode = targetNode
         self.precision = precision
         self.nIterations = 0              # deliverRanks() calls so far
-        self._fixed_total = 0
+        self._fixed_total = 0             # run(int) and updateRanks() iterations so far: the count a fallback run replays
         self._res: Optional[_Result] = None
+        self._res_restart: Optional[np.ndarray] = None   # `restart` as it was when _res ran
+        self._delivered: Optional[np.ndarray] = None     # deliverRanks() has advanced _res: the rank before it
+        self._held: Optional[np.ndarray] = None          # a host copy of the rank _res holds (None: not read since it changed)
         self.residual = float("nan")
         self.nextRank = np.zeros(self.nNodes)         # Model.cs:8
         self._restart: Optional[np.ndarray] = None    # None: the constructor's restart vector
@@ -456,29 +482,60 @@ class Model:
         init = INIT_UNIFORM if self.targetNode is None else INIT_NODE
         return run_fixed_restart(self.graph, s[0], s[1], self.dampingFactor, n_iter, init, max(self._seed(), 0), self.precision)
 
+    def _fresh(self, n_iter: int) -> None:
+        """the live result becomes a run of n_iter iterations from the constructor state"""
+        self._res = self._run_fixed(n_iter)
+        self._held = None
+        self._res_restart = None if self._restart is None else self._restart.copy()
+
+    def _live(self) -> bool:
+        """the live result can be continued: it exists, the graph is not row-partitioned, `restart` has not changed"""
+        if self._res is None or self.graph._comm is not None:
+            return False
+        a, b = self._res_restart, self._restart
+        return (a is None and b is None) or (a is not None and b is not None and np.array_equal(a, b))
+
+    def _settle(self) -> None:
+        """a deliverRanks() without its updateRanks(): `rank` is still the rank before it, put it back"""
+        if self._delivered is not None:
+            prev, self._delivered = self._delivered, None
+            self._res.set_rank(0, prev)
+            self._held = prev
+            self.nextRank = np.zeros(self.nNodes)
+
     def run(self, arg=None, max_iter: int = 0) -> None:
         """run(int nIterations) / run(double threshold) / run() -- Model.cs:68-73, :57-66, :52-55."""
+        self._settle()
+        self._held = None
         if isinstance(arg, (int, np.integer)) and not isinstance(arg, bool):
-            # successive run(int) calls accumulate in the reference; re-run from the constructor state
-            self._fixed_total += max(int(arg), 0)
-            self._res = self._run_fixed(self._fixed_total)
-            self.nIterations = self._fixed_total
+            n = max(int(arg), 0)
+            self._fixed_total += n
+            if self._live():
+                self._res.continue_fixed(n)
+                self.nIterations += n
+            else:
+                self._fresh(self._fixed_total)
+                self.nIterations = self._fixed_total
             return
-        if self._fixed_total:
-            raise NotImplementedError("threshold run after run(int) on the same Model is not supported")
         thr = 0.0 if arg is None else float(arg)      # thr <= 0 selects Model.run(): (1/double.MaxValue) * N
-        s = self._set()
-        if s is None:
-            self._res, it = run_threshold(self.graph, [self._seed()], self.dampingFactor, thr, max_iter, self.precision)
-            self.nIterations = int(it[0])
+        if self._live():
+            self.nIterations += int(self._res.continue_threshold(thr, max_iter)[0])
         else:
-            init = INIT_UNIFORM if self.targetNode is None else INIT_NODE
-            self._res, self.nIterations = run_threshold_restart(self.graph, s[0], s[1], self.dampingFactor, thr, max_iter, init,
-                                                                max(self._seed(), 0), self.precision)
+            if self._fixed_total:
+                raise NotImplementedError("threshold run after run(int) / updateRanks() on a row-partitioned graph or after "
+                                          "`restart` changed")
+            s = self._set()
+            self._res_restart = None if self._restart is None else self._restart.copy()
+            if s is None:
+                self._res, it = run_threshold(self.graph, [self._seed()], self.dampingFactor, thr, max_iter, self.precision)
+                self.nIterations = int(it[0])
+            else:
+                init = INIT_UNIFORM if self.targetNode is None else INIT_NODE
+                self._res, self.nIterations = run_threshold_restart(self.graph, s[0], s[1], self.dampingFactor, thr, max_iter,
+                                                                    init, max(self._seed(), 0), self.precision)
         self.residual = self._res.info().residual
 
-    # -- the step methods of Model.cs:76-115.  Nobody in the reference calls them one by one; here each deliverRanks()
-    #    re-runs the device loop from the constructor state (O(step) per call) so that the surface stays usable.
+    # -- the step methods of Model.cs:76-115: each deliverRanks() / updateRanks() pair is one iteration on the device
     def _constructor_restart(self) -> np.ndarray:     # Model.cs:25, :45-48
         r = np.zeros(self.nNodes)
         if self.targetNode is None:
@@ -496,17 +553,37 @@ class Model:
         r = np.array(value, np.float64)
         if r.shape != (self.nNodes,):
             raise ValueError(f"restart must hold {self.nNodes} weights")
+        self._settle()
         self._restart = r
 
     def deliverRanks(self) -> None:
-        res = self._run_fixed(self._fixed_total + 1)
-        self.nextRank = res.scores(0)
-        res.close()
+        """nextRank = one iteration from rank; rank is unchanged.  A second call before updateRanks() changes nothing."""
+        if self._delivered is not None:
+            return
+        if self._res is None:
+            self._fresh(0)
+        if not self._live():                          # from the constructor state, O(step) per call
+            res = self._run_fixed(self._fixed_total + 1)
+            self.nextRank = res.scores(0)
+            res.close()
+            return
+        self._delivered = self._held if self._held is not None else self._res.scores(0)
+        self._res.continue_fixed(1)
+        self.nextRank = self._held = self._res.scores(0)
 
     def updateRanks(self) -> None:
+        """rank = nextRank: the iteration deliverRanks() computed (without it, one iteration is computed here)."""
         self._fixed_total += 1
-        self.nIterations = self._fixed_total
-        self._res = self._run_fixed(self._fixed_total)
+        if self._delivered is not None:
+            self._delivered = None
+            self.nIterations += 1
+        elif self._live():
+            self._held = None
+            self._res.continue_fixed(1)
+            self.nIterations += 1
+        else:
+            self._fresh(self._fixed_total)
+            self.nIterations = self._fixed_total
         self.nextRank = np.zeros(self.nNodes)
 
     def checkConvergence(self, threshold: float) -> bool:
@@ -517,12 +594,29 @@ class Model:
 
     @property
     def rank(self) -> np.ndarray:
+        if self._delivered is not None:
+            return self._delivered
         if self._res is None:             # constructor state, Model.cs:24 / :44
             r = np.ones(self.nNodes) if self.targetNode is None else np.zeros(self.nNodes)
             if self.targetNode is not None and 0 <= self.targetNode < self.nNodes:
                 r[self.targetNode] = self.nNodes
             return r
         return self._res.scores(0)
+
+    @rank.setter
+    def rank(self, value) -> None:
+        """`model.rank = v` (Model.cs:7): the next run starts from v (a warm start).  Not on a row-partitioned graph."""
+        v = np.array(value, np.float64)
+        if v.shape != (self.nNodes,):
+            raise ValueError(f"rank must hold {self.nNodes} values")
+        if self.graph._comm is not None:
+            raise RwrError(N.RWR_E_UNSUPPORTED, "a rank cannot be written on a row-partitioned graph")
+        self._delivered = None
+        self.nextRank = np.zeros(self.nNodes)
+        if not self._live():
+            self._fresh(0)
+        self._res.set_rank(0, v)
+        self._held = None
 
 
 class Recommender:
