@@ -13,10 +13,13 @@ instructions.  It needs no GPU and nothing from /root/reference; it uses the CPU
     python profiles/microbench/wavefront_model.py [--scale 0.25] [--precision fp64|fp32]
 
 Layouts (a stage is 256 consecutive links of the stream, 8 instructions of 32 lanes):
-    lane8   (in use)  lane L owns links 8L..8L+7 of the stage; instruction k gathers link 8L+k
+    lane8             lane L owns links 8L..8L+7 of the stage; instruction k gathers link 8L+k
     lane2             lane L owns links 2L, 2L+1 of a 64-link quarter stage; instruction k gathers 2L+k
     link              instruction i gathers links 32i..32i+31 (lane L <- link 32i+L)
-each with the sources of a row in the order in use (original source ascending) and sorted by internal label.
+    hybrid  (in use)  link for a stage without a row end (one that lies inside a row), lane8 for every other stage
+each with the sources of a row in three orders: original source ascending ("by source", the order before the hybrid
+layout), sorted by internal label ("by label"), and sorted by internal label in the rows of more than 256 links only
+("long by label", the order in use: shorter rows never fill a stage without a row end).
 """
 from __future__ import annotations
 
@@ -62,16 +65,19 @@ def relabel(n, src, dst):
 
 
 def build_stream(n, src, dst, new_of_old, sort_in_row):
-    """stream.cu: rows of W^T by ascending internal label, one padding link (label n) for a row without in-links."""
+    """stream.cu: rows of W^T by ascending internal label, one padding link (label n) for a row without in-links.
+    sort_in_row: False (sources in original order), True (by internal label), "long" (by internal label in the rows of
+    more than STAGE links only)."""
     row = new_of_old[dst]
     s_lab = new_of_old[src]
+    indeg = np.bincount(row, minlength=n)
     if sort_in_row:
-        key = row.astype(np.int64) * (n + 1) + s_lab
+        lab = s_lab if sort_in_row is True else np.where(indeg[row] > STAGE, s_lab, 0)
+        key = row.astype(np.int64) * (n + 1) + lab
         o = np.argsort(key, kind="stable")
     else:
         o = np.argsort(row, kind="stable")                  # links arrive source-ascending: stable keeps that order
     s_sorted = s_lab[o]
-    indeg = np.bincount(row, minlength=n)
     length = np.maximum(indeg, 1)
     ptr2 = np.zeros(n + 1, np.int64)
     np.cumsum(length, out=ptr2[1:])
@@ -97,10 +103,26 @@ def blocked_stats(n, src, dst, new_of_old, blocks):
     return plain, blocked, virtual - len(pairs)
 
 
-def instr_matrix(stream, layout, n):
-    """[instructions, 32] labels, one row per warp-level gather instruction."""
+def row_ends(n, dst, new_of_old):
+    """[stream links] True on the last link of every row (the end flag of stream.cu)"""
+    ptr2 = np.cumsum(np.maximum(np.bincount(new_of_old[dst], minlength=n), 1))
+    ends = np.zeros(ptr2[-1], bool)
+    ends[ptr2 - 1] = True
+    return ends
+
+
+def instr_matrix(stream, layout, n, ends=None):
+    """[instructions, 32] labels, one row per warp-level gather instruction (hybrid: needs the row ends)."""
     pad = (-len(stream)) % STAGE
     s = np.concatenate([stream, np.full(pad, n, np.int32)]) if pad else stream
+    if layout == "hybrid":
+        st = s.reshape(-1, STAGE)
+        e = np.concatenate([ends, np.zeros(pad, bool)]) if pad else ends
+        inside = ~e.reshape(-1, STAGE).any(axis=1)        # (the last stage holds the last row end)
+        m = np.empty((len(st), STAGE // 32, 32), np.int32)
+        m[inside] = st[inside].reshape(-1, STAGE // 32, 32)
+        m[~inside] = st[~inside].reshape(-1, 32, 8).transpose(0, 2, 1)
+        return m.reshape(-1, 32)
     if layout == "lane8":
         return s.reshape(-1, 32, 8).transpose(0, 2, 1).reshape(-1, 32)
     if layout == "lane2":
@@ -169,15 +191,18 @@ def main():
     hub_bytes = (99 if elt == 8 else 163) * 1024 - 128
     hub = min((hub_bytes // elt) & ~3, n)
     print(f"n_hot={n_hot}  hub entries={hub}  elt={elt}", flush=True)
-    print(f"{'order':10s} {'layout':6s} {'links':>11s} {'glob lanes':>11s} {'glob wf':>11s} {'wf/lane':>8s} {'shr lanes':>11s} "
+    ends = row_ends(n, dst, new_of_old)
+    print(f"stages without a row end: {int((~ends[:len(ends) // STAGE * STAGE].reshape(-1, STAGE).any(axis=1)).sum())} "
+          f"of {-(-len(ends) // STAGE)}", flush=True)
+    print(f"{'order':13s} {'layout':6s} {'links':>11s} {'glob lanes':>11s} {'glob wf':>11s} {'wf/lane':>8s} {'shr lanes':>11s} "
           f"{'shr wf':>10s} {'wf total':>11s} {'wf/link':>8s}")
-    for sort_in_row in (False, True):
+    for sort_in_row, name in ((False, "by source"), (True, "by label"), ("long", "long by label")):
         stream = build_stream(n, src, dst, new_of_old, sort_in_row)
-        for layout in ("lane8", "lane2", "link"):
-            m = instr_matrix(stream, layout, n)
+        for layout in ("lane8", "lane2", "link", "hybrid") if sort_in_row != "long" else ("lane8", "hybrid"):
+            m = instr_matrix(stream, layout, n, ends)
             g_wf, s_wf, g_l, s_l = count(m, hub, elt)
             tot = g_wf + s_wf
-            print(f"{'by label' if sort_in_row else 'by source':10s} {layout:6s} {len(stream):11d} {g_l:11d} {g_wf:11d} "
+            print(f"{name:13s} {layout:6s} {len(stream):11d} {g_l:11d} {g_wf:11d} "
                   f"{g_wf / max(g_l, 1):8.3f} {s_l:11d} {s_wf:10d} {tot:11d} {tot / len(stream):8.3f}", flush=True)
 
 

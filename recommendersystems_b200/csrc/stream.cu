@@ -14,7 +14,11 @@
 //   ws_src[q]   source label of the q-th stored link of W^T, rows back to back; bit 31 set on the LAST link of a row.
 //               A row without in-links gets one padding link to the always-zero entry x[n], so every row owns >= 1
 //               link, row ids are implicit (count the end flags) and y / x_next of such rows are written like any other.
-//               Inside a 256-link stage the links are stored lane-major (a lane owns 8 consecutive links).
+//               A row of more than 256 links holds its links by ascending source label (ties by pull-CSR position);
+//               shorter rows keep the pull CSR's order.  A 256-link stage that holds a row end is stored lane-major
+//               (a lane owns 8 consecutive links, what the segmented scan needs); a stage inside one row, without a
+//               row end, is stored link-major (gather instruction (j, k) reads the 32 consecutive links j*128 + k*32 ..),
+//               so that the label-sorted sources of a long row share 128-byte lines (ws_stage_link).
 //   ws_val[q]   normalised weight of the link (valued layout only; the index-only layout folds the row's common
 //               weight into x, see graph.cu)
 //   ws_tile[t]  row of the first link of tile t | bit 31 when that row started in an earlier tile.  A tile is 4096 links
@@ -95,33 +99,100 @@ __device__ __forceinline__ u32 hub_translate(const HubMap& m, u32 label) {
     return label + (u32)m.H;
 }
 
+// Link of a stage (0 .. WS_STAGE-1) that physical offset o of the stage holds.  Lane L loads the int4 at o = j*128 + L*4
+// in round j, and gathers its element k with instruction (j, k).
+//   lane-major: o holds link L*8 + j*4 + k -- a lane owns 8 consecutive links, which the segmented scan of a stage with
+//               row ends needs;
+//   link-major: o holds link j*128 + k*32 + L -- instruction (j, k) gathers 32 consecutive links, so a row sorted by
+//               source label touches fewer 128-byte lines.
+// The build stores a stage link-major exactly when it holds no end-of-row flag (it lies inside one row whose last link
+// comes after it).  ws_consume sums such a stage on its H == 0 path, where every lane adds its own 8 values into its own
+// partial and which links a lane holds does not matter; any other stage must stay lane-major.
+__device__ __forceinline__ u32 ws_stage_link(u32 o, bool link_major) {
+    const u32 rnd = o / WS_STEP, ln = (o % WS_STEP) / 4, k = o % 4;
+    return link_major ? rnd * WS_STEP + k * 32 + ln : ln * (WS_R * 4) + rnd * 4 + k;
+}
+
 // The stream covers the links [q0, q0 + nnz2) of the whole-graph numbering (q0 > 0 for a row slice of a partitioned graph).
+// A row of more than WS_STAGE links (the only rows that can hold a flag-free stage) is stored in the order of lperm:
+// row i of the slice owns lperm[loff[i] ..], pull-CSR positions sorted by source label (ws_long_row_order).  Every other
+// row keeps the pull CSR's order.
 __global__ void k_ws_fill(const u32* __restrict__ ptr2, const u32* __restrict__ in_ptr, const int32_t* __restrict__ in_src,
-                          const double* __restrict__ in_val, int n, u32 q0, u32 nnz2, size_t padded, const HubMap hm,
-                          int32_t* __restrict__ ws_src, double* __restrict__ ws_val /* may be null */) {
+                          const double* __restrict__ in_val, const u32* __restrict__ loff, const u32* __restrict__ lperm, int n,
+                          int row_begin, u32 q0, u32 nnz2, size_t padded, const HubMap hm, int32_t* __restrict__ ws_src,
+                          double* __restrict__ ws_val /* may be null */) {
     const size_t phys = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (phys >= padded) return;
-    // Inside a stage of WS_STAGE links the stream is stored lane-major: the int4 that lane L loads in round j (physical
-    // offset j*128 + L*4) holds the links L*8 + j*4 .. +3 of the stage, so a lane owns 8 consecutive links.
     const u32 o = (u32)(phys % WS_STAGE);
-    const u32 rnd = o / WS_STEP, ln = (o % WS_STEP) / 4, k = o % 4;
-    const size_t q = phys - o + (size_t)(ln * (WS_R * 4) + rnd * 4 + k);
+    const size_t qs = phys - o;                   // first link of the stage
     const u32 zero_entry = (u32)n + (u32)hm.H;   // x[n] == 0
+    bool link_major = false;
+    int r = 0;
+    if (qs < nnz2) {
+        r = ws_row_of(ptr2, n, q0 + (u32)qs);
+        link_major = ptr2[r + 1] > q0 + (u32)qs + WS_STAGE;      // the row's last link lies after the stage: no end flag
+    }
+    const size_t q = qs + ws_stage_link(o, link_major);
     if (q >= nnz2) {                          // tail padding of the last tile: zero entry, no flag
         ws_src[phys] = (int32_t)zero_entry;
         if (ws_val) ws_val[phys] = 0.0;
         return;
     }
-    const int r = ws_row_of(ptr2, n, q0 + (u32)q);
+    if (!link_major) r = ws_row_of(ptr2, n, q0 + (u32)q);
     const u32 j = q0 + (u32)q - ptr2[r];
     const u32 b = in_ptr[r], deg = in_ptr[r + 1] - b;
     if (deg == 0) {
         ws_src[phys] = (int32_t)(zero_entry | END_BIT);
         if (ws_val) ws_val[phys] = 0.0;
     } else {
-        ws_src[phys] = (int32_t)(hub_translate(hm, (u32)in_src[b + j]) | (j == deg - 1 ? END_BIT : 0u));
-        if (ws_val) ws_val[phys] = in_val[b + j];
+        const u32 pos = deg > (u32)WS_STAGE ? lperm[loff[r - row_begin] + j] : b + j;
+        ws_src[phys] = (int32_t)(hub_translate(hm, (u32)in_src[pos]) | (j == deg - 1 ? END_BIT : 0u));
+        if (ws_val) ws_val[phys] = in_val[pos];
     }
+}
+
+// ---- source-label order of the long rows ------------------------------------------------------------------------------
+// Rows of the slice [row_begin, row_begin + R) with more than WS_STAGE links: cnt[i] = their link count, 0 for the others.
+__global__ void k_ws_long_len(const u32* __restrict__ in_ptr, int row_begin, int R, u32* __restrict__ cnt) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < R) {
+        const u32 d = in_ptr[row_begin + i + 1] - in_ptr[row_begin + i];
+        cnt[i] = d > (u32)WS_STAGE ? d : 0u;
+    }
+}
+// one warp per row: key (row, source label), value the pull-CSR position
+__global__ void k_ws_long_keys(const u32* __restrict__ in_ptr, const int32_t* __restrict__ in_src, const u32* __restrict__ loff,
+                               int row_begin, int R, int label_bits, u64* __restrict__ keys, u32* __restrict__ vals) {
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (i >= (size_t)R) return;
+    const u32 b = in_ptr[row_begin + i], deg = in_ptr[row_begin + i + 1] - b;
+    if (deg <= (u32)WS_STAGE) return;
+    const u32 base = loff[i];
+    for (u32 j = lane; j < deg; j += 32) {
+        keys[base + j] = ((u64)i << label_bits) | (u64)(u32)in_src[b + j];
+        vals[base + j] = b + j;
+    }
+}
+
+// The pull-CSR positions of the slice's rows of more than WS_STAGE links, row after row, each row by ascending source label
+// (ties by position: the sort is stable and starts from position order); loff (R + 1 entries) = where each row starts.
+// Returns an empty buffer when no row is that long.
+static DevBuf<u32> ws_long_row_order(rwr_graph* g, int row_begin, int R, DevBuf<u32>& loff) {
+    cudaStream_t st = g->stream;
+    loff.alloc((size_t)R + 1);
+    k_ws_long_len<<<div_up((size_t)R, 256), 256, 0, st>>>(g->in_ptr.p, row_begin, R, loff.p);
+    KERNEL_CHECK();
+    const u32 m = prim::scan_total<u32>(loff.p, loff.p, (size_t)R, true, st, &g->pool);
+    if (m == 0) return DevBuf<u32>();
+    prim::SortBuffers<u64> sb;
+    sb.alloc(m, true);
+    const int label_bits = ceil_log2_u64((u64)g->n);
+    k_ws_long_keys<<<div_up((size_t)R * 32, 256), 256, 0, st>>>(g->in_ptr.p, g->in_src.p, loff.p, row_begin, R, label_bits,
+                                                               sb.keys(), sb.vals());
+    KERNEL_CHECK();
+    sb.sort(m, label_bits + ceil_log2_u64((u64)R), st, &g->pool);
+    return sb.take_vals();
 }
 
 __global__ void k_ws_tiles(const u32* __restrict__ ptr2, int n, u32 q0, int row_end, int n_tiles, u32 tile_links,
@@ -465,9 +536,13 @@ void stream_prepare(rwr_graph* g) {
                                                                   g->ws_src.p, valued ? g->ws_val64.p : nullptr);
         k_ws_tiles<<<div_up((size_t)n_tiles + 1, 256), 256, 0, st>>>(ptr2v.p, V, 0u, V, n_tiles, (u32)tile_links, g->ws_tile.p);
     } else {
+        DevBuf<u32> loff;                                  // freed with the order after the fill
+        const DevBuf<u32> lperm = ws_long_row_order(g, g->row_begin, g->row_end - g->row_begin, loff);
         if (padded)
-            k_ws_fill<<<div_up(padded, 256), 256, 0, st>>>(ptr2.p, g->in_ptr.p, g->in_src.p, valued ? g->in_val64.p : nullptr, n, q0,
-                                                          nnz2, padded, hm, g->ws_src.p, valued ? g->ws_val64.p : nullptr);
+            k_ws_fill<<<div_up(padded, 256), 256, 0, st>>>(ptr2.p, g->in_ptr.p, g->in_src.p, valued ? g->in_val64.p : nullptr, loff.p,
+                                                          lperm.p, n, g->row_begin, q0, nnz2, padded, hm, g->ws_src.p,
+                                                          valued ? g->ws_val64.p : nullptr);
+        CUDA_CHECK(cudaStreamSynchronize(st));
         k_ws_tiles<<<div_up((size_t)n_tiles + 1, 256), 256, 0, st>>>(ptr2.p, n, q0, g->row_end, n_tiles, (u32)tile_links, g->ws_tile.p);
     }
     KERNEL_CHECK();
@@ -571,8 +646,9 @@ struct WsState {
     int tile;
 };
 
-// One stage of WS_STAGE links: this lane owns 8 consecutive links of the stream (the build stores a stage lane-major
-// so that the two int4 loads stay coalesced); e = their end-of-row flags (bit k), v = their products in storage order.
+// One stage of WS_STAGE links: this lane owns 8 consecutive links of the stream when the stage holds a row end (the build
+// stores such a stage lane-major so that the two int4 loads stay coalesced), 8 links 32 apart when it does not (link-major,
+// ws_stage_link); e = their end-of-row flags (bit k), v = their products in storage order.
 // Registers and shuffles only: a load here would sit behind every gather already queued in the SM's L1TEX FIFO.
 template <typename T, bool DBG>
 __device__ __forceinline__ void ws_consume(const IterParams<T>& p, WsState& s, const u32 e, const double (&v)[8], const int lane,
@@ -580,7 +656,8 @@ __device__ __forceinline__ void ws_consume(const IterParams<T>& p, WsState& s, c
     const u32 FULL = 0xffffffffu;
     const u32 H = __ballot_sync(FULL, e != 0);
     if (H == 0 || (DBG && p.debug == 1)) {
-        // inside one long row: per-lane partial, no cross-lane traffic
+        // inside one long row: per-lane partial, no cross-lane traffic (the only path on which the build may store a stage
+        // link-major: which links a lane holds does not matter here, see ws_stage_link)
         const double a = __dadd_rn(__dadd_rn(v[0], v[1]), __dadd_rn(v[2], v[3]));
         const double b = __dadd_rn(__dadd_rn(v[4], v[5]), __dadd_rn(v[6], v[7]));
         s.lane_acc = __dadd_rn(s.lane_acc, __dadd_rn(a, b));
