@@ -232,6 +232,13 @@ int rwr_recommend(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c,
  * bench.py for the roofline of the dominant kernel.                                                                  */
 int rwr_profile_iteration(rwr_graph* g, int32_t seed, double c, int32_t precision, int32_t reps, float* spmv_ms,
                           float* fixup_ms);
+/* ---- parity probe: the rank vectors the batched request path (rwr_recommend with n_seeds >= 2, rwr_evaluate_users)
+ * computes -- seeds in SpMM tiles of 8 (FP64) / 16 (FP32) consecutive seeds, n_iter iterations from the seeded
+ * constructor state -- written to out[n_seeds * N] in original labels, widened to double.  For tests.  Validation as in
+ * rwr_recommend (seed -1: RWR_E_INVALID, outside [0, N): RWR_E_BADSEED, row-partitioned handle: RWR_E_UNSUPPORTED); a seed
+ * without raw links is accepted: that rule belongs to the recommendation, not to the iteration.                      */
+int rwr_probe_tile_ranks(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, int32_t n_iter,
+                         int32_t precision, double* out);
 
 /* ---- evaluation (next row N1): Experiment.cs:121-128 on a ranking held on the host ---- */
 int rwr_evaluate(const int64_t* ranked_ids, int64_t n, const int64_t* test_ids, int64_t n_test, int32_t* hits,

@@ -80,6 +80,7 @@ SYMBOLS = {
     "rwr_result_destroy": (None, [_vp]),
     "rwr_recommend": (C.c_int, [_vp, _vp, _i32, _f64, _i32, _i32, _i32, _vp, _vp, _vp, C.POINTER(rwr_run_info)]),
     "rwr_profile_iteration": (C.c_int, [_vp, _i32, _f64, _i32, _i32, _vp, _vp]),
+    "rwr_probe_tile_ranks": (C.c_int, [_vp, _vp, _i32, _f64, _i32, _i32, _vp]),
     "rwr_evaluate": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp]),
     "rwr_methodology_masks": (C.c_int, [_i32, _vp, _vp, _vp]),
     "rwr_graph_hold_out": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _i64, _vp]),

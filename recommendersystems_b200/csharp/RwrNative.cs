@@ -114,6 +114,9 @@ namespace Recommenders.RWRBased.Native {
             out RwrRunInfo info);
         [DllImport(Lib)] public static extern int rwr_profile_iteration(GraphHandle g, int seed, double c, int precision, int reps,
             out float spmvMs, out float fixupMs);
+        // parity probe (tests): the ranks of the batched request path, out[nSeeds * N] in original labels
+        [DllImport(Lib)] public static extern int rwr_probe_tile_ranks(GraphHandle g, int[] seeds, int nSeeds, double c, int nIter,
+            int precision, double[] output);
 
         // row-partitioned mode: one process per GPU; the 128-byte id goes from rank 0 to the other ranks by any channel
         [DllImport(Lib)] public static extern int rwr_comm_unique_id(byte[] id128);

@@ -796,6 +796,57 @@ int rwr_recommend(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c,
 
 }  // extern "C"
 
+// The ranks of the batched request path, tile by tile as recommend_tiles / evaluate_tiles compose them, unpermuted and
+// widened on the host (not timed: no kernel of its own)
+template <typename T>
+static void probe_tiles(rwr_graph* g, const int32_t* seeds, int n_seeds, double c, int n_iter, double* out) {
+    cudaStream_t st = g->stream;
+    const int B = spmm_tile_width(sizeof(T) == 4 ? RWR_FP32 : RWR_FP64);
+    const size_t n = (size_t)g->n;
+    if (sizeof(T) == 4) ensure_fp32_arrays(g);
+    Scratch<int32_t> d_seeds_all;
+    const std::vector<int32_t> n2o = seed_labels(g, seeds, n_seeds, d_seeds_all);
+    Scratch<T> y;
+    y.alloc(&g->scratch, n * B + 16);
+    std::vector<T> h_y(n * B);
+    std::vector<int32_t> new_of_old(n);
+    CUDA_CHECK(cudaMemcpyAsync(new_of_old.data(), g->new_of_old.p, n * 4, cudaMemcpyDeviceToHost, st));
+    int64_t launches = 0;
+    for (int s0 = 0; s0 < n_seeds; s0 += B) {
+        const int cnt = std::min(B, n_seeds - s0);
+        spmm_run_tile<T>(g, n2o.data() + s0, cnt, c, n_iter, y.p, &launches);
+        CUDA_CHECK(cudaMemcpyAsync(h_y.data(), y.p, n * B * sizeof(T), cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        for (int j = 0; j < cnt; j++)
+            for (size_t i = 0; i < n; i++) out[(size_t)(s0 + j) * n + i] = (double)h_y[(size_t)new_of_old[i] * B + j];
+    }
+}
+
+extern "C" {
+
+int rwr_probe_tile_ranks(rwr_graph* g, const int32_t* seeds, int32_t n_seeds, double c, int32_t n_iter, int32_t precision,
+                         double* out) {
+    RWR_API_BEGIN
+    if (!g || (n_seeds && (!seeds || !out)) || n_seeds < 0) RWR_FAIL(RWR_E_INVALID, "NULL argument");
+    if (!g->built) RWR_FAIL(RWR_E_NOT_BUILT, "buildGraph() has not run");
+    if (precision != RWR_FP64 && precision != RWR_FP32) RWR_FAIL(RWR_E_INVALID, "unknown precision %d", precision);
+    for (int s = 0; s < n_seeds; s++) {
+        if (seeds[s] == -1) RWR_FAIL(RWR_E_INVALID, "seed -1 (uniform restart) is not a target user: use rwr_run_fixed + rwr_scores");
+        if (seeds[s] < 0 || seeds[s] >= g->n) RWR_FAIL(RWR_E_BADSEED, "seed %d outside [0, %d)", seeds[s], g->n);
+    }
+    if (g->comm) RWR_FAIL(RWR_E_UNSUPPORTED, "the seed tiles need the whole pull CSR: a row-partitioned handle has a slice of it");
+    if (n_seeds == 0) return RWR_OK;
+    if (n_iter < 0) n_iter = 0;
+    CUDA_CHECK(cudaSetDevice(g->device));
+    AllocStream alloc_on(g->stream);
+    if (precision == RWR_FP64) probe_tiles<double>(g, seeds, n_seeds, c, n_iter, out);
+    else probe_tiles<float>(g, seeds, n_seeds, c, n_iter, out);
+    return RWR_OK;
+    RWR_API_END
+}
+
+}  // extern "C"
+
 // ------------------------------------------------------------------------------------------------ N1: evaluation on the device
 // Experiment.cs:121-128 walks the full ranking and, for every test item it meets, adds nHits / (i + 1).  The ranking is a
 // total order (score desc, id desc: Recommender.cs:34-38), so the position of a test item is 1 + the number of candidates

@@ -264,9 +264,22 @@ __global__ void __launch_bounds__(MM_THREADS, 1) k_spmm(const MMParams<T> p) {
             else mm_finalize<T, WRITE_Y>(p, seeds_s, r, piece, pol_keep, pol_stream, acc, accS);
         }
         mm_group_sync(group);
-        // ---- pass B: rows of 32..255 nnz, one warp each: 8 quads stride over the edges, fixed shuffle tree
+        // ---- pass B: rows of 32..255 nnz, one warp each: 8 quads stride over the edges, fixed shuffle tree.  The lists
+        // fill in atomicAdd order, which depends on the timing of the warps; passes B and C visit them in an order of their
+        // own, so that every thread adds the same rows to its restart-mass partials (accS) in the same order on every run.
+        // Pass B: longest first (ties by row), dealt to the 4 warps in snake order (0 1 2 3 3 2 1 0 ...) -- balanced
         const int n_long = *l_cnt;
-        for (int li = gwarp; li < n_long; li += GROUP_THREADS / 32) {
+        int my_rank = lane;                                 // rank of list entry `lane` (the keys are distinct)
+        if (n_long > 1) {
+            const int my_key = lane < n_long ? ((1023 - (l_e[lane] - l_s[lane])) << 10) | (l_r[lane] - row0) : 0x7fffffff;
+            my_rank = 0;
+#pragma unroll
+            for (int j = 0; j < 32; j++) my_rank += __shfl_sync(0xffffffffu, my_key, j) < my_key;
+        }
+        for (int k = 0;; k++) {
+            const int q = 4 * k + ((k & 1) ? 3 - gwarp : gwarp);
+            if (q >= n_long) break;
+            const int li = __ffs(__ballot_sync(0xffffffffu, my_rank == q)) - 1;
             const int r = l_r[li];
             const u32 s = (u32)l_s[li], e = (u32)l_e[li], rs = (u32)l_rs[li];
             double acc[CW];
@@ -280,10 +293,14 @@ __global__ void __launch_bounds__(MM_THREADS, 1) k_spmm(const MMParams<T> p) {
                 else mm_finalize<T, WRITE_Y>(p, seeds_s, r, piece, pol_keep, pol_stream, acc, accS);
             }
         }
-        // ---- pass C: rows of >= 256 nnz (at most 3 per tile): the whole group
+        // ---- pass C: rows of >= 256 nnz (at most 3 per tile), in row order: the whole group
         const int n_huge = *h_cnt;
-        for (int hi = 0; hi < n_huge; hi++) {
+        for (int q = 0, prev = -1; q < n_huge; q++) {
+            int hi = 0;                                     // the entry with the q-th smallest row
+            for (int j = 1; j < n_huge; j++)
+                if (h_r[j] > prev && (h_r[hi] <= prev || h_r[j] < h_r[hi])) hi = j;
             const int r = h_r[hi];
+            prev = r;
             const u32 s = (u32)h_s[hi], e = (u32)h_e[hi], rs = (u32)h_rs[hi];
             double acc[CW];
 #pragma unroll
